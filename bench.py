@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — DEM cells/s end-to-end (fill -> D8 -> accum -> bluespot / watershed labels) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--size S] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--size S] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the whole raster hot path over ONE S x S synthetic fractal DEM (default S = 32768,
 BASELINE.json configs[2], the largest single-GPU configuration):
@@ -313,6 +313,40 @@ def timed_steps(job, lib, pipe, steps, warmup, profile=True, sampler=None):
     return job.max_over_ranks([ms])[0], launches, prof, clocks
 
 
+# --dump-outputs: a fixed, seeded sample of what RasterPipeline.run hands its caller, so that two builds can be compared
+# output for output.  2^19 cells of each raster and 2^18 entries of each table stay under 64 MB in float64.
+DUMP_CELLS, DUMP_LABELS, DUMP_SEED = 1 << 19, 1 << 18, 20240601
+
+
+def sample_index(n, k, seed):
+    """`min(n, k)` distinct indices of [0, n), ascending; the same for the same (n, k, seed)."""
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False)).astype(np.int64)
+
+
+def dump_outputs(pipe, out_dir):
+    """Every raster and per-label table of the pipeline's last run at the sampled positions as `<out_dir>/<name>.npy`:
+    float32 for the float32 and uint8 rasters, float64 (exact) for the rest.  `cell_index` / `label_index` hold the
+    sampled flat cell positions and label ids; `nlabels`, `short_eps` and `diag_eps` are the run's scalars."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cells = sample_index(pipe.rows * pipe.cols, DUMP_CELLS, DUMP_SEED)
+    labels = sample_index(pipe.nlabels + 1, DUMP_LABELS, DUMP_SEED + 1)
+    arrays = {"cell_index": cells.astype(np.float64), "label_index": labels.astype(np.float64),
+              "nlabels": np.array([pipe.nlabels], np.float64), "short_eps": np.array([pipe.short], np.float64),
+              "diag_eps": np.array([pipe.diag], np.float64)}
+    for index, source in ((cells, {k: t.view(-1) for k, t in pipe.out.items()}), (labels, pipe.tables)):
+        idx = torch.from_numpy(index).to(pipe.device)
+        for name, t in source.items():
+            v = t.index_select(0, idx).cpu().numpy()
+            exact32 = v.dtype == np.float32 or v.dtype == np.uint8
+            arrays[name] = v.astype(np.float32 if exact32 else np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sum(a.nbytes for a in arrays.values())
+
+
 def timed_e2e(job, pipe, steps):
     """Host buffers in, host buffers out: H2D of the DEM and D2H of every raster + table inside the timed region."""
     import torch
@@ -565,6 +599,8 @@ def run_ours(args):
     torch.cuda.synchronize()
     ms, launches, prof, clocks = timed_steps(job, lib, pipe, args.steps, args.warmup, profile=True,
                                              sampler=(lambda: ClockSampler(job.local)) if rank == 0 else None)
+    if args.dump_outputs:
+        dumped = dump_outputs(pipe, args.dump_outputs)
     # ---- e2e: host buffers in, host buffers out
     e2e_steps = max(1, min(args.steps, 2))
     e2e_ms = timed_e2e(job, pipe, e2e_steps)
@@ -660,6 +696,9 @@ def run_ours(args):
                              "kernel_ms_per_step_rank0": round(tot_ms / args.steps, 3),
                              "pipeline_frac": round(value * 1e6 * BYTES_PER_CELL / (world * peak * 1e9), 5)},
                 "parity": parity, "kernels": kernels, "clocks": clocks}
+        if args.dump_outputs:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "bytes": dumped,
+                                    "sample": "%d cells, %d labels, seed %d" % (DUMP_CELLS, DUMP_LABELS, DUMP_SEED)}
         line.update(sub)
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_baseline(args)
@@ -702,7 +741,14 @@ def main():
     ap.add_argument("--no-config5", action="store_true", help="skip the pathological-DEM sub-record (N = 1 and N = 8)")
     ap.add_argument("--config5-size", type=int, default=0, help="edge of the `config5` sub-record (default: --size)")
     ap.add_argument("--config4-size", type=int, default=0, help="N > 1: edge of the `config4` sub-record (default: 65536 at N = 8, none otherwise)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write a seeded sample of every raster and table of the last step as "
+                         "DIR/<name>.npy (one GPU, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs a single-GPU run of --impl ours")
     if args.warmup < 3 and args.impl != "reference":
         args.warmup = 3
     # exactly one JSON line on stdout: libraries that write to fd 1 (NCCL's version banner) go to stderr instead

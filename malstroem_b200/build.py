@@ -1,4 +1,5 @@
 """Build libmalstroem_b200.so in-tree with nvcc for sm_100a (no JIT cache: the .so travels with the repo)."""
+import glob
 import os
 import subprocess
 import sys
@@ -26,7 +27,7 @@ def _stale(target, deps):
 
 def build(force=False, verbose=False):
     os.makedirs(OBJ, exist_ok=True)
-    hdrs = [os.path.join(CSRC, "common.cuh"), os.path.join(HERE, "..", "include", "malstroem_b200.h")]
+    hdrs = sorted(glob.glob(os.path.join(CSRC, "*.cuh"))) + [os.path.join(HERE, "..", "include", "malstroem_b200.h")]
     jobs = []
     for src in SOURCES:
         sp = os.path.join(CSRC, src)

@@ -94,29 +94,65 @@ def test_enable_disable_rebinds_the_twelve_names():
     assert pkg.fill.fill_terrain() == "orig:fill_terrain" and pkg.label.label_count() == "orig:label_count"
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/malstroem"), reason="reference tree not present")
-def test_enable_on_the_real_reference_package():
-    sys.path.insert(0, "/root/reference")
+# A stand-in with the module layout of the reference package and the binding styles its tool layer relies on: modules
+# that bind `fill` / `flow` / `label` / `net` by module and resolve the functions at call time (dem.py:67, streams.py:72),
+# a `Network` class with its own `rain_event` (network.py:113), and a module that binds vectorize_labels_file by name at
+# import (bluespots.py:17).  Function bodies are irrelevant: the tests check which object each name resolves to.
+REFERENCE_LAYOUT = {
+    "malstroem/__init__.py": "",
+    "malstroem/algorithms/__init__.py": "from . import speedups\n",
+    "malstroem/algorithms/speedups/__init__.py": "enabled = False\n",
+    "malstroem/algorithms/fill.py": "def fill_terrain(dtm): pass\ndef fill_terrain_no_flats(dtm, short, diag): pass\n"
+                                    "def minimum_safe_short_and_diag(dtm): pass\n",
+    "malstroem/algorithms/flow.py": "def terrain_flowdirection(t, edges_flow_outward=True): pass\n"
+                                    "def accumulated_flow(fd): pass\ndef watersheds_from_labels(fd, lab, unassigned=0): pass\n",
+    "malstroem/algorithms/label.py": "".join("def %s(*a, **k): pass\n" % n for n in (
+        "connected_components", "label_stats", "keep_labels", "label_min_index", "label_max_index", "label_count")),
+    "malstroem/algorithms/net.py": "def next_downstream_label(*a, **k): pass\ndef pourpoint_network(*a, **k): pass\n"
+                                   "def geometric_pourpoint_network(*a, **k): pass\n",
+    "malstroem/network.py": "class Network(object):\n    def rain_event(self, mmrain): pass\n",
+    "malstroem/vector.py": "def vectorize_labels_file(*a, **k): pass\n",
+    "malstroem/bluespots.py": "from malstroem.vector import vectorize_labels_file\n",
+    "malstroem/dem.py": "from malstroem.algorithms import fill, flow\n",
+    "malstroem/streams.py": "from malstroem.algorithms import net\n",
+}
+
+
+@pytest.fixture
+def reference_layout(tmp_path):
+    for rel, src in REFERENCE_LAYOUT.items():
+        p = tmp_path / rel
+        p.parent.mkdir(parents=True, exist_ok=True)
+        p.write_text(src)
+    sys.path.insert(0, str(tmp_path))
     for k in [k for k in sys.modules if k == "malstroem" or k.startswith("malstroem.")]:
         del sys.modules[k]
     try:
-        import malstroem.algorithms as alg
-        from malstroem.algorithms import fill as rfill, flow as rflow, label as rlabel
-        orig = rfill.fill_terrain
-        speedups.enable()
-        assert alg.speedups.enabled and rfill.fill_terrain is fill.fill_terrain
-        assert rflow.watersheds_from_labels is flow.watersheds_from_labels
-        assert rlabel.label_max_index is label.label_max_index
-        # the tool layer resolves through the module at call time (malstroem/dem.py:67)
-        from malstroem import dem as rdem
-        assert rdem.fill.fill_terrain is fill.fill_terrain
-        speedups.disable()
-        assert rfill.fill_terrain is orig
+        yield
     finally:
         speedups.disable()
-        sys.path.remove("/root/reference")
+        sys.path.remove(str(tmp_path))
         for k in [k for k in sys.modules if k == "malstroem" or k.startswith("malstroem.")]:
             del sys.modules[k]
+
+
+def test_enable_on_a_package_with_the_reference_layout(reference_layout):
+    import malstroem.algorithms as alg
+    from malstroem.algorithms import fill as rfill, flow as rflow, label as rlabel
+    orig = rfill.fill_terrain
+    speedups.enable()
+    assert alg.speedups.enabled and rfill.fill_terrain is fill.fill_terrain
+    assert rflow.watersheds_from_labels is flow.watersheds_from_labels
+    assert rlabel.label_max_index is label.label_max_index
+    # the tool layer resolves through the module at call time (malstroem/dem.py:67)
+    from malstroem import dem as rdem
+    assert rdem.fill.fill_terrain is fill.fill_terrain
+    # BluespotTool's import-time binding is replaced as well (bluespots.py:17)
+    from malstroem import bluespots as rbluespots
+    from malstroem_b200 import vector
+    assert rbluespots.vectorize_labels_file is vector.vectorize_labels_file
+    speedups.disable()
+    assert rfill.fill_terrain is orig and not alg.speedups.enabled
 
 
 def test_minimum_safe_short_and_diag_scalar_part():
@@ -179,26 +215,17 @@ def test_network_class_bookkeeping_matches_reference_contract():
             net.pourpoint_network(np.zeros((4, 4), np.uint8), np.zeros((4, 4), np.int32), [(1, 1)], 0)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/malstroem"), reason="reference tree not present")
-def test_enable_rebinds_net_and_network_on_the_real_reference():
-    sys.path.insert(0, "/root/reference")
-    for k in [k for k in sys.modules if k == "malstroem" or k.startswith("malstroem.")]:
-        del sys.modules[k]
-    try:
-        import malstroem.algorithms as alg          # noqa: F401
-        from malstroem.algorithms import net as rnet
-        from malstroem import network as rnetwork
-        from malstroem_b200.algorithms import net
-        orig_pp, orig_rain = rnet.pourpoint_network, rnetwork.Network.rain_event
-        speedups.enable()
-        assert rnet.pourpoint_network is net.pourpoint_network
-        assert rnet.next_downstream_label is net.next_downstream_label
-        assert rnet.geometric_pourpoint_network is net.geometric_pourpoint_network
-        assert rnetwork.Network.rain_event is not orig_rain
-        speedups.disable()
-        assert rnet.pourpoint_network is orig_pp and rnetwork.Network.rain_event is orig_rain
-    finally:
-        speedups.disable()
-        sys.path.remove("/root/reference")
-        for k in [k for k in sys.modules if k == "malstroem" or k.startswith("malstroem.")]:
-            del sys.modules[k]
+def test_enable_rebinds_net_and_network_on_the_reference_layout(reference_layout):
+    from malstroem.algorithms import fill as rfill, flow as rflow, label as rlabel      # noqa: F401
+    from malstroem.algorithms import net as rnet
+    from malstroem import network as rnetwork, streams as rstreams
+    from malstroem_b200.algorithms import net
+    orig_pp, orig_rain = rnet.pourpoint_network, rnetwork.Network.rain_event
+    speedups.enable()
+    assert rnet.pourpoint_network is net.pourpoint_network
+    assert rnet.next_downstream_label is net.next_downstream_label
+    assert rnet.geometric_pourpoint_network is net.geometric_pourpoint_network
+    assert rstreams.net.pourpoint_network is net.pourpoint_network      # StreamTool resolves at call time
+    assert rnetwork.Network.rain_event is not orig_rain
+    speedups.disable()
+    assert rnet.pourpoint_network is orig_pp and rnetwork.Network.rain_event is orig_rain
