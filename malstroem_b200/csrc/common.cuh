@@ -66,6 +66,8 @@ double now_s();
 // requests and cost 7-46 ms per step at 8192^2 (profiles/r01_host_overhead.txt).
 void *arena_alloc(size_t bytes, cudaStream_t s);
 void arena_free(void *p, cudaStream_t s);
+// bytes the arena can still hand out without a cudaMallocAsync (0 before a call has sized it)
+size_t arena_room();
 
 template <typename T>
 struct DevBuf {

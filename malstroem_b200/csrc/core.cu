@@ -98,6 +98,8 @@ void arena_free(void *p, cudaStream_t s) {
     }
 }
 
+size_t arena_room() { return g_arena ? g_arena_cap - g_arena_top : 0; }
+
 // ---- per-kernel event timing -------------------------------------------------------------------
 int g_prof = 0;
 int64_t g_prof_units = 0;

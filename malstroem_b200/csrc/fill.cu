@@ -11,13 +11,15 @@
 //   2. forest_resolve_list  pointer jumping for the cells whose path leaves their tile -> every cell knows the
 //                     local minimum ("catchment") it drains to
 //   3. scan           dense catchment ids (0 = outside), straight from the root pointers
-//   4. Boruvka rounds on the catchment graph (edge weight = max(z_a, z_b) over adjacent cells of two
-//                     catchments): every component not yet merged with "outside" finds its lowest
-//                     outgoing edge (64-bit atomicMin of (weight, edge id); round 1 over the raster, later rounds
-//                     over the cells that still border another component), hooks to the other side, and every
-//                     catchment in it raises E = max(E, that weight).
-//                     Claim (DESIGN.md §K1): when the component reaches "outside", E is the catchment's
-//                     spill elevation.
+//   4. Boruvka on the catchment graph (edge weight = max(z_a, z_b) over adjacent cells of two catchments).
+//                     One CTA per tile (k_tile_edges) writes the catchment ids and the catchment-pair edge list,
+//                     aggregated per tile, and finds every catchment's lowest edge (64-bit atomicMin of (weight,
+//                     list position)).  Each round every live component hooks across its lowest edge and records
+//                     that weight (wk); the roots that have not reached "outside" get dense new ids, and the edges
+//                     are relabelled, those inside one component dropped, the rest compacted and searched for the
+//                     next round's lowest edges.  After the last round E = max of wk over the levels of the
+//                     catchment's component until it reaches outside (k_spill_down, top level first).
+//                     Claim (DESIGN.md §K1): E is the catchment's spill elevation.
 //   5. k_fill_final   filled = max(z, E[catchment]), depths = filled - z
 #include <string.h>
 
@@ -27,6 +29,7 @@
 namespace ms {
 
 constexpr unsigned long long KEY_NONE = ~0ull;
+constexpr unsigned long long HASH_EMPTY = ~0ull;
 
 // ---- K0 -------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_minmax(const float *z, int64_t n, uint32_t *keys, int vec) {
@@ -193,8 +196,8 @@ __global__ void __launch_bounds__(256) k_boruvka_init(int *comp, uint32_t *E, in
     }
 }
 
-// lowest outgoing edge of every component that has not reached "outside" (component 0) yet.
-// Row bands: an edge into a halo row (the neighbouring band) is "foreign": its key carries FOREIGN_BIT, which also
+// Row-band fill: lowest outgoing edge of every component that has not reached "outside" (component 0) yet.
+// An edge into a halo row (the neighbouring band) is "foreign": its key carries FOREIGN_BIT, which also
 // sorts it behind every local edge of the same weight; a component whose lowest edge is foreign freezes (k_hook).
 constexpr unsigned FOREIGN_BIT = 0x80000000u;
 
@@ -202,19 +205,18 @@ constexpr int ME_PER_THREAD = 4;      // cells per thread: one list append (atom
 
 // FIRST: round 1, where every catchment is its own component (comp[l] == l) and nothing is frozen yet — the component
 // lookups (a gather per neighbour across a catchment boundary) are skipped.
-// BAND: row bands (frozen != nullptr).
 // r: the cell's row, or for a cell given by its index alone (the list rounds) 0 / 1 / rows - 1 for first / any other /
 // last row - only "does the neighbour row exist" is asked; c < 0: the column is worked out if a foreign edge needs it
-template <bool FIRST, bool BAND>
+template <bool FIRST>
 __device__ inline bool minedge_cell(const float *__restrict__ z, const int *__restrict__ lab,
                                     const int *__restrict__ comp, const uint8_t *__restrict__ frozen,
                                     unsigned long long *best, int rows, int cols, int i, int r, int c) {
     int l = lab[i];
     int cc = FIRST ? l : (l ? comp[l] : 0);
     if (cc == 0) return false;
-    // row bands: a cell of a FROZEN component no longer searches, but stays listed while a neighbour lies in another
-    // component - the boundary graph of the frozen components is built from the last list (k_band_edges)
-    const bool fz = BAND && !FIRST && frozen[cc];      // BAND: frozen != nullptr
+    // a cell of a FROZEN component no longer searches, but stays listed while a neighbour lies in another component -
+    // the boundary graph of the frozen components is built from the last list (k_band_edges)
+    const bool fz = !FIRST && frozen[cc];
     bool other = false;
     float zc = z[i];
     unsigned long long bk = KEY_NONE;
@@ -279,11 +281,11 @@ __device__ __forceinline__ void minedge_append(unsigned keepbits, const int (&ce
         if (keepbits & (1u << u)) list_out[pos++] = cell[u];
 }
 
-template <bool LIST, bool BAND>
-__device__ __forceinline__ void minedge_body(const float *__restrict__ z, const int *__restrict__ lab,
-                                                 const int *__restrict__ comp, const uint8_t *__restrict__ frozen,
-                                                 unsigned long long *best, int rows, int cols,
-                                                 const int *__restrict__ list_in, int n_in, int *list_out, int *n_out) {
+template <bool LIST>
+__global__ void __launch_bounds__(256) k_minedge_band(const float *__restrict__ z, const int *__restrict__ lab,
+                                                      const int *__restrict__ comp, const uint8_t *__restrict__ frozen,
+                                                      unsigned long long *best, int rows, int cols,
+                                                      const int *__restrict__ list_in, int n_in, int *list_out, int *n_out) {
     int cell[ME_PER_THREAD];
     unsigned keepbits = 0;
 #pragma unroll
@@ -303,80 +305,9 @@ __device__ __forceinline__ void minedge_body(const float *__restrict__ z, const 
             if (r < rows && c < cols) i = r * cols + c;
         }
         cell[u] = i;
-        if (i >= 0 && minedge_cell<!LIST, BAND>(z, lab, comp, frozen, best, rows, cols, i, r, c)) keepbits |= 1u << u;
+        if (i >= 0 && minedge_cell<!LIST>(z, lab, comp, frozen, best, rows, cols, i, r, c)) keepbits |= 1u << u;
     }
     minedge_append(keepbits, cell, list_out, n_out);
-}
-
-// Round 1 on one GPU, cols % 4 == 0: a thread takes FOUR consecutive cells of a row and loads the three label rows and
-// the three elevation rows around them as 16-byte vectors plus the two columns either side (18 loads for 4 cells where
-// the generic form issues up to 18 per cell); every catchment is its own component and nothing is frozen.
-__global__ void __launch_bounds__(256) k_minedge_first4(const float *__restrict__ z, const int *__restrict__ lab,
-                                                        unsigned long long *best, int rows, int cols, int *list_out,
-                                                        int *n_out) {
-    const int c = (blockIdx.x * 16 + (threadIdx.x & 15)) * 4;
-    const int r = blockIdx.y * 16 + (threadIdx.x >> 4);
-    int cell[ME_PER_THREAD] = {-1, -1, -1, -1};
-    unsigned keepbits = 0;
-    if (r > 0 && r < rows - 1 && c < cols) {          // cells of the first / last row carry label 0
-        int L[3][6];
-        float Z[3][6];
-#pragma unroll
-        for (int a = 0; a < 3; a++) {
-            const size_t row = (size_t)(r - 1 + a) * cols + c;
-            const int4 l4 = __ldg(reinterpret_cast<const int4 *>(lab + row));
-            const float4 z4 = __ldg(reinterpret_cast<const float4 *>(z + row));
-            L[a][1] = l4.x; L[a][2] = l4.y; L[a][3] = l4.z; L[a][4] = l4.w;
-            Z[a][1] = z4.x; Z[a][2] = z4.y; Z[a][3] = z4.z; Z[a][4] = z4.w;
-            L[a][0] = c > 0 ? __ldg(lab + row - 1) : 0;
-            Z[a][0] = c > 0 ? __ldg(z + row - 1) : 0.f;
-            L[a][5] = c + 4 < cols ? __ldg(lab + row + 4) : 0;
-            Z[a][5] = c + 4 < cols ? __ldg(z + row + 4) : 0.f;
-        }
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const int l = L[1][j + 1];
-            const int i = r * cols + c + j;
-            cell[j] = i;
-            if (l == 0) continue;                      // raster border (first / last column)
-            const float zc = Z[1][j + 1];
-            unsigned long long bk = KEY_NONE;
-#pragma unroll
-            for (int dr = -1; dr <= 1; dr++)
-#pragma unroll
-                for (int dc = -1; dc <= 1; dc++) {
-                    if (dr == 0 && dc == 0) continue;
-                    if (L[1 + dr][j + 1 + dc] == l) continue;
-                    const float w = fmaxf(zc, Z[1 + dr][j + 1 + dc]);
-                    const int jn = i + dr * cols + dc;
-                    const int lo = jn < i ? jn : i;
-                    const int code = (dr == 0) ? 0 : ((dr * dc == -1) ? 1 : (dc == 0 ? 2 : 3));
-                    const unsigned long long key = ((unsigned long long)okey32(w) << 32) | (unsigned)(((unsigned)lo << 2) | code);
-                    bk = key < bk ? key : bk;
-                }
-            if (bk == KEY_NONE) continue;
-            if (bk < best[l]) atomicMin(&best[l], bk);
-            keepbits |= 1u << j;
-        }
-    }
-    minedge_append(keepbits, cell, list_out, n_out);
-}
-
-// two kernels from one body: the single-GPU form carries none of the frozen-component logic (compiled into one kernel
-// behind a uniform branch it cost 2 ms of 12 in round 1: the body is instruction-cache-sized)
-template <bool LIST>
-__global__ void __launch_bounds__(256) k_minedge(const float *__restrict__ z, const int *__restrict__ lab,
-                                                 const int *__restrict__ comp, const uint8_t *__restrict__ frozen,
-                                                 unsigned long long *best, int rows, int cols,
-                                                 const int *__restrict__ list_in, int n_in, int *list_out, int *n_out) {
-    minedge_body<LIST, false>(z, lab, comp, frozen, best, rows, cols, list_in, n_in, list_out, n_out);
-}
-template <bool LIST>
-__global__ void __launch_bounds__(256) k_minedge_band(const float *__restrict__ z, const int *__restrict__ lab,
-                                                      const int *__restrict__ comp, const uint8_t *__restrict__ frozen,
-                                                      unsigned long long *best, int rows, int cols,
-                                                      const int *__restrict__ list_in, int n_in, int *list_out, int *n_out) {
-    minedge_body<LIST, true>(z, lab, comp, frozen, best, rows, cols, list_in, n_in, list_out, n_out);
 }
 
 __device__ inline int edge_other(int lo, int code, int cols) {
@@ -475,11 +406,10 @@ static int descent_resolve(const float *dem, int *lab, int *scratch, int64_t row
     return forest_resolve_list(lab, scratch, *(int *)h, rounds_out, s);
 }
 
-// The Boruvka rounds shared by the single-GPU and the row-band fill.  comp / E initialised by k_boruvka_init;
-// `frozen` (row bands only, may be NULL) zeroed.  Returns the number of rounds.
-static int boruvka_rounds(const float *dem, const int *lab, int *comp, uint32_t *E, uint8_t *frozen, int nC,
-                          int64_t rows, int64_t cols, int *rounds_out, const char *what, cudaStream_t s,
-                          ms_band *B = nullptr) {
+// The Boruvka rounds of the row-band fill, on the band's cells.  comp / E initialised by k_boruvka_init, `frozen`
+// zeroed.  The last work list goes to B (BB_BLIST) for the boundary graph.
+static int boruvka_rounds_band(const float *dem, const int *lab, int *comp, uint32_t *E, uint8_t *frozen, int nC,
+                               int64_t rows, int64_t cols, cudaStream_t s, ms_band *B) {
     int64_t n = rows * cols;
     DevBuf<int> parent, counters, listA, listB;
     DevBuf<uint32_t> wk;
@@ -489,7 +419,6 @@ static int boruvka_rounds(const float *dem, const int *lab, int *comp, uint32_t 
     MS_TRY(best.alloc(nC, s));
     MS_TRY(counters.alloc(2, s));
     MS_TRY(listA.alloc((size_t)n, s));
-    dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
     unsigned gc = cdiv(nC, 256);
     int64_t *h = host_flags().h;
     MS_CUDA(cudaMemsetAsync(best.p, 0xff, (size_t)nC * sizeof(unsigned long long), s));
@@ -502,23 +431,12 @@ static int boruvka_rounds(const float *dem, const int *lab, int *comp, uint32_t 
         if (rounds == 0) {
             prof_units(n);
             dim3 g2m(cdiv(cols, 64), cdiv(rows, 4 * ME_PER_THREAD));
-            if (frozen)
-                MS_LAUNCH(k_minedge_band<false>, g2m, 256, 0, s, dem, lab, (const int *)comp, (const uint8_t *)frozen, best.p,
-                          (int)rows, (int)cols, (const int *)nullptr, 0, lout, counters.p + 1);
-            else if ((cols & 3) == 0 && ((uintptr_t)dem & 15) == 0 && ((uintptr_t)lab & 15) == 0)
-                MS_LAUNCH(k_minedge_first4, dim3(cdiv(cols, 64), cdiv(rows, 16)), 256, 0, s, dem, lab, best.p, (int)rows, (int)cols,
-                          lout, counters.p + 1);
-            else
-                MS_LAUNCH(k_minedge<false>, g2m, 256, 0, s, dem, lab, (const int *)comp, (const uint8_t *)frozen, best.p,
-                          (int)rows, (int)cols, (const int *)nullptr, 0, lout, counters.p + 1);
+            MS_LAUNCH(k_minedge_band<false>, g2m, 256, 0, s, dem, lab, (const int *)comp, (const uint8_t *)frozen, best.p,
+                      (int)rows, (int)cols, (const int *)nullptr, 0, lout, counters.p + 1);
         } else {
             prof_units(n_list);
-            if (frozen)
-                MS_LAUNCH(k_minedge_band<true>, cdiv(n_list, 256 * ME_PER_THREAD), 256, 0, s, dem, lab, (const int *)comp,
-                          (const uint8_t *)frozen, best.p, (int)rows, (int)cols, (const int *)lin, n_list, lout, counters.p + 1);
-            else
-                MS_LAUNCH(k_minedge<true>, cdiv(n_list, 256 * ME_PER_THREAD), 256, 0, s, dem, lab, (const int *)comp,
-                          (const uint8_t *)frozen, best.p, (int)rows, (int)cols, (const int *)lin, n_list, lout, counters.p + 1);
+            MS_LAUNCH(k_minedge_band<true>, cdiv(n_list, 256 * ME_PER_THREAD), 256, 0, s, dem, lab, (const int *)comp,
+                      (const uint8_t *)frozen, best.p, (int)rows, (int)cols, (const int *)lin, n_list, lout, counters.p + 1);
         }
         MS_LAUNCH(k_hook, gc, 256, 0, s, best.p, comp, lab, parent.p, wk.p, frozen, nC, (int)cols);
         MS_LAUNCH(k_boruvka_update, gc, 256, 0, s, comp, E, parent.p, wk.p, (const uint8_t *)frozen, nC, best.p,
@@ -529,13 +447,13 @@ static int boruvka_rounds(const float *dem, const int *lab, int *comp, uint32_t 
         n_list = ((int *)h)[1];
         rounds++;
         if (now >= live || rounds > 64) {
-            set_error("%s: Boruvka contraction stalled (%lld -> %lld live components, round %d)", what,
+            set_error("band fill: Boruvka contraction stalled (%lld -> %lld live components, round %d)",
                       (long long)live, (long long)now, rounds);
             return MS_ERR_NOCONV;
         }
         live = now;
         if (live > 0 && n_list == 0) {
-            set_error("%s: live components without an outgoing edge", what);
+            set_error("band fill: live components without an outgoing edge");
             return MS_ERR_NOCONV;
         }
         // the survivors of this round are the next round's work; the second list is sized by the first's count
@@ -543,20 +461,219 @@ static int boruvka_rounds(const float *dem, const int *lab, int *comp, uint32_t 
         lin = lout;
         lout = (lout == listA.p) ? listB.p : listA.p;
     }
-    if (rounds_out) *rounds_out = rounds;
-    if (B) {
-        // the last list: every cell that had a neighbour in another component in the last round (components only
-        // merge, so it is a superset of the cells on the borders between the frozen components)
-        B->n_blist = 0;
-        if (rounds > 0 && n_list > 0) {
-            int *dst = (int *)band_buf(B, BB_BLIST, (size_t)n_list * sizeof(int));
-            if (!dst) return MS_ERR_CUDA;
-            MS_CUDA(cudaMemcpyAsync(dst, lin, (size_t)n_list * sizeof(int), cudaMemcpyDeviceToDevice, s));
-            MS_TRY(ms::stream_sync(s));      // the list buffers go back to the arena when this function returns
-            B->n_blist = n_list;
-        }
+    // the last list: every cell that had a neighbour in another component in the last round (components only
+    // merge, so it is a superset of the cells on the borders between the frozen components)
+    B->n_blist = 0;
+    if (rounds > 0 && n_list > 0) {
+        int *dst = (int *)band_buf(B, BB_BLIST, (size_t)n_list * sizeof(int));
+        if (!dst) return MS_ERR_CUDA;
+        MS_CUDA(cudaMemcpyAsync(dst, lin, (size_t)n_list * sizeof(int), cudaMemcpyDeviceToDevice, s));
+        MS_TRY(ms::stream_sync(s));      // the list buffers go back to the arena when this function returns
+        B->n_blist = n_list;
     }
     return MS_OK;
+}
+
+// ---- single GPU: Boruvka on an explicit catchment edge list -------------------------------------------------------
+// The tile pass numbers the catchments and collects, per 64x64 tile, the lowest cell-pair edge between every pair of
+// catchments that touch inside it (or across its right / lower edge); later rounds work on that list only.  At
+// 32768^2 (fractal DEM) it holds 68.8 M entries for 20.3 M catchments, where the cell-list rounds visited ~650 M
+// boundary cells in round 2 alone; the list and the vertex arrays shrink every round (DESIGN.md §K1).
+constexpr int TE_SLOTS = 1024;       // shared hash slots per tile: a tile of a DEM holds ~80 catchments, white noise ~450
+constexpr int TE_PROBES = 32;        // a candidate that finds no slot within this many goes straight to the global list
+constexpr int TE_LD = FT + 2;        // catchment ids of rows r0 .. r0 + 64, columns c0 - 1 .. c0 + 64
+constexpr int TE_N = (FT + 1) * TE_LD;
+constexpr int TE_LOADS = (TE_N + 255) / 256;
+
+// list entry `pos` = edge (a < b, ordered weight w); Boruvka's key of the entry for both endpoints is (w, pos), a strict
+// total order over the list, so the same pair listed by two tiles cannot form a hook cycle.  Vertex 0 ("outside")
+// does not search.
+__device__ __forceinline__ void edge_put(int *ea, int *eb, uint32_t *ew, unsigned long long *best, int pos, int a, int b,
+                                         uint32_t w) {
+    ea[pos] = a;
+    eb[pos] = b;
+    ew[pos] = w;
+    unsigned long long key = ((unsigned long long)w << 32) | (unsigned)pos;
+    if (a && key < best[a]) atomicMin(&best[a], key);
+    if (key < best[b]) atomicMin(&best[b], key);
+}
+
+__device__ __forceinline__ void tile_edge_insert(unsigned long long *hk, uint32_t *hw, int a, int b, uint32_t w,
+                                                 int *ea, int *eb, uint32_t *ew, int cap, int *n_edges,
+                                                 unsigned long long *best) {
+    unsigned long long key = ((unsigned long long)(unsigned)a << 32) | (unsigned)b;
+    unsigned h = (unsigned)((key * 0x9E3779B97F4A7C15ull) >> 32) & (TE_SLOTS - 1);
+    for (int p = 0; p < TE_PROBES; p++) {
+        unsigned long long cur = hk[h];
+        if (cur == HASH_EMPTY) {
+            unsigned long long old = atomicCAS(hk + h, HASH_EMPTY, key);
+            cur = (old == HASH_EMPTY) ? key : old;
+        }
+        if (cur == key) {
+            atomicMin(hw + h, w);
+            return;
+        }
+        h = (h + 1) & (TE_SLOTS - 1);
+    }
+    int pos = atomicAdd(n_edges, 1);      // table full: unaggregated (counted even past the capacity)
+    if (pos < cap) edge_put(ea, eb, ew, best, pos, a, b, w);
+}
+
+// One CTA per 64x64 tile (the tiling of k_descent_tile, and its TMA box of z).  lab = cid[ptr] for the tile's cells;
+// every cell pair is looked at from its lower cell (directions E, SW, S, SE); a pair of different catchments a < b is
+// an edge of weight max(z_i, z_j) (a = 0: an edge to "outside"), aggregated per pair in shared memory (minimum weight),
+// then appended to the list with one atomic per CTA, which also does round 1's lowest-edge search.  Past `cap` the
+// entries are counted but not written (the caller re-runs the pass with the counted size).
+template <bool TMA>
+__global__ void __launch_bounds__(256) k_tile_edges(const float *__restrict__ z, const int *__restrict__ ptr,
+                                                    const int *__restrict__ cid, int *__restrict__ lab, int rows,
+                                                    int cols, int tiles_x, int *ea, int *eb, uint32_t *ew, int cap,
+                                                    int *n_edges, unsigned long long *best,
+                                                    const __grid_constant__ CUtensorMap zmap) {
+    constexpr int LD = TMA ? DT_LD_TMA : FT + 2;
+    constexpr int X0 = TMA ? DT_X0_TMA : 1;
+    __shared__ __align__(128) float sz[(FT + 2) * LD];
+    __shared__ int sl[TE_N];
+    __shared__ unsigned long long hk[TE_SLOTS];
+    __shared__ uint32_t hw[TE_SLOTS];
+    __shared__ uint64_t bar;
+    int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
+    int r0 = ty * FT, c0 = tx * FT, tid = threadIdx.x;
+    for (int k = tid; k < TE_SLOTS; k += 256) { hk[k] = HASH_EMPTY; hw[k] = 0xffffffffu; }
+    if (TMA) {
+        if (tid == 0) mbar_init(&bar, 1);
+        __syncthreads();
+        if (tid == 0) {
+            mbar_expect_tx(&bar, (unsigned)sizeof(sz));
+            tma_load_2d(sz, &zmap, &bar, c0 - DT_X0_TMA, r0 - 1);
+        }
+    } else {
+        for (int k = tid; k < (FT + 2) * (FT + 2); k += 256) {
+            int lr = k / (FT + 2), lc = k - lr * (FT + 2);
+            int r = r0 + lr - 1, c = c0 + lc - 1;
+            sz[k] = (r >= 0 && r < rows && c >= 0 && c < cols) ? z[(size_t)r * cols + c] : INFINITY;
+        }
+    }
+    // catchment ids while the copy engine brings z: all root pointers first, then their ids
+    int pv[TE_LOADS];
+#pragma unroll
+    for (int u = 0; u < TE_LOADS; u++) {
+        int k = tid + 256 * u, lr = k / TE_LD, lc = k - lr * TE_LD;
+        int r = r0 + lr, c = c0 + lc - 1;
+        pv[u] = (k < TE_N && r < rows && c >= 0 && c < cols) ? __ldg(ptr + (size_t)r * cols + c) : -1;
+    }
+#pragma unroll
+    for (int u = 0; u < TE_LOADS; u++) {
+        int k = tid + 256 * u, lr = k / TE_LD, lc = k - lr * TE_LD;
+        if (k >= TE_N) break;
+        int l = pv[u] >= 0 ? __ldg(cid + pv[u]) : -1;
+        sl[k] = l;
+        if (l >= 0 && lr < FT && lc >= 1 && lc <= FT) lab[(size_t)(r0 + lr) * cols + c0 + lc - 1] = l;
+    }
+    if (TMA) mbar_wait(&bar, 0);
+    __syncthreads();
+    // a thread walks 16 cells down one column: the pairs of a catchment border repeat along it, so consecutive
+    // candidates of the same pair are merged in registers before they reach the table
+    const int lc = tid & 63, lr0 = (tid >> 6) * 16, c = c0 + lc;
+    int pa = -1, pb = -1;
+    uint32_t pw = 0;
+    if (c < cols) {
+        for (int u = 0; u < 16; u++) {
+            const int lr = lr0 + u, r = r0 + lr;
+            if (r >= rows) break;
+            const int l = sl[lr * TE_LD + lc + 1];
+            const float zc = sz[(lr + 1) * LD + lc + X0];
+#pragma unroll
+            for (int d = 0; d < 4; d++) {
+                const int dr = d == 0 ? 0 : 1, dc = d == 0 ? 1 : d - 2;
+                if (r + dr >= rows || c + dc < 0 || c + dc >= cols) continue;
+                const int m = sl[(lr + dr) * TE_LD + lc + 1 + dc];
+                if (m == l) continue;
+                const uint32_t w = okey32(fmaxf(zc, sz[(lr + 1 + dr) * LD + lc + X0 + dc]));
+                const int a = min(l, m), b = max(l, m);
+                if (a == pa && b == pb) { pw = min(pw, w); continue; }
+                if (pa >= 0) tile_edge_insert(hk, hw, pa, pb, pw, ea, eb, ew, cap, n_edges, best);
+                pa = a; pb = b; pw = w;
+            }
+        }
+    }
+    if (pa >= 0) tile_edge_insert(hk, hw, pa, pb, pw, ea, eb, ew, cap, n_edges, best);
+    __syncthreads();
+    int cnt = 0;
+#pragma unroll
+    for (int k = tid; k < TE_SLOTS; k += 256) cnt += hk[k] != HASH_EMPTY;
+    int pos = block_append_pos(cnt, n_edges);
+#pragma unroll
+    for (int k = tid; k < TE_SLOTS; k += 256) {
+        unsigned long long key = hk[k];
+        if (key == HASH_EMPTY) continue;
+        if (pos < cap) edge_put(ea, eb, ew, best, pos, (int)(key >> 32), (int)(key & 0xffffffffu), hw[k]);
+        pos++;
+    }
+}
+
+// every live vertex v != 0 hooks across its lowest edge (mutual pairs keep the smaller id); wk = that edge's weight,
+// flag = 1 for the roots of the new components that have not reached outside
+__global__ void __launch_bounds__(256) k_hook_edges(const unsigned long long *__restrict__ best,
+                                                    const int *__restrict__ ea, const int *__restrict__ eb,
+                                                    int *parent, uint32_t *wk, int *flag, int V) {
+    int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= V) return;
+    int p = v;
+    uint32_t w = okey32(-INFINITY);
+    unsigned long long b = v ? best[v] : KEY_NONE;
+    if (b != KEY_NONE) {
+        unsigned e = (unsigned)(b & 0xffffffffu);
+        int x = ea[e], y = eb[e];
+        int t = (x == v) ? y : x;
+        w = (uint32_t)(b >> 32);
+        if (t != 0 && best[t] == b && v < t) t = v;
+        p = t;
+    }
+    parent[v] = p;
+    wk[v] = w;
+    flag[v] = (v != 0 && p == v) ? 1 : 0;
+}
+
+// the next level's id of v's component (0 = outside); nid = exclusive scan of the live-root flags.  The root is
+// looked up, not stored over parent: another thread's path halving may still overwrite parent[v] with an ancestor.
+__global__ void __launch_bounds__(256) k_level_map(int *parent, const int *__restrict__ nid, int *map, int V) {
+    int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= V) return;
+    int r = uf_find(parent, v);
+    map[v] = r ? nid[r] + 1 : 0;
+}
+
+// endpoints -> next level's ids; an edge inside one component (or between two that reached outside) goes; the rest
+// is compacted and searched for the next round's lowest edges
+__global__ void __launch_bounds__(256) k_edges_relabel(const int *__restrict__ ia, const int *__restrict__ ib,
+                                                       const uint32_t *__restrict__ iw, int m,
+                                                       const int *__restrict__ map, int *oa, int *ob, uint32_t *ow,
+                                                       int *n_out, unsigned long long *best) {
+    int e = blockIdx.x * blockDim.x + threadIdx.x;
+    int a = 0, b = 0;
+    uint32_t w = 0;
+    if (e < m) {
+        a = __ldg(map + ia[e]);
+        b = __ldg(map + ib[e]);
+        w = iw[e];
+        if (a > b) { int t = a; a = b; b = t; }
+    }
+    int keep = a != b;
+    int pos = block_append_pos(keep, n_out);
+    if (keep) edge_put(oa, ob, ow, best, pos, a, b, w);
+}
+
+// spill elevations, top level down: X_t[v] = max(wk_t[v], X_{t+1}[map_t(v)]) unless map_t(v) = 0 (written over wk_t)
+__global__ void __launch_bounds__(256) k_spill_down(uint32_t *wk, const int *__restrict__ map,
+                                                    const uint32_t *__restrict__ x_up, int V) {
+    int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= V) return;
+    int u = map[v];
+    if (u) {
+        uint32_t x = x_up[u];
+        if (x > wk[v]) wk[v] = x;
+    }
 }
 
 int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_t rows, int64_t cols,
@@ -567,32 +684,124 @@ int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_
         return MS_ERR_SHAPE;
     }
     int64_t n = rows * cols;
-    DevBuf<int> lab, tmp;
-    DevBuf<int64_t> total;
+    DevBuf<int> lab, ptr, cid;
+    DevBuf<int64_t> ctr;
     MS_TRY(lab.alloc((size_t)n, s));
-    MS_TRY(tmp.alloc((size_t)n, s));
-    MS_TRY(total.alloc(1, s));
-    dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
-    unsigned g1 = cdiv(n, 256);
+    MS_TRY(ptr.alloc((size_t)n, s));
+    MS_TRY(cid.alloc((size_t)n, s));
+    MS_TRY(ctr.alloc(2, s));
     int64_t *h = host_flags().h;
 
     int64_t jump_rounds = 0;
-    MS_TRY(descent_resolve(dtm, lab.p, tmp.p, rows, cols, 0, &jump_rounds, s));
-    MS_TRY(exclusive_scan_selfptr(lab.p, tmp.p, n, total.p, s));
-    MS_LAUNCH(k_catchment_ids, g1, 256, 0, s, lab.p, tmp.p, n);
-    MS_TRY(ms::readback(h, total.p, sizeof(int64_t), s));
+    MS_TRY(descent_resolve(dtm, ptr.p, cid.p, rows, cols, 0, &jump_rounds, s));
+    MS_TRY(exclusive_scan_selfptr(ptr.p, cid.p, n, ctr.p, s));
+    MS_TRY(ms::readback(h, ctr.p, sizeof(int64_t), s));
     MS_TRY(ms::stream_sync(s));
-    int nC = (int)h[0];
-    tmp.release();
+    const int nC = (int)h[0];
 
-    DevBuf<int> comp;
-    DevBuf<uint32_t> E;
-    MS_TRY(comp.alloc(nC, s));
-    MS_TRY(E.alloc(nC, s));
-    MS_LAUNCH(k_boruvka_init, cdiv(nC, 256), 256, 0, s, comp.p, E.p, nC);
-    int rounds = 0;
-    MS_TRY(boruvka_rounds(dtm, lab.p, comp.p, E.p, nullptr, nC, rows, cols, &rounds, "fill_terrain", s));
-    MS_LAUNCH(k_fill_final, g1, 256, 0, s, dtm, lab.p, E.p, filled, depths, n);
+    // per vertex: the lowest edge and the parent / flags of the current level; wk and map of every level (the live
+    // vertices at least halve per round, so all levels together hold < 2 nC + rounds)
+    const int64_t lv_cap = 2 * (int64_t)nC + 64;
+    DevBuf<unsigned long long> best;
+    DevBuf<int> parent, nid, map_all;
+    DevBuf<uint32_t> wk_all;
+    MS_TRY(best.alloc(nC, s));
+    MS_TRY(parent.alloc(nC, s));
+    MS_TRY(nid.alloc(nC, s));
+    MS_TRY(map_all.alloc((size_t)lv_cap, s));
+    MS_TRY(wk_all.alloc((size_t)lv_cap, s));
+
+    // the edge list takes half of what the arena has left from earlier calls (the other half is for the compacted
+    // copy); when that is too small the pass has counted every edge and runs once more with the counted size plus a
+    // quarter (a tile whose table fills lists some pairs more than once, and how often depends on the timing)
+    const int64_t cap_max = n * 4 < 0x7fffffffll ? n * 4 : 0x7fffffffll;
+    int64_t cap = (int64_t)(arena_room() / (2 * (2 * sizeof(int) + sizeof(uint32_t))));
+    if (cap < n / 16 + 4096) cap = n / 16 + 4096;
+    if (cap > cap_max) cap = cap_max;
+    DevBuf<int> ea[2], eb[2];
+    DevBuf<uint32_t> ew[2];
+    CUtensorMap zmap;
+    memset(&zmap, 0, sizeof(zmap));
+    const bool tma = tma_map_2d(&zmap, dtm, rows, cols, FT + 2, DT_LD_TMA, true, true);
+    const int tiles_x = (int)cdiv(cols, FT), tiles = tiles_x * (int)cdiv(rows, FT);
+    int64_t m = 0;
+    for (int attempt = 0;; attempt++) {
+        MS_TRY(ea[0].alloc((size_t)cap, s));
+        MS_TRY(eb[0].alloc((size_t)cap, s));
+        MS_TRY(ew[0].alloc((size_t)cap, s));
+        MS_CUDA(cudaMemsetAsync(best.p, 0xff, (size_t)nC * sizeof(unsigned long long), s));
+        MS_CUDA(cudaMemsetAsync(ctr.p + 1, 0, sizeof(int64_t), s));
+        prof_units(n);
+        if (tma)
+            MS_LAUNCH(k_tile_edges<true>, tiles, 256, 0, s, dtm, ptr.p, cid.p, lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
+                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap);
+        else
+            MS_LAUNCH(k_tile_edges<false>, tiles, 256, 0, s, dtm, ptr.p, cid.p, lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
+                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap);
+        MS_TRY(ms::readback(h, ctr.p + 1, sizeof(int), s));
+        MS_TRY(ms::stream_sync(s));
+        m = (int64_t)(unsigned)((int *)h)[0];
+        if (m <= cap) break;
+        if (attempt > 0 || cap == cap_max) {
+            set_error("fill_terrain: %lld catchment edges do not fit the list (%lld)", (long long)m, (long long)cap);
+            return MS_ERR_NOCONV;
+        }
+        ew[0].release();
+        eb[0].release();
+        ea[0].release();
+        cap = m + m / 4 < cap_max ? m + m / 4 : cap_max;
+    }
+    cid.release();
+    ptr.release();
+    MS_TRY(ea[1].alloc((size_t)m, s));
+    MS_TRY(eb[1].alloc((size_t)m, s));
+    MS_TRY(ew[1].alloc((size_t)m, s));
+
+    // Boruvka rounds on the list; level t has V vertices (0 = outside), its wk / map at lv_off[t]
+    int64_t lv_off[66];
+    int64_t V = nC, live = nC - 1;
+    int rounds = 0, cur = 0;
+    lv_off[0] = 0;
+    if (live == 0) MS_LAUNCH(k_hook_edges, 1, 256, 0, s, best.p, ea[0].p, eb[0].p, parent.p, wk_all.p, nid.p, (int)V);
+    while (live > 0) {
+        uint32_t *wk = wk_all.p + lv_off[rounds];
+        int *map = map_all.p + lv_off[rounds];
+        unsigned gv = cdiv(V, 256);
+        MS_LAUNCH(k_hook_edges, gv, 256, 0, s, best.p, ea[cur].p, eb[cur].p, parent.p, wk, nid.p, (int)V);
+        MS_TRY(exclusive_scan_i32(nid.p, nid.p, V, ctr.p, s));
+        MS_LAUNCH(k_level_map, gv, 256, 0, s, parent.p, nid.p, map, (int)V);
+        MS_CUDA(cudaMemsetAsync(best.p, 0xff, (size_t)V * sizeof(unsigned long long), s));
+        MS_CUDA(cudaMemsetAsync(ctr.p + 1, 0, sizeof(int64_t), s));
+        prof_units(m);
+        if (m > 0)
+            MS_LAUNCH(k_edges_relabel, cdiv(m, 256), 256, 0, s, ea[cur].p, eb[cur].p, ew[cur].p, (int)m, map, ea[1 - cur].p,
+                      eb[1 - cur].p, ew[1 - cur].p, (int *)(ctr.p + 1), best.p);
+        MS_TRY(ms::readback(h, ctr.p, 2 * sizeof(int64_t), s));
+        MS_TRY(ms::stream_sync(s));
+        int64_t now = h[0];
+        m = (int64_t)((int *)(h + 1))[0];
+        rounds++;
+        lv_off[rounds] = lv_off[rounds - 1] + V;
+        if (now >= live || rounds > 64 || lv_off[rounds] + now + 1 > lv_cap) {
+            set_error("fill_terrain: Boruvka contraction stalled (%lld -> %lld live components, round %d)",
+                      (long long)live, (long long)now, rounds);
+            return MS_ERR_NOCONV;
+        }
+        live = now;
+        if (live > 0 && m == 0) {
+            set_error("fill_terrain: live components without an outgoing edge");
+            return MS_ERR_NOCONV;
+        }
+        V = live + 1;
+        cur = 1 - cur;
+    }
+    // the last level's components all reached outside: X = wk there; E = X_0
+    for (int t = rounds - 2; t >= 0; t--) {
+        int64_t Vt = lv_off[t + 1] - lv_off[t];
+        MS_LAUNCH(k_spill_down, cdiv(Vt, 256), 256, 0, s, wk_all.p + lv_off[t], (const int *)map_all.p + lv_off[t],
+                  (const uint32_t *)wk_all.p + lv_off[t + 1], (int)Vt);
+    }
+    MS_LAUNCH(k_fill_final, cdiv(n, 256), 256, 0, s, dtm, lab.p, wk_all.p, filled, depths, n);
     if (stats) { stats[0] = rounds; stats[1] = nC; stats[5] = jump_rounds; }
     return MS_OK;
 }
@@ -623,8 +832,6 @@ __global__ void __launch_bounds__(256) k_band_edge_ids(const int *__restrict__ l
     top[c] = band_gid(comp[lab[c]], frank, base);
     bot[c] = band_gid(comp[lab[(size_t)(rows - 1) * cols + c]], frank, base);
 }
-
-constexpr unsigned long long HASH_EMPTY = ~0ull;
 
 __device__ inline void edge_insert(unsigned long long *hk, uint32_t *hv, unsigned H, int ga, int gb, uint32_t w,
                                    int *overflow) {
@@ -769,7 +976,7 @@ int fill_band_local(ms_band *B, const float *dem, int64_t *n_frozen, cudaStream_
     unsigned gc = cdiv(nC, 256);
     MS_LAUNCH(k_boruvka_init, gc, 256, 0, s, comp, E, nC);
     MS_CUDA(cudaMemsetAsync(frozen, 0, (size_t)nC, s));
-    MS_TRY(boruvka_rounds(dem, lab, comp, E, frozen, nC, rows, cols, nullptr, "band fill", s, B));
+    MS_TRY(boruvka_rounds_band(dem, lab, comp, E, frozen, nC, rows, cols, s, B));
     // dense ranks of the frozen component roots
     MS_LAUNCH(k_frozen_flags, gc, 256, 0, s, comp, frozen, frank, nC);
     MS_TRY(exclusive_scan_i32(frank, frank, nC, total.p, s));
