@@ -425,6 +425,32 @@ int ms_polygonize(const int32_t *labels, int64_t rows, int64_t cols, int connect
 int ms_polygonize_fetch(int64_t *ring_vertex_offset, int32_t *ring_value, int64_t *ring_cell, int64_t *ring_region,
                         uint8_t *ring_hole, int32_t *vertex_row, int32_t *vertex_col);
 
+/* ---- Bluespot water levels and water-depth rasters after rain events.
+ * Bluespot l >= 1 is the set of cells with labels == l; z = dem widened to float64, F = the plain fill (uniform over
+ * a bluespot: L_l), ca = cell_area > 0, cap_l = st_sum[l] * ca, v = the stored volume of a bluespot per event
+ * (e.g. the `v` of ms_rain_events / ms_bluespot_network_dev), row-major [n_events][nlabels+1].
+ * Level-pool approximation: a bluespot's water is one flat surface at level h holding ca * sum max(0, h - z_c); this
+ * ignores that separate sub-pits of one bluespot may fill one after another.
+ * ms_flood_levels: level[e][l] and wet[e][l] (cells with z < level), both [n_events][nlabels+1]:
+ *   v NaN -> NaN, 0;  v >= cap_l -> L_l, #cells of l;  otherwise, with z_(1) <= ... <= z_(n) the bluespot's values,
+ *   S_j = z_(1) + ... + z_(j), T = v / ca and k = max{ j : j * z_(j) - S_j <= T }: h = min(L_l, (T + S_k) / k),
+ *   wet = #{ z_c < h };  label 0 -> NaN, 0.  Results are bitwise reproducible.  MS_ERR_ARG for bad sizes, null
+ *   pointers or cell_area <= 0 (before any device work), for a label whose F is not uniform and for a negative v;
+ *   MS_ERR_LABEL for a label outside [0, nlabels].
+ * ms_water_depth: the depth raster of one event's levels (nlabels+1 entries): level_l == L_l -> F - z in float32
+ *   (bitwise the `depths` raster of the fill); z < level_l -> (float)(level_l - z) from float64; 0 elsewhere and
+ *   outside bluespots.  MS_ERR_LABEL for a label outside [0, nlabels]. */
+int ms_flood_levels_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                        int64_t nlabels, const double *st_sum, double cell_area, int64_t n_events, const double *v,
+                        double *out_level, int64_t *out_wet, void *stream);
+int ms_flood_levels(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                    int64_t nlabels, const double *st_sum, double cell_area, int64_t n_events, const double *v,
+                    double *out_level, int64_t *out_wet);
+int ms_water_depth_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                       int64_t nlabels, const double *level, float *out_depth, void *stream);
+int ms_water_depth(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                   int64_t nlabels, const double *level, float *out_depth);
+
 #ifdef __cplusplus
 }
 #endif

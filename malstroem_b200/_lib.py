@@ -122,6 +122,10 @@ SIGNATURES = {
     "ms_polygonize": (c_int, [c_p, c_i64, c_i64, c_int, c_int, ctypes.c_int32, c_p]),
     "ms_polygonize_fetch": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_bluespot_network_dev": (c_int, [c_p, c_dbl, c_int, c_i64, c_p, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ms_flood_levels_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_dbl, c_i64, c_p, c_p, c_p, c_p]),
+    "ms_flood_levels": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_dbl, c_i64, c_p, c_p, c_p]),
+    "ms_water_depth_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p, c_p]),
+    "ms_water_depth": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p]),
 }
 
 

@@ -183,6 +183,11 @@ __device__ inline int d8_border(int code, bool top, bool bot, int c, int cols) {
 int exclusive_scan_i32(const int *flags, int *out, int64_t n, int64_t *total_dev, cudaStream_t s);
 // the same over the flags "ptr[i] == i" (roots of a parent-pointer array); out must not alias ptr
 int exclusive_scan_selfptr(const int *ptr, int *out, int64_t n, int64_t *total_dev, cudaStream_t s);
+// stable LSD sort of int (key, val) pairs on key bits [0, bits), one binary split per bit (network.cu: the network's
+// upstream lists, flood.cu's large segments).  The passes ping-pong between the buffers; on return *key / *val point
+// at the sorted pairs and *key_alt / *val_alt at the other pair of buffers.  flag: n ints of scratch.
+int radix_sort_split(int **key, int **val, int **key_alt, int **val_alt, int *flag, int64_t *total, int n, int bits,
+                     cudaStream_t s);
 // pointer jumping on a forest given as parent indices (roots point to themselves); in place.
 // rounds_out (host, optional) receives the number of rounds.  MS_ERR_NOCONV after 64 rounds (cycles).
 int forest_resolve(int *ptr, int64_t n, int64_t *rounds_out, cudaStream_t s);

@@ -59,6 +59,19 @@ __global__ void __launch_bounds__(256) k_net_split(const int *__restrict__ key, 
     val_out[dst] = val[i];
 }
 
+int radix_sort_split(int **key, int **val, int **key_alt, int **val_alt, int *flag, int64_t *total, int n, int bits,
+                     cudaStream_t s) {
+    unsigned g = cdiv(n, 256);
+    for (int b = 0; b < bits; b++) {
+        MS_LAUNCH(k_net_bitflag, g, 256, 0, s, *key, n, b, flag);
+        MS_TRY(exclusive_scan_i32(flag, flag, n, total, s));
+        MS_LAUNCH(k_net_split, g, 256, 0, s, *key, *val, flag, total, n, b, *key_alt, *val_alt);
+        int *t = *key; *key = *key_alt; *key_alt = t;
+        t = *val; *val = *val_alt; *val_alt = t;
+    }
+    return MS_OK;
+}
+
 __global__ void __launch_bounds__(256) k_net_present_ptr(const int32_t *__restrict__ parent, int n, int *ptr) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) ptr[i] = parent[i] >= 0 ? parent[i] : i;
@@ -158,13 +171,7 @@ int rain_events_dev_impl(int64_t n64, const int32_t *parent, const double *area,
     int bits = 1;
     while ((1ll << bits) <= n) bits++;                      // keys are 0..n
     int *ka = key.p, *va = val.p, *kb = key2.p, *vb = val2.p;
-    for (int b = 0; b < bits; b++) {
-        MS_LAUNCH(k_net_bitflag, g, 256, 0, s, ka, n, b, flag.p);
-        MS_TRY(exclusive_scan_i32(flag.p, flag.p, n, total.p, s));
-        MS_LAUNCH(k_net_split, g, 256, 0, s, ka, va, flag.p, total.p, n, b, kb, vb);
-        int *t = ka; ka = kb; kb = t;
-        t = va; va = vb; vb = t;
-    }
+    MS_TRY(radix_sort_split(&ka, &va, &kb, &vb, flag.p, total.p, n, bits, s));
     MS_LAUNCH(k_net_fill_nan, cdiv((int64_t)n * ne, 256), 256, 0, s, rainv, spillv, v, pctv, (int64_t)n * ne);
     int64_t *h = host_flags().h;
     MS_TRY(ms::readback(h, bad.p, sizeof(int), s));

@@ -109,6 +109,46 @@ class RasterPipeline(object):
                 ctypes.c_void_p(stream)), "ms_bluespot_network_dev")
         return res
 
+    # ---- water levels and depth rasters after the rain events (csrc/flood.cu) -------------------------
+    def flood(self, net, cell_area):
+        """Water level and wet-cell count of every bluespot per event of `net` (the dict `network()` returned, with
+        the same cell_area), device resident: dict of cuda tensors `level` float64 and `wet` int64 [n_events,
+        nlabels+1].  Level-pool approximation, see malstroem_b200.flood."""
+        v = net["v"].contiguous()
+        n = self.nlabels + 1
+        if v.dim() != 2 or v.shape[1] != n or v.dtype != torch.float64 or v.device != self.device:
+            raise ValueError("flood: net['v'] must be a float64 tensor [n_events, %d] on %s" % (n, self.device))
+        ne = int(v.shape[0])
+        res = {"level": torch.empty((ne, n), dtype=torch.float64, device=self.device),
+               "wet": torch.empty((ne, n), dtype=torch.int64, device=self.device)}
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with _lib.lock:
+            _lib.check(_lib.lib().ms_flood_levels_dev(
+                self.dem.data_ptr(), self.out["filled"].data_ptr(), self.out["labels"].data_ptr(), self.rows,
+                self.cols, self.nlabels, self.tables["st_sum"].data_ptr(), float(cell_area), ne, v.data_ptr(),
+                res["level"].data_ptr(), res["wet"].data_ptr(), ctypes.c_void_p(stream)), "ms_flood_levels_dev")
+        return res
+
+    def water_depth(self, level_row, out=None):
+        """Water depth raster (cuda float32, rows x cols) of one event: `level_row` is one row of flood()'s `level`.
+        Rasters are made one event at a time: at 32768^2 each is 4 GB."""
+        n = self.nlabels + 1
+        level_row = level_row.contiguous()
+        if level_row.shape != (n,) or level_row.dtype != torch.float64 or level_row.device != self.device:
+            raise ValueError("water_depth: level_row must be a float64 tensor [%d] on %s" % (n, self.device))
+        if out is None:
+            out = torch.empty((self.rows, self.cols), dtype=torch.float32, device=self.device)
+        elif (out.shape != (self.rows, self.cols) or out.dtype != torch.float32 or not out.is_contiguous()
+              or out.device != self.device):
+            raise ValueError("water_depth: out must be a contiguous float32 tensor of the raster's shape on %s" % self.device)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with _lib.lock:
+            _lib.check(_lib.lib().ms_water_depth_dev(
+                self.dem.data_ptr(), self.out["filled"].data_ptr(), self.out["labels"].data_ptr(), self.rows,
+                self.cols, self.nlabels, level_row.data_ptr(), out.data_ptr(), ctypes.c_void_p(stream)),
+                "ms_water_depth_dev")
+        return out
+
     # ---- host-buffer run (bench `e2e`): H2D of the DEM, the run, D2H of every raster + table ---------
     def host_rasters(self):
         return [k for k in self.out if k in self.HOST_RASTERS or (k == "fnf" and self.host_fnf)]
