@@ -213,17 +213,16 @@ int ms_band_nf_p2p_solve_dev(ms_band *band, const float *filled, double *fnf, do
  * (seed or raster border) of the band's first / last own row (cols bytes each) - the caller hands them to the
  * neighbours, whose halo rows they describe.  prepare: the band's padded int32 distance raster, its edge rows stored
  * into the neighbours' mailboxes (peer memory), FIFO := tiles holding lake cells; *queued, *irbad (the band does not
- * fit the integer form).  All ranks synchronise, ms_band_nf_p2p_arm_dev, synchronise, solve (all ranks at once).
- * finish: the float64 surface written once and verified against the fixed-point equation with the halo rows
- * (*nviol), the D8 codes of the band's rows (flow.py:142-167, edges of the raster flowing outward) on the way. */
+ * fit the integer form).  All ranks synchronise, ms_band_nf_p2p_arm_dev, synchronise, solve (all ranks at once):
+ * solve_launch returns once the solver kernel is queued, and the host is free for CPU work until solve_wait (no
+ * library call on this band in between).  finish: the float64 surface written once and verified against the
+ * fixed-point equation with the halo rows (*nviol), the D8 codes of the band's rows (flow.py:142-167, edges of the
+ * raster flowing outward) on the way. */
 int ms_band_nf_ir_edgefix_dev(ms_band *band, const float *dem, const float *filled, uint8_t *fix_top, uint8_t *fix_bot,
                               void *stream);
 int ms_band_nf_ir_prepare_dev(ms_band *band, const float *dem, const float *filled, double short_eps, double diag_eps,
                               double cap_bound, const uint8_t *fix_top, const uint8_t *fix_bot, int64_t *queued,
                               int *irbad, void *stream);
-int ms_band_nf_ir_solve_dev(ms_band *band, const float *filled, double short_eps, double diag_eps, int64_t *tile_visits,
-                            int *irbad, void *stream);
-/* solve = launch + wait; between the two the host is free for CPU work (no library call on this band) */
 int ms_band_nf_ir_solve_launch_dev(ms_band *band, const float *filled, double short_eps, double diag_eps, void *stream);
 int ms_band_nf_ir_solve_wait_dev(ms_band *band, int64_t *tile_visits, int *irbad, void *stream);
 int ms_band_nf_ir_finish_dev(ms_band *band, const float *dem, const float *filled, double *fnf, uint8_t *flowdir,
@@ -268,14 +267,6 @@ int ms_band_ws_local_dev(ms_band *band, const uint8_t *flowdir, const int32_t *l
 int ms_chain_resolve_dev(int64_t n, const int32_t *arr, int32_t *out, void *stream);
 int ms_band_ws_finish_dev(ms_band *band, const uint8_t *flowdir, int32_t *labelled, int32_t unassigned,
                           const int32_t *exit_label, void *stream);
-
-/* label.label_min_index / label_max_index (label.py:101-166) in two phases whose tables combine across bands with
- * min / max all-reduces: the extreme value per label, then the smallest global flat index holding it
- * (INT64_MAX: label not seen). */
-int ms_band_extreme_value_dev(const double *data, const int32_t *labels, int64_t n, int64_t nlabels, int want_max,
-                              double *out_value, void *stream);
-int ms_band_extreme_index_dev(const double *data, const int32_t *labels, int64_t n, int64_t nlabels,
-                              const double *value, int64_t cell_offset, int64_t *out_index, void *stream);
 
 /* All per-label tables of a band in two fused passes over its rasters.  Phase A: partial label_stats(depths, labels),
  * label_count(wsheds) and the extreme values of fnf (min) / accum (max) per label, +-inf where the band does not see

@@ -83,7 +83,6 @@ SIGNATURES = {
     "ms_band_nf_p2p_solve_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_dbl, c_p, c_p]),
     "ms_band_nf_ir_edgefix_dev": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_band_nf_ir_prepare_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_dbl, c_p, c_p, c_p, c_p, c_p]),
-    "ms_band_nf_ir_solve_dev": (c_int, [c_p, c_p, c_dbl, c_dbl, c_p, c_p, c_p]),
     "ms_band_nf_ir_solve_launch_dev": (c_int, [c_p, c_p, c_dbl, c_dbl, c_p]),
     "ms_band_nf_ir_solve_wait_dev": (c_int, [c_p, c_p, c_p, c_p]),
     "ms_band_nf_ir_finish_dev": (c_int, [c_p, c_p, c_p, c_p, c_p, c_dbl, c_dbl, c_p, c_p]),
@@ -99,8 +98,6 @@ SIGNATURES = {
     "ms_band_ws_local_dev": (c_int, [c_p, c_p, c_p, ctypes.c_int32, c_p, c_p, c_p]),
     "ms_chain_resolve_dev": (c_int, [c_i64, c_p, c_p, c_p]),
     "ms_band_ws_finish_dev": (c_int, [c_p, c_p, c_p, ctypes.c_int32, c_p, c_p]),
-    "ms_band_extreme_value_dev": (c_int, [c_p, c_p, c_i64, c_i64, c_int, c_p, c_p]),
-    "ms_band_extreme_index_dev": (c_int, [c_p, c_p, c_i64, c_i64, c_p, c_i64, c_p, c_p]),
     "ms_band_tables_a_dev": (c_int, [c_p, c_p, c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_band_tables_b_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_p, c_p, c_i64, c_p, c_p, c_p]),
     "ms_pipeline_dev": (c_int, [c_p, c_p]),

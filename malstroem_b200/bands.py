@@ -345,7 +345,7 @@ class BandPipeline(object):
         self._tick("minmax")
         # K5/K6 phase 1 (needs the depths only): its host-side merge then overlaps the no-flats solver kernel
         self._cc_allr = None
-        if self.p2p and os.environ.get("MS_BAND_OVERLAP", "1") != "0":
+        if self.p2p:
             self._labels_local(st)
             self._tick("labels_local")
         # K2 no-flats fill
@@ -365,19 +365,8 @@ class BandPipeline(object):
         self._labels(st)
         ship(("labels",))
         self._tick("labels")
-        if os.environ.get("MS_BAND_FUSED_TABLES", "1") == "0":
-            self._stats(st)
-            self._tick("stats")
-            # K7 watersheds, K10 counts
-            self._watersheds(st)
-            ship(("wsheds",))
-            self._tick("watersheds")
-            # K8'/K8'' pour points
-            self._pour_points(st)
-            self._tick("pour_points")
-            return self
         # K7 watersheds, then every per-label table (K8, K10, K8', K8'') in two fused passes and three all-reduces
-        self._watersheds(st, count=False)
+        self._watersheds(st)
         ship(("wsheds",))
         self._tick("watersheds")
         self._tables(st)
@@ -385,12 +374,11 @@ class BandPipeline(object):
         return self
 
     def _noflats(self, st):
-        import os
         comm, dev, cols = self.comm, self.device, self.cols
         fnf = self.ext["fnf"]
         i64 = ctypes.c_int64
         self._flowdir_done = False
-        if self.p2p and os.environ.get("MS_BAND_IR", "1") != "0" and self._noflats_ir(st):
+        if self.p2p and self._noflats_ir(st):
             return
         if self.p2p and self._noflats_p2p(st):
             return
@@ -616,27 +604,6 @@ class BandPipeline(object):
                    label_offset, _p(self.out["labels"]), st)
         self.stats["cc_boundary_roots"] = int(k.value)
 
-    def _table(self, name, dtype):
-        t = torch.empty(self.nlabels + 1, dtype=dtype, device=self.device)
-        self.tables[name] = t
-        return t
-
-    def _stats(self, st):
-        comm, n = self.comm, self.rows * self.cols
-        tmin, tmax, tsum = (self._table(k, torch.float64) for k in ("st_min", "st_max", "st_sum"))
-        tcnt = self._table("st_count", torch.int64)
-        self._call("ms_label_stats_dev", _p(self.out["depths"]), _lib.MS_F32, _p(self.out["labels"]), n, self.nlabels,
-                   _p(tmin), _p(tmax), _p(tsum), _p(tcnt), st)
-        m = self.nlabels + 1
-        lohi = torch.cat([tmin, -tmax])                      # max(x) = -min(-x): one reduction for both
-        comm.all_reduce(lohi, "min")
-        tmin.copy_(lohi[:m])
-        tmax.copy_(-lohi[m:])
-        sums = torch.cat([tsum, tcnt.double()])              # counts < 2^53: exact in float64
-        comm.all_reduce(sums, "sum")
-        tsum.copy_(sums[:m])
-        tcnt.copy_(sums[m:].round().long())
-
     def _tables(self, st):
         """label_stats(depths, labels), label_count(wsheds), label_min_index(fnf, labels), label_max_index(accum,
         labels) (bluespots.py:160-205) for the whole raster, complete on every rank."""
@@ -669,7 +636,7 @@ class BandPipeline(object):
             t[key + "_row"] = rows_[k * m:(k + 1) * m]
             t[key + "_col"] = cols_[k * m:(k + 1) * m]
 
-    def _watersheds(self, st, count=True):
+    def _watersheds(self, st):
         comm, dev, cols = self.comm, self.device, self.cols
         G, g = comm.size, comm.rank
         ws = self.out["wsheds"]
@@ -685,33 +652,6 @@ class BandPipeline(object):
         node, ok = exit_targets(all_to, cols, g)
         exit_label = torch.where(ok, final[node.clamp(0, arr.numel() - 1)], torch.zeros_like(final[:1])).to(torch.int32)
         self._call("ms_band_ws_finish_dev", self.h, _p(self.out["flowdir"]), _p(ws), 0, _p(exit_label.contiguous()), st)
-        if not count:
-            return
-        cnt = self._table("ws_count", torch.int64)
-        self._call("ms_label_count_dev", _p(ws), self.rows * cols, self.nlabels + 1, _p(cnt), st)
-        comm.all_reduce(cnt, "sum")
-
-    def _pour_points(self, st):
-        comm, n, cols, m = self.comm, self.rows * self.cols, self.cols, self.nlabels + 1
-        keys = (("ppmin", self.out["fnf"], 0), ("ppmax", self.out["accum"], 1))
-        vals = torch.empty(2 * m, dtype=torch.float64, device=self.device)
-        for k, (key, data, want_max) in enumerate(keys):
-            self._call("ms_band_extreme_value_dev", _p(data), _p(self.out["labels"]), n, self.nlabels, want_max,
-                       _p(vals[k * m:]), st)
-        vals[m:].neg_()                                      # max(x) = -min(-x): one reduction for both tables
-        comm.all_reduce(vals, "min")
-        vals[m:].neg_()
-        idx = torch.empty(2 * m, dtype=torch.int64, device=self.device)
-        for k, (key, data, want_max) in enumerate(keys):
-            self._call("ms_band_extreme_index_dev", _p(data), _p(self.out["labels"]), n, self.nlabels, _p(vals[k * m:]),
-                       self.cell_offset, _p(idx[k * m:]), st)
-        comm.all_reduce(idx, "min")
-        none = idx == torch.iinfo(torch.int64).max
-        rows_, cols_ = torch.where(none, torch.full_like(idx, -1), idx // cols), torch.where(none, torch.full_like(idx, -1), idx % cols)
-        for k, (key, data, want_max) in enumerate(keys):
-            self.tables[key + "_value"] = vals[k * m:(k + 1) * m]
-            self.tables[key + "_row"] = rows_[k * m:(k + 1) * m]
-            self.tables[key + "_col"] = cols_[k * m:(k + 1) * m]
 
     # ---- the bluespot network and rain events on the finished tables (SURVEY.md §8(f1,f2)) -----------------------
     def network(self, cell_area=1.0, events_mm=(), use_accum_pourpoints=False, sum_mode=None):

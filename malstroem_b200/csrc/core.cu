@@ -138,9 +138,7 @@ __global__ void k_readback(const uint32_t *__restrict__ src, uint32_t *dst_host,
 }
 
 int readback(void *host_pinned, const void *dev, size_t bytes, cudaStream_t s) {
-    static int mode = -1;       // MS_READBACK=copy: the copy engine, as before
-    if (mode < 0) { const char *e = getenv("MS_READBACK"); mode = (e && e[0] == 'c') ? 0 : 1; }
-    if (!mode || (bytes & 3) || bytes > 4096 || ((uintptr_t)dev & 3) || ((uintptr_t)host_pinned & 3)) {
+    if ((bytes & 3) || bytes > 4096 || ((uintptr_t)dev & 3) || ((uintptr_t)host_pinned & 3)) {
         MS_CUDA(cudaMemcpyAsync(host_pinned, dev, bytes, cudaMemcpyDeviceToHost, s));
         return MS_OK;
     }
@@ -203,16 +201,13 @@ bool tma_map_2d(CUtensorMap *out, const void *base, int64_t rows, int64_t cols, 
                 bool nan_fill) {
     if (!g_encode_tried) {
         g_encode_tried = 1;
-        const char *e = getenv("MS_TMA");
-        if (!(e && e[0] == '0')) {
-            void *fn = nullptr;
-            cudaDriverEntryPointQueryResult q;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
-                q == cudaDriverEntryPointSuccess)
-                g_encode = (EncodeTiledFn)fn;
-            else
-                cudaGetLastError();
-        }
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
+            q == cudaDriverEntryPointSuccess)
+            g_encode = (EncodeTiledFn)fn;
+        else
+            cudaGetLastError();
     }
     if (getenv("MS_TMA_DEBUG") && !g_encode) fprintf(stderr, "tma_map_2d: no cuTensorMapEncodeTiled entry point\n");
     if (!g_encode || ((uintptr_t)base & 15) || (cols & 3) || ((box_cols * 4) & 15) || box_rows > 256 || box_cols > 256 ||

@@ -666,119 +666,17 @@ int label_extreme_dev_impl(const double *data, const int32_t *lab, int64_t rows,
 // The per-label tables of the whole path in two passes (device-resident pipeline only; the numpy-level functions
 // keep their one-table kernels above).  BluespotTool asks for label_stats(depths, labels), label_count(wsheds),
 // label_min_index(fnf, labels) and label_max_index(accum, labels) (bluespots.py:160-205): five rasters, the labels
-// read four times.  Pass A reads every raster once — depth min / max / sum / count, the extreme keys of the no-flats
-// surface and of the accumulation per bluespot (warp-aggregated: lanes of one label grouped with match.any, one lane
-// issues the atomics; label 0 stays in registers) and the watershed histogram.  Pass B finds the smallest flat index
-// holding each extreme (raster-order tie-break, label.py:101-166) for both tables at once.
+// read four times.  Pass A (k_tables_a2) reads every raster once — depth min / max / sum / count, the extreme keys of
+// the no-flats surface and of the accumulation per bluespot and the watershed histogram.  Pass B (k_tables_b) finds
+// the smallest flat index holding each extreme (raster-order tie-break, label.py:101-166) for both tables at once.
 // 28 + 20 B/cell instead of 8 + 4 + 12 + 12 + 12 + 12.
 // ------------------------------------------------------------------------------------------------
-template <bool ACC>
-__global__ void __launch_bounds__(256) k_tables_a(const float *__restrict__ depths, const int32_t *__restrict__ lab,
-                                                  const double *__restrict__ fnf, const double *__restrict__ accum,
-                                                  const int32_t *__restrict__ ws, int64_t n, int64_t nlabels,
-                                                  uint32_t *tmin, uint32_t *tmax, double *tsum,
-                                                  unsigned long long *tcnt, unsigned long long *kmin,
-                                                  unsigned long long *kmax, unsigned long long *wcnt, int *err) {
-    const unsigned full = 0xffffffffu;
-    uint32_t bmin = 0xffffffffu, bmax = 0;
-    double bsum = 0.0;
-    unsigned long long bcnt = 0, bwz = 0, bkmin = ~0ull, bkmax = 0ull;
-    int64_t span = (int64_t)gridDim.x * blockDim.x;
-    int64_t nround = (n + span - 1) / span;
-    for (int64_t it = 0; it < nround; it++) {
-        int64_t i = it * span + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-        int lbl = -1, w = -1;
-        float v = 0.f;
-        double f = 0.0, a = 0.0;
-        if (i < n) {
-            lbl = lab[i];
-            w = ws[i];
-            v = depths[i];
-            f = fnf[i];
-            if (ACC) a = accum[i];
-            if (lbl < 0 || lbl > nlabels) { *err = 1; lbl = -1; }
-            if (w < 0 || w > nlabels) { *err = 1; w = -1; }
-        }
-        const bool vok = (v == v), fok = (f == f), aok = (a == a);
-        const unsigned long long fk = fok ? okey64(f) : ~0ull, ak = aok ? okey64(a) : 0ull;
-        if (lbl == 0) {
-            uint32_t k = okey32(v);
-            if (vok) { bmin = k < bmin ? k : bmin; bmax = k > bmax ? k : bmax; }
-            bsum += (double)v;
-            bcnt++;
-            bkmin = fk < bkmin ? fk : bkmin;
-            if (ACC) bkmax = ak > bkmax ? ak : bkmax;
-        }
-        if (w == 0) bwz++;
-        unsigned act = __ballot_sync(full, lbl > 0);
-        if (lbl > 0) {
-            unsigned g = __match_any_sync(act, lbl);
-            uint32_t k = okey32(vok ? v : 0.f);
-            uint32_t kmn = grp_min(g, vok ? k : 0xffffffffu);
-            uint32_t kmx = grp_max(g, vok ? k : 0u);
-            double sm = grp_sum(g, (double)v);
-            unsigned long long gfk = grp_min(g, fk);
-            unsigned long long gak = ACC ? grp_max(g, ak) : 0ull;
-            if ((int)(__ffs(g) - 1) == (int)(threadIdx.x & 31)) {
-                if (kmn < tmin[lbl]) atomicMin(tmin + lbl, kmn);
-                if (kmx > tmax[lbl]) atomicMax(tmax + lbl, kmx);
-                atomicAdd(tsum + lbl, sm);
-                atomicAdd(tcnt + lbl, (unsigned long long)__popc(g));
-                if (gfk < kmin[lbl]) atomicMin(kmin + lbl, gfk);
-                if (ACC && gak > kmax[lbl]) atomicMax(kmax + lbl, gak);
-            }
-        }
-        unsigned actw = __ballot_sync(full, w > 0);
-        if (w > 0) {
-            unsigned g = __match_any_sync(actw, w);
-            if ((int)(__ffs(g) - 1) == (int)(threadIdx.x & 31)) atomicAdd(wcnt + w, (unsigned long long)__popc(g));
-        }
-    }
-    // CTA reduction of the label-0 accumulators
-    uint32_t wmin = grp_min(full, bmin), wmax = grp_max(full, bmax);
-    unsigned long long wkmin = grp_min(full, bkmin), wkmax = grp_max(full, bkmax);
-    double wsum = bsum;
-    unsigned long long wc = bcnt, wz = bwz;
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        wsum += __shfl_xor_sync(full, wsum, o);
-        wc += __shfl_xor_sync(full, wc, o);
-        wz += __shfl_xor_sync(full, wz, o);
-    }
-    __shared__ uint32_t smin[8], smax[8];
-    __shared__ double ssum[8];
-    __shared__ unsigned long long scnt[8], swz[8], skmin[8], skmax[8];
-    int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-    if (lane == 0) { smin[wp] = wmin; smax[wp] = wmax; ssum[wp] = wsum; scnt[wp] = wc; swz[wp] = wz; skmin[wp] = wkmin; skmax[wp] = wkmax; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int k = 1; k < 8; k++) {
-            wmin = smin[k] < wmin ? smin[k] : wmin;
-            wmax = smax[k] > wmax ? smax[k] : wmax;
-            wsum += ssum[k];
-            wc += scnt[k];
-            wz += swz[k];
-            wkmin = skmin[k] < wkmin ? skmin[k] : wkmin;
-            wkmax = skmax[k] > wkmax ? skmax[k] : wkmax;
-        }
-        if (wc) {
-            atomicMin(tmin, wmin);
-            atomicMax(tmax, wmax);
-            atomicAdd(tsum, wsum);
-            atomicAdd(tcnt, wc);
-            atomicMin(kmin, wkmin);
-            if (ACC) atomicMax(kmax, wkmax);
-        }
-        if (wz) atomicAdd(wcnt, wz);
-    }
-}
-
-// Pass A, tile form: one CTA per 64 x 64 tile, a thread walks 16 consecutive cells of a tile row.  Bluespots and
-// watersheds are blobs, so a thread sees runs of one label: it keeps the run's partial results in registers and folds
-// a finished run into a small shared-memory table keyed by label (open addressing, 256 slots; a tile holds a few dozen
-// labels), and the table goes to the global per-label tables with one set of atomics per label and tile - instead of
-// one warp-aggregated set per label and 32 cells (k_tables_a above: 21.6 ms at 32768^2, 54 % issue-bound on the
-// match / group-reduction instructions).  Label 0 stays in registers as before.
+// Pass A: one CTA per 64 x 64 tile, a thread walks 16 consecutive cells of a tile row.  Bluespots and watersheds are
+// blobs, so a thread sees runs of one label: it keeps the run's partial results in registers and folds a finished run
+// into a small shared-memory table keyed by label (open addressing, 256 slots; a tile holds a few dozen labels), and
+// the table goes to the global per-label tables with one set of atomics per label and tile - instead of one
+// warp-aggregated set per label and 32 cells (measured: 21.6 ms at 32768^2, 54 % issue-bound on the match /
+// group-reduction instructions).  Label 0 stays in registers.
 constexpr int TA_SLOTS = 256;
 template <bool ACC>
 __global__ void __launch_bounds__(256) k_tables_a2(const float *__restrict__ depths, const int32_t *__restrict__ lab,
@@ -1051,8 +949,8 @@ __global__ void __launch_bounds__(256) k_idx_global(const int *__restrict__ tidx
 
 extern "C" {
 
-/* The per-label tables of a band in two fused passes (k_tables_a / k_tables_b; see pipeline_tables_dev_impl).  Phase
- * A: the band's partial stats, watershed histogram and extreme values (float64, +-inf where the band does not see a
+/* The per-label tables of a band in two fused passes (k_tables_a2 / k_tables_b; see pipeline_tables_dev_impl).
+ * Phase A: the band's partial stats, watershed histogram and extreme values (float64, +-inf where the band does not see a
  * label) — combine across bands with min / max / sum all-reduces.  Phase B: with the GLOBAL extremes, the smallest
  * global flat index holding each (INT64_MAX: not in this band) — combine with a min all-reduce. */
 int ms_band_tables_a_dev(const float *depths, const int32_t *labels, const double *fnf, const double *accum,
@@ -1084,10 +982,7 @@ int ms_band_tables_a_dev(const float *depths, const int32_t *labels, const doubl
     MS_LAUNCH(k_fill_u64, gm, 256, 0, s, kmin.p, ~0ull, scratch.p, INT32_MAX, m);
     MS_LAUNCH(k_fill_u64, gm, 256, 0, s, kmax.p, 0ull, scratch.p, INT32_MAX, m);
     MS_CUDA(cudaMemsetAsync(ws_count, 0, (size_t)m * sizeof(int64_t), s));
-    int64_t want = (n + 255) / 256;
-    int blocks = (int)(want > 148 * 16 ? 148 * 16 : want);
     prof_units(n);
-    (void)blocks;
     const int64_t rows = n / cols;
     const int tiles_x = (int)cdiv(cols, 64), ntiles = tiles_x * (int)cdiv(rows, 64);
     MS_LAUNCH(k_tables_a2<true>, ntiles, 256, 0, s, depths, labels, fnf, accum, wsheds, (int)rows, (int)cols, tiles_x, nlabels,
@@ -1124,54 +1019,6 @@ int ms_band_tables_b_dev(const int32_t *labels, const double *fnf, const double 
     MS_LAUNCH(k_tables_b<true>, blocks, 256, 0, s, labels, fnf, accum, n, nlabels, kmin.p, kmax.p, imin.p, imax.p);
     MS_LAUNCH(k_idx_global, gm, 256, 0, s, imin.p, cell_offset, idx_min, m);
     MS_LAUNCH(k_idx_global, gm, 256, 0, s, imax.p, cell_offset, idx_max, m);
-    return MS_OK;
-}
-
-}  // extern "C"
-
-
-extern "C" {
-
-int ms_band_extreme_value_dev(const double *data, const int32_t *labels, int64_t n, int64_t nlabels, int want_max,
-                              double *out_value, void *stream) {
-    using namespace ms;
-    MS_TRY(ensure_init());
-    if (!data || !labels || !out_value || n < 1 || nlabels < 0) { set_error("band label_min/max_index: bad argument"); return MS_ERR_ARG; }
-    cudaStream_t s = (cudaStream_t)stream;
-    int64_t m = nlabels + 1;
-    DevBuf<unsigned long long> tkey;
-    DevBuf<int> tidx, err;
-    MS_TRY(tkey.alloc((size_t)m, s));
-    MS_TRY(tidx.alloc((size_t)m, s));
-    MS_TRY(err.alloc(1, s));
-    MS_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), s));
-    unsigned gm = cdiv(m, 256);
-    MS_LAUNCH(k_fill_u64, gm, 256, 0, s, tkey.p, want_max ? 0ull : ~0ull, tidx.p, INT32_MAX, m);
-    int64_t want = (n + 255) / 256;
-    int blocks = (int)(want > 148 * 16 ? 148 * 16 : want);
-    if (want_max) MS_LAUNCH(k_extreme_key<true>, blocks, 256, 0, s, data, labels, n, nlabels, tkey.p, err.p);
-    else MS_LAUNCH(k_extreme_key<false>, blocks, 256, 0, s, data, labels, n, nlabels, tkey.p, err.p);
-    MS_LAUNCH(k_key_to_val, gm, 256, 0, s, tkey.p, out_value, m, want_max);
-    return MS_OK;
-}
-
-int ms_band_extreme_index_dev(const double *data, const int32_t *labels, int64_t n, int64_t nlabels,
-                              const double *value, int64_t cell_offset, int64_t *out_index, void *stream) {
-    using namespace ms;
-    MS_TRY(ensure_init());
-    if (!data || !labels || !value || !out_index || n < 1 || nlabels < 0) { set_error("band label_min/max_index: bad argument"); return MS_ERR_ARG; }
-    cudaStream_t s = (cudaStream_t)stream;
-    int64_t m = nlabels + 1;
-    DevBuf<unsigned long long> tkey;
-    DevBuf<int> tidx;
-    MS_TRY(tkey.alloc((size_t)m, s));
-    MS_TRY(tidx.alloc((size_t)m, s));
-    unsigned gm = cdiv(m, 256);
-    MS_LAUNCH(k_val_to_key, gm, 256, 0, s, value, tkey.p, tidx.p, m);
-    int64_t want = (n + 255) / 256;
-    int blocks = (int)(want > 148 * 16 ? 148 * 16 : want);
-    MS_LAUNCH(k_extreme_index, blocks, 256, 0, s, data, labels, n, nlabels, tkey.p, tidx.p);
-    MS_LAUNCH(k_idx_global, gm, 256, 0, s, tidx.p, cell_offset, out_index, m);
     return MS_OK;
 }
 

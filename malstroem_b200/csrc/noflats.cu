@@ -49,16 +49,6 @@ constexpr int NF_T = 64;             // tile edge
 constexpr int NF_LD = NF_T + 3;      // shared row stride in doubles (odd: spreads the rows of a block over banks)
 constexpr int NF_SMEM = (NF_T + 2) * NF_LD * 8 + NF_T * NF_T * 4;
 constexpr int NF_BLOCK_ITERS = 64;   // in-block iteration guard (a block that hits it stays dirty)
-// Forwarding a tile's ring to its neighbours before the tile has settled (after iterations 1, 2, 4, ... or after
-// every iteration) was measured at 8192^2: the kernel is throughput-bound for two thirds of its run (every CTA slot
-// busy, profiles/r01_nf_timeline.txt), so the extra visits cost more than the shorter chains save (11.1 ms -> 12.9 /
-// 13.8 ms).  Kept behind these switches, off.
-#ifndef NF_FLUSH_ALWAYS
-#define NF_FLUSH_ALWAYS 0
-#endif
-#ifndef NF_MIDFLUSH
-#define NF_MIDFLUSH 0
-#endif
 
 #ifdef NF_STATS
 __device__ unsigned long long g_nf_dbg[16];
@@ -280,7 +270,6 @@ struct NfTileShared {
     int ring;          // bit 0/1/2/3: the tile's top / bottom / left / right ring changed
     int nb;            // neighbour tiles to queue: bit (dy+1)*3 + (dx+1)
     int grab[3];       // next dirty block to hand out (per iteration, rotating like `dirty`)
-    int midflush;      // forward ring changes before the tile has settled (only while CTAs are idle)
     unsigned char blist[64];   // the dirty blocks of the current iteration
     int2 wtab[NF_NBIN];
     int k;             // ticket
@@ -305,8 +294,11 @@ __device__ inline unsigned long long nf_region(int flags) {
 // Runs the dirty-block iteration of one tile to quiescence.  On entry S.dirty[0] holds the initial mask,
 // S.dirty[1] = S.dirty[2] = S.chgmask = 0, S.ring = 0, all visible (a __syncthreads() has passed).
 // `flush()` (called by all threads right after a __syncthreads) writes the blocks in S.chgmask back, queues the
-// neighbours that can gain from the changed ring, and clears S.chgmask / S.ring.  It is called at the end (and,
-// with NF_MIDFLUSH, while the tile is still settling).
+// neighbours that can gain from the changed ring, and clears S.chgmask / S.ring.  It is called once, when the tile
+// has settled.  Forwarding the ring before that (after iterations 1, 2, 4, ... or after every iteration) was
+// measured at 8192^2: the kernel is throughput-bound for two thirds of its run (every CTA slot busy,
+// profiles/r01_nf_timeline.txt), so the extra visits cost more than the shorter chains save (11.1 ms -> 12.9 /
+// 13.8 ms).
 template <class R, class F>
 __device__ inline int nf_tile_iterate(const R &rx, NfTileShared &S, F &flush) {
     const int tid = threadIdx.x, lane = tid & 31;
@@ -352,7 +344,6 @@ __device__ inline int nf_tile_iterate(const R &rx, NfTileShared &S, F &flush) {
             if (rings) atomicOr(&S.ring, rings);
         }
         __syncthreads();
-        if (S.midflush && S.ring && (NF_FLUSH_ALWAYS || ((it + 1) & it) == 0)) flush();
     }
     if (S.chgmask) flush();
     return it;
@@ -454,6 +445,33 @@ __device__ inline void nf_push(int *ring, int cap, NfCtl *ctl, int tile, bool sy
     *slot = tile;
 }
 
+// take the next FIFO entry (one thread of a solver CTA): wait for it to be filled unless all work is done, and free
+// the slot.  Returns the tile, or -1 when the solve has ended.
+__device__ __forceinline__ int nf_take(int *ring, int cap, NfCtl *ctl, bool p2p, const NfP2P *pp) {
+    unsigned my = atomicAdd(&ctl->head, 1u);
+    volatile int *slot = ring + (my % (unsigned)cap);
+    int t = -1;
+    const unsigned long long t_start = nf_globaltimer();
+    for (unsigned spins = 0;; spins++) {
+        t = *slot;
+        if (t >= 0) break;
+        if (*(volatile int *)&ctl->done) break;
+        __nanosleep(100);
+        // watchdog on the wall clock (never hang the GPU): generous, so that a profiler or a time-sliced GPU
+        // does not trip it
+        if ((spins & 1023u) == 1023u && nf_globaltimer() - t_start > NF_WATCHDOG_NS) {
+            if (p2p) for (int k = 0; k < pp->world; k++) *(volatile int *)pp->done_all[k] = 2;      // every rank stops
+            atomicExch(&ctl->done, 2);
+            break;
+        }
+    }
+    if (t >= 0) {
+        *slot = -1;
+        __threadfence();
+    }
+    return t;
+}
+
 // converts one loaded row pair of the integer form (cells 2*lane, 2*lane+1 and, for lanes 0/1, an apron column)
 struct NfRowRegs {
     double w0, w1, wa;
@@ -463,7 +481,7 @@ struct NfRowRegs {
 template <bool CAP>
 __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ zsrc, double *W, int *ring, int cap,
                                                   int *tileflag, const int *__restrict__ tilesides, NfCtl *ctl, int rows, int cols, int tiles_x,
-                                                  int tiles_y, double sh, double dg, int use_int, double capB_in,
+                                                  int tiles_y, double sh, double dg, int use_int, double capB,
                                                   int open, const NfP2P *pp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double *sw = reinterpret_cast<double *>(smem_raw);
@@ -473,7 +491,6 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
     float *sfi = reinterpret_cast<float *>(se + NF_T * NF_T);        // integer form: F per interior cell (write-back)
     __shared__ NfTileShared S;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const double capB = CAP ? (capB_in >= 0 ? capB_in : ((double)ctl->nonseed + 16.0) * dg * 1.001) : 0.0;
     // rows the aprons may read: a band that continues above / below has a halo row there
     const int rlo = (open & 1) ? -1 : 0, rhi = rows + ((open & 2) ? 1 : 0);
     const bool p2p = pp != nullptr;
@@ -486,20 +503,8 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
         // The next tile is taken by thread 32 while thread 0 is still signing off the previous one (below): both are
         // chains of global atomics, and nobody touches S between the barrier that ends a visit and this point.
         if (tid == 32) {
-            // take the next FIFO entry; wait for it to be filled unless all work is done
-            unsigned my = atomicAdd(&ctl->head, 1u);
-            volatile int *slot = ring + (my % (unsigned)cap);
-            int t = -1;
-            for (unsigned spins = 0;; spins++) {
-                t = *slot;
-                if (t >= 0) break;
-                if (*(volatile int *)&ctl->done) break;
-                __nanosleep(200);
-                if (spins > (1u << 23)) { atomicExch(&ctl->done, 2); break; }      // watchdog (~2 s): never hang the GPU
-            }
+            const int t = nf_take(ring, cap, ctl, p2p, pp);
             if (t >= 0) {
-                *slot = -1;
-                __threadfence();
                 // taken: while the tile runs, neighbours only leave their side bits; they are looked at when it ends
                 S.flags = (p2p ? atomicExch_system(tileflag + t, NF_RUNNING) : atomicExch(tileflag + t, NF_RUNNING)) & NF_SIDES;
                 S.dirty[1] = 0;
@@ -508,8 +513,6 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
                 S.ring = 0;
                 S.nb = 0;
                 S.grab[0] = S.grab[1] = S.grab[2] = 0;
-                // NF_MIDFLUSH 1: always; 2: only while fewer tiles are queued or running than there are CTAs
-                S.midflush = NF_MIDFLUSH == 1 || (NF_MIDFLUSH == 2 && *(volatile int *)&ctl->pending < (int)gridDim.x);
                 S.e = INT_MIN;
                 S.elo = INT_MAX;
                 S.bad = 0;
@@ -1087,24 +1090,13 @@ __global__ void __launch_bounds__(256) k_nf_verify(const float *__restrict__ z, 
 // with the one direction that reads that side.
 constexpr int IR_LD = NF_T + 3;                 // 67: odd
 constexpr int IR_SMEM = (NF_T + 2) * IR_LD * 4 + NF_T * NF_T;
-#ifndef IR_NT
-#define IR_NT 128
-#endif
-#ifndef IR_CTAS
-#define IR_CTAS 6
-#endif
-#ifndef IR_UNCOND
-#define IR_UNCOND 1
-#endif
-#ifndef IR_MIDFLUSH
-#define IR_MIDFLUSH 1
-#endif
-#ifndef IR_MID_SHIFT
-#define IR_MID_SHIFT 2        // tail mode (edges forwarded after the first round) below grid >> IR_MID_SHIFT queued or running tiles
+constexpr int IR_NT = 128;
+constexpr int IR_CTAS = 6;
+// tail mode (edges forwarded after the first round) below grid >> IR_TAIL_SHIFT queued or running tiles
 // (measured: shift 0 / 1 / 2 / 3 -> 3.15 / 3.21 / 3.42 / 3.47 ms at 8192^2, 38.8 / 38.8 / 38.6 / 38.8 ms at 32768^2; on two
 // bands of 4096 / 16384 rows shift 0 gives 6.6 / 29.5 ms against 7.0 / 29.0: it helps where the tail dominates and costs
-// where the bulk does - left at 2)
-#endif
+// where the bulk does)
+constexpr int IR_TAIL_SHIFT = 2;
 
 // the wall frame of the padded raster: row 0, the rows below the tiles, and 4 columns either side of every tile row
 // (k_nf_init_tile writes everything inside, including the cells of edge tiles that lie beyond the raster)
@@ -1139,11 +1131,6 @@ struct IrShared {
 
 // One sweep of the tile in direction `dir` (0 top->bottom, 1 bottom->top, 2 left->right, 3 right->left) by one warp.
 // Cell (line, k) of the sweep sits at sd[org + line * SL + k * SK]; lines and k run -1..64 (apron included).
-__device__ __forceinline__ void ir_red_min(int *p, int v, bool pred) {
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.s32 q, %2, 0;\n\t@q red.shared.min.s32 [%0], %1;\n\t}"
-                 :: "r"((unsigned)__cvta_generic_to_shared(p)), "r"(v), "r"((int)pred) : "memory");
-}
-
 // `start`: first position (in sweep order: position p is line p of a forward sweep, line 63 - p of a backward one) to
 // relax; `lastext`: from this position on the sweep stops at the first line it does not change (everything that
 // could disturb the lines beyond lies behind it).
@@ -1203,19 +1190,11 @@ __device__ __forceinline__ void ir_sweep(int *sd, const unsigned char *se, IrSha
         // lane without an improvement reduces with INT_MAX): ptxas wraps a conditional ATOMS into a divergent branch
         // region, which costs more than the reduction (measured at 8192^2 / 32768^2: 4.03 / 41.5 ms against 4.46 / 43.8;
         // plain predicated stores with the sweeps restarted on the first changed line: 4.07 / 42.0 and more rounds)
-#if IR_UNCOND
         // (tried and dropped: skipping the two reductions on lines no lane improves - a vote and a uniform branch per
         // step - and plain stores when only one direction sweeps: 3.37 -> 4.00 ms at 8192^2, 38.6 -> 45.1 ms at 32768^2;
         // the branch costs the step more scheduling freedom than the reductions cost LSU time)
         atomicMin(pa, chA ? candA : 0x7fffffff);
         atomicMin(pb, chB ? candB : 0x7fffffff);
-#elif IR_PLAIN
-        if (chA) *pa = candA;
-        if (chB) *pb = candB;
-#else
-        ir_red_min(pa, candA, chA);
-        ir_red_min(pb, candB, chB);
-#endif
         hist = (hist << 1) | (unsigned long long)(chA | chB);
         everA |= chA;
         everB |= chB;
@@ -1270,26 +1249,8 @@ __global__ void __launch_bounds__(IR_NT, IR_CTAS) k_nf_solve_ir(const float *__r
     for (;;) {
         // thread 32 takes the next tile while thread 0 still signs off the previous one
         if (tid == 32) {
-            unsigned my = atomicAdd(&ctl->head, 1u);
-            volatile int *slot = ring + (my % (unsigned)cap);
-            int t = -1;
-            const unsigned long long t_start = nf_globaltimer();
-            for (unsigned spins = 0;; spins++) {
-                t = *slot;
-                if (t >= 0) break;
-                if (*(volatile int *)&ctl->done) break;
-                __nanosleep(100);
-                // watchdog on the wall clock (never hang the GPU): generous, so that a profiler or a time-sliced GPU
-                // does not trip it
-                if ((spins & 1023u) == 1023u && nf_globaltimer() - t_start > NF_WATCHDOG_NS) {
-                    if (p2p) for (int k = 0; k < pp->world; k++) *(volatile int *)pp->done_all[k] = 2;      // every rank stops
-                    atomicExch(&ctl->done, 2);
-                    break;
-                }
-            }
+            const int t = nf_take(ring, cap, ctl, p2p, pp);
             if (t >= 0) {
-                *slot = -1;
-                __threadfence();
                 S.flags = (p2p ? atomicExch_system(tileflag + t, NF_RUNNING) : atomicExch(tileflag + t, NF_RUNNING)) & NF_SIDES;
                 S.ring = 0;
                 S.nb = 0;
@@ -1302,7 +1263,7 @@ __global__ void __launch_bounds__(IR_NT, IR_CTAS) k_nf_solve_ir(const float *__r
                 S.elo = (int)(short)(meta & 0xffff);
                 S.e = S.elo + ((meta >> 16) & 15);
                 S.has = (meta >> 20) & 1;
-                S.mid = IR_MIDFLUSH && *(volatile int *)&ctl->pending < (int)(gridDim.x >> IR_MID_SHIFT);
+                S.mid = *(volatile int *)&ctl->pending < (int)(gridDim.x >> IR_TAIL_SHIFT);
                 atomicAdd(&ctl->visits, 1);
             }
             S.k = t;
@@ -1493,11 +1454,7 @@ __global__ void __launch_bounds__(IR_NT, IR_CTAS) k_nf_solve_ir(const float *__r
                         if (rnd > 0) {
                             unsigned long long m = warp < 2 ? mrow : mcol;
                             if (warp & 1) m = __brevll(m);
-#if IR_PLAIN
-                            start = __ffsll((long long)m) - 1;           // the first changed position itself (see ir_sweep)
-#else
                             start = __ffsll((long long)m);               // first changed position + 1 (m != 0 here)
-#endif
                             lastext = 64 - __clzll((long long)m);        // ... up to the one after the last changed one
                         }
                         if (start < NF_T) {
@@ -1714,7 +1671,7 @@ template <bool CAP>
 static int nf_launch_solve(const float *zsrc, double *W, int *ring, int cap, int *tileflag, const int *tilesides,
                            NfCtl *ctl, int rows,
                            int cols, int tiles_x, int tiles_y, int ntiles, double sh, double dg, int use_int,
-                           double capB_in, int open, int64_t units, cudaStream_t s, const NfP2P *pp = nullptr) {
+                           double capB, int open, int64_t units, cudaStream_t s, const NfP2P *pp = nullptr) {
     static int grid_blocks = 0;
     if (!grid_blocks) {
         MS_CUDA(cudaFuncSetAttribute(k_nf_solve<CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, NF_SMEM));
@@ -1728,7 +1685,7 @@ static int nf_launch_solve(const float *zsrc, double *W, int *ring, int cap, int
     void *args[] = {(void *)&zsrc, (void *)&W, (void *)&ring, (void *)&cap, (void *)&tileflag, (void *)&tilesides,
                     (void *)&ctl,
                     (void *)&rows, (void *)&cols, (void *)&tiles_x, (void *)&tiles_y, (void *)&sh, (void *)&dg,
-                    (void *)&use_int, (void *)&capB_in, (void *)&open, (void *)&pp};
+                    (void *)&use_int, (void *)&capB, (void *)&open, (void *)&pp};
     // consumers wait on the FIFO, so every CTA must be resident: cooperative launch guarantees it (or fails)
     int g = (grid_blocks < ntiles || pp) ? grid_blocks : ntiles;
     prof_units(units);
@@ -1742,8 +1699,6 @@ static int nf_launch_solve(const float *zsrc, double *W, int *ring, int cap, int
     }
     return MS_OK;
 }
-
-int g_nf_ir = 1;           // MS_NF_IR=0 keeps the W-based solver (k_nf_solve) on the single-GPU capped path
 
 static int nf_launch_solve_ir(const float *F, int *Dg, int P, int *ring, int cap, int *tileflag, const int *tilesides,
                               const int *tmeta, NfCtl *ctl, int *irbad, int rows, int cols, int tiles_x, int tiles_y,
@@ -1799,8 +1754,6 @@ int fill_no_flats_dev_impl(const float *dtm, const float *filled, double sh, dou
     if (!env_done) {
         const char *e = getenv("MS_NF_INT");
         if (e && e[0] == '0') g_nf_use_int = 0;
-        e = getenv("MS_NF_IR");
-        if (e && e[0] == '0') g_nf_ir = 0;
         env_done = true;
     }
     int tiles_x = (int)cdiv(cols, NF_T), tiles_y = (int)cdiv(rows, NF_T);
@@ -1816,7 +1769,7 @@ int fill_no_flats_dev_impl(const float *dtm, const float *filled, double sh, dou
     bool cap = sh > 0 && dg > 0;      // capped fast path first; a verification failure falls back to the generic one
     const double cap_bound = ms_nf_cap_bound(rows, cols, dg);
     // integer-raster form of the capped solve: padded int32 raster (see k_nf_solve_ir)
-    bool use_ir = cap && g_nf_use_int && g_nf_ir;
+    bool use_ir = cap && g_nf_use_int;
     const int P = tiles_x * NF_T + 8;
     const size_t dg_cells = (size_t)P * ((size_t)tiles_y * NF_T + 2);
     DevBuf<int> Dg, tmeta, irbad;
@@ -1869,7 +1822,7 @@ int fill_no_flats_dev_impl(const float *dtm, const float *filled, double sh, dou
                                          tiles_y, ntiles, sh, dg, g_nf_use_int, cap_bound, 0, n, s));
         } else {
             MS_TRY(nf_launch_solve<false>(dtm, out, ring.p, cap_ring, tileflag.p, tilesides.p, ctl.p, (int)rows, (int)cols, tiles_x,
-                                          tiles_y, ntiles, sh, dg, 0, -1.0, 0, n, s));
+                                          tiles_y, ntiles, sh, dg, 0, 0.0, 0, n, s));
         }
         if (!ir) MS_LAUNCH(k_nf_verify, g2, 256, 0, s, dtm, out, banned.p, ctl.p, (int)rows, (int)cols, sh, dg, 0);
         MS_TRY(ms::readback(h, ctl.p, sizeof(NfCtl), s));
@@ -2030,7 +1983,7 @@ int ms_band_nf_solve_dev(ms_band *B, const float *dem, const float *filled, doub
                                      B->open, B->rows * B->cols, s));
     else
         MS_TRY(nf_launch_solve<false>(dem, fnf, nb.ring, nb.cap_ring, nb.tileflag, nb.tilesides, nb.ctl, rows, cols,
-                                      nb.tiles_x, nb.tiles_y, nb.ntiles, short_eps, diag_eps, 0, -1.0, B->open,
+                                      nb.tiles_x, nb.tiles_y, nb.ntiles, short_eps, diag_eps, 0, 0.0, B->open,
                                       B->rows * B->cols, s));
     NfCtl *h = (NfCtl *)(host_flags().h + 32);
     MS_TRY(ms::readback(h, nb.ctl, sizeof(NfCtl), s));
@@ -2250,7 +2203,7 @@ int ms_band_nf_p2p_solve_dev(ms_band *B, const float *filled, double *fnf, doubl
  *    rows stored into the neighbours' mailboxes, FIFO := tiles with lake cells.  *queued = tiles queued, *irbad = the
  *    band does not fit the integer form.  The caller synchronises all ranks, then ms_band_nf_p2p_arm_dev, synchronises
  *    again, then
- * 3. ms_band_nf_ir_solve_dev: every band's k_nf_solve_ir at once; ends when no band has work left.
+ * 3. ms_band_nf_ir_solve_launch_dev / _wait_dev: every band's k_nf_solve_ir at once; ends when no band has work left.
  * 4. ms_band_nf_ir_finish_dev: W = F + D ulp(F) written once, verified against the fixed-point equation with the
  *    halo rows (*nviol), D8 codes of the band's rows written on the way (K3 fused, edges of the RASTER flow outward). */
 int ms_band_nf_ir_edgefix_dev(ms_band *B, const float *dem, const float *filled, uint8_t *fix_top, uint8_t *fix_bot,
@@ -2348,12 +2301,6 @@ int ms_band_nf_ir_solve_wait_dev(ms_band *B, int64_t *tile_visits, int *irbad_ou
         return MS_ERR_NOCONV;
     }
     return MS_OK;
-}
-
-int ms_band_nf_ir_solve_dev(ms_band *B, const float *filled, double short_eps, double diag_eps, int64_t *tile_visits,
-                            int *irbad_out, void *stream) {
-    MS_TRY(ms_band_nf_ir_solve_launch_dev(B, filled, short_eps, diag_eps, stream));
-    return ms_band_nf_ir_solve_wait_dev(B, tile_visits, irbad_out, stream);
 }
 
 int ms_band_nf_ir_finish_dev(ms_band *B, const float *dem, const float *filled, double *fnf, uint8_t *flowdir,

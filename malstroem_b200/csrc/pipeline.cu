@@ -157,7 +157,7 @@ extern "C" int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, voi
                   (long long)io->table_capacity);
         return MS_ERR_ARG;
     }
-    // every table asked for (the usual case): two fused passes over the rasters (labels.cu: k_tables_a / k_tables_b)
+    // every table asked for (the usual case): two fused passes over the rasters (labels.cu: k_tables_a2 / k_tables_b)
     const bool fused = io->st_min && io->st_max && io->st_sum && io->st_count && io->ws_count && io->ppmin_value &&
                        io->ppmin_row && io->ppmin_col;
     if (io->st_min && !fused)
