@@ -228,6 +228,9 @@ void *band_buf(ms_band *b, int slot, size_t bytes);      // grow-only cudaMalloc
 // pointer jumping restricted to the cells in `list` (device, n_list entries): every other cell already points at its
 // root or at a listed cell.  Used after a tile-local compression (k_descent_tile, k_ws_tile).
 int forest_resolve_list(int *ptr, const int *list, int n_list, int64_t *rounds_out, cudaStream_t s);
+// the same for the fill's catchment ids (k_descent_tile): lab[i] >= 0 is an id, lab[i] < 0 a link to cell -(1 + lab[i]);
+// only the cells in `list` hold links.  Afterwards every listed cell holds an id.
+int forest_resolve_ids(int *lab, const int *list, int n_list, int64_t *rounds_out, cudaStream_t s);
 
 #ifdef __CUDACC__
 // ---- tile-local pointer compression (64x64 tiles, 256 threads, 16 cells per thread) -----------------------------
@@ -301,7 +304,8 @@ struct HostCall {
 void poly_release();
 
 // internal device-pointer stage entry points used by the pipeline (pipeline.cu)
+// minmax_out (optional, 2 floats on the device): min / max of dtm, as minmax_dev computes them
 int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_t rows, int64_t cols,
-                          int64_t *stats, cudaStream_t s);
+                          int64_t *stats, cudaStream_t s, float *minmax_out = nullptr);
 
 }  // namespace ms

@@ -6,21 +6,21 @@
 // min/max of input values are involved, so any algorithm that reaches the fixed point is bit-exact.
 //
 //   1. k_descent_tile every interior cell points at the smallest cell of its 3x3 window in the strict
-//                     total order (z, flat index); border cells point at cell 0 ("outside"); in-tile paths are
-//                     compressed in shared memory
-//   2. forest_resolve_list  pointer jumping for the cells whose path leaves their tile -> every cell knows the
-//                     local minimum ("catchment") it drains to
-//   3. scan           dense catchment ids (0 = outside), straight from the root pointers
-//   4. Boruvka on the catchment graph (edge weight = max(z_a, z_b) over adjacent cells of two catchments).
-//                     One CTA per tile (k_tile_edges) writes the catchment ids and the catchment-pair edge list,
-//                     aggregated per tile, and finds every catchment's lowest edge (64-bit atomicMin of (weight,
-//                     list position)).  Each round every live component hooks across its lowest edge and records
-//                     that weight (wk); the roots that have not reached "outside" get dense new ids, and the edges
-//                     are relabelled, those inside one component dropped, the rest compacted and searched for the
-//                     next round's lowest edges.  After the last round E = max of wk over the levels of the
+//                     total order (z, flat index); border cells drain to "outside" (id 0); the local minima
+//                     ("catchments") get dense ids in tile order (a decoupled look-back over the per-tile counts);
+//                     in-tile paths are compressed in shared memory
+//   2. forest_resolve_ids  pointer jumping for the cells whose path leaves their tile -> every cell holds the id of
+//                     the catchment it drains to
+//   3. Boruvka on the catchment graph (edge weight = max(z_a, z_b) over adjacent cells of two catchments).
+//                     One CTA per tile (k_tile_edges) writes the catchment-pair edge list, aggregated per tile, and
+//                     finds every catchment's lowest edge (64-bit atomicMin of (weight, list position)).  Each
+//                     round every live component hooks across its lowest edge and records that weight (wk); the
+//                     roots that have not reached "outside" get dense new ids, and the edges are relabelled, those
+//                     inside one component dropped, the rest compacted and searched for the next round's lowest
+//                     edges.  After the last round E = max of wk over the levels of the
 //                     catchment's component until it reaches outside (k_spill_down, top level first).
 //                     Claim (DESIGN.md §K1): E is the catchment's spill elevation.
-//   5. k_fill_final   filled = max(z, E[catchment]), depths = filled - z
+//   4. k_fill_final   filled = max(z, E[catchment]), depths = filled - z
 #include <string.h>
 
 #include "common.cuh"
@@ -87,33 +87,81 @@ int minmax_dev(const float *z, int64_t n, float *out2, cudaStream_t s) {
 }
 
 // ---- K1 -------------------------------------------------------------------------------------------
+// Catchment numbering in tile order: the local minima of tile T get the ids base(T) + 1 .. base(T) + count(T), where
+// base(T) is the number of local minima in the tiles before T (0 = "outside").  base comes from a single-pass
+// decoupled look-back over one status word per tile: flag in the high half, catchment count in the low half, so that
+// one load reads both.  TS_AGG: the tile's own count; TS_INCL: the count of the tile and every tile before it.
+constexpr unsigned long long TS_AGG = 1ull << 32, TS_INCL = 2ull << 32;
+
+__device__ __forceinline__ void st_release_u64(unsigned long long *p, unsigned long long v) {
+    asm volatile("st.release.gpu.global.b64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long *p) {
+    unsigned long long v;
+    asm volatile("ld.acquire.gpu.global.b64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+// one full warp: catchments of the tiles before `tile`.  Every tile before it has taken its ticket (so it runs) and
+// publishes its TS_AGG word before it waits for anything, so the wait ends.
+__device__ int tile_lookback(const unsigned long long *status, int tile) {
+    const int lane = threadIdx.x & 31;
+    int excl = 0;
+    for (int end = tile - 1; end >= 0; end -= 32) {
+        const int j = end - lane;
+        unsigned long long st;
+        for (;;) {
+            st = j >= 0 ? ld_acquire_u64(status + j) : TS_INCL;
+            if (__all_sync(0xffffffffu, (st >> 32) != 0)) break;
+        }
+        const unsigned incl = __ballot_sync(0xffffffffu, (st >> 32) == 2);
+        // the nearest inclusive word ends the look-back: add it and the aggregates after it
+        int v = (int)(unsigned)st;
+        if (incl && lane > __ffs(incl) - 1) v = 0;
+        excl += __reduce_add_sync(0xffffffffu, v);
+        if (incl) break;
+    }
+    return excl;
+}
+
 // `open` (row bands): bit 0 / 1 = the first / last row is not the raster border but continues in another band; its
 // cells are ordinary cells whose window is clipped to the band (a catchment never crosses a band edge).
-// Descent pointers + most of the pointer jumping: a CTA holds a 64x64 tile of z (+ apron) in shared memory,
-// finds every cell's pointer, compresses the in-tile paths by pointer doubling, and writes for every cell the
-// GLOBAL index its tile-local root stands for: itself (a local minimum), 0 (raster border = "outside"), or - when
-// the root's lowest neighbour lies in another tile - that neighbour.  Only cells of the last kind still need global
-// pointer jumping; they are appended to `list` (catchments are ~50 cells, so that is a small fraction).
+// Descent pointers + most of the pointer jumping: a CTA holds a 64x64 tile of z (+ apron) in shared memory, finds
+// every cell's pointer, numbers the tile's local minima, compresses the in-tile paths by pointer doubling, and writes
+// for every cell what its tile-local root stands for: the catchment id of a local minimum, 0 (raster border =
+// "outside"), or - when the root's lowest neighbour lies in another tile - -(1 + that neighbour's index).  Only cells
+// of the last kind still need global pointer jumping (forest_resolve_ids); they are appended to `list` (catchments
+// are ~50 cells, so that is a small fraction).  The tile index comes from a ticket (`ticket`, zeroed), not from
+// blockIdx, so that every tile before it has started: the look-back waits for them.
+// mm_keys (optional, {okey32 max, 0} on entry): K0's min / max keys of the raster, reduced from the z tile.
 // TMA = true: the tile + apron comes in with ONE cp.async.bulk.tensor.2d issued by thread 0 - a 66 x 72 box starting at
 // column c0 - 4 (the innermost box coordinate and width must be multiples of 16 bytes: measured with tools/tma_probe.cu,
 // a start at c0 - 1 raises an illegal-instruction fault); cells outside the raster arrive as NaN, which no comparison
 // below selects - the same effect as the +inf the LDG -> STS form stores for them.
 constexpr int DT_LD_TMA = FT + 8, DT_X0_TMA = 4;
 template <bool TMA>
-__global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ z, int *__restrict__ ptr, int rows,
+__global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ z, int *__restrict__ lab, int rows,
                                                       int cols, int tiles_x, int open, int *list, int *n_list,
+                                                      unsigned long long *status, int *ticket, uint32_t *mm_keys,
                                                       const __grid_constant__ CUtensorMap zmap) {
     constexpr int LD = TMA ? DT_LD_TMA : FT + 2;
     constexpr int X0 = TMA ? DT_X0_TMA : 1;          // shared column of the tile's first cell
     __shared__ __align__(128) float sz[(FT + 2) * LD];
     __shared__ unsigned short sp[FT * FT];
-    __shared__ int tgt[FT * FT];          // per tile-local root: >= 0 final global index, < 0: -(1 + cell in another tile)
+    __shared__ int tgt[FT * FT];          // per tile-local root: > 0 catchment rank in the tile, 0 outside, < 0: -(1 + cell in another tile)
     __shared__ uint64_t bar;
-    int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
-    int r0 = ty * FT, c0 = tx * FT, tid = threadIdx.x;
+    __shared__ int tile_s, base_s, wcnt[8];
+    __shared__ uint32_t wlo[8], whi[8];
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    if (tid == 0) {
+        tile_s = atomicAdd(ticket, 1);
+        if (TMA) mbar_init(&bar, 1);
+    }
+    __syncthreads();
+    const int tile = tile_s;
+    const int ty = tile / tiles_x, tx = tile - ty * tiles_x;
+    const int r0 = ty * FT, c0 = tx * FT;
     if (TMA) {
-        if (tid == 0) mbar_init(&bar, 1);
-        __syncthreads();
         if (tid == 0) {
             mbar_expect_tx(&bar, (unsigned)sizeof(sz));
             tma_load_2d(sz, &zmap, &bar, c0 - DT_X0_TMA, r0 - 1);
@@ -127,6 +175,8 @@ __global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ 
         }
         __syncthreads();
     }
+    unsigned minbits = 0;                 // which of this thread's cells are local minima
+    uint32_t klo = 0xffffffffu, khi = 0u;
 #pragma unroll 4
     for (int u = 0; u < 16; u++) {
         int k = tid + 256 * u;
@@ -136,10 +186,13 @@ __global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ 
         int t = 0;
         if (r < rows && c < cols) {
             int i = r * cols + c;
+            float bz = sz[(lr + 1) * LD + lc + X0];
+            uint32_t key = okey32(bz);
+            klo = min(klo, key);
+            khi = max(khi, key);
             if ((r == 0 && !(open & 1)) || c == 0 || (r == rows - 1 && !(open & 2)) || c == cols - 1) {
-                t = 0;                                   // raster border: points at "outside" (cell 0)
+                t = 0;                                   // raster border: "outside"
             } else {
-                float bz = sz[(lr + 1) * LD + lc + X0];
                 int bi = i, bdr = 0, bdc = 0;
 #pragma unroll
                 for (int dr = -1; dr <= 1; dr++)
@@ -152,7 +205,7 @@ __global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ 
                         if (zj < bz || (zj == bz && j < bi)) { bz = zj; bi = j; bdr = dr; bdc = dc; }
                     }
                 int tr = lr + bdr, tc = lc + bdc;
-                if (bi == i) t = i;                                           // local minimum
+                if (bi == i) minbits |= 1u << u;                              // local minimum (ranked below)
                 else if (tr >= 0 && tr < FT && tc >= 0 && tc < FT) p = (unsigned short)(tr * FT + tc);
                 else t = -(1 + bi);                                           // lowest neighbour is in another tile
             }
@@ -160,9 +213,49 @@ __global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ 
         sp[k] = p;
         tgt[k] = t;
     }
+    // rank of the tile's local minima: (warp, lane, cell) order
+    const int cnt = __popc(minbits);
+    int inc = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        int y = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += y;
+    }
+    if (mm_keys) {
+        klo = __reduce_min_sync(0xffffffffu, klo);
+        khi = __reduce_max_sync(0xffffffffu, khi);
+        if (lane == 0) { wlo[w] = klo; whi[w] = khi; }
+    }
+    if (lane == 31) wcnt[w] = inc;
     __syncthreads();
+    int rank = inc - cnt, total = 0;
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        rank += k < w ? wcnt[k] : 0;
+        total += wcnt[k];
+    }
+    if (tid == 0) {
+        st_release_u64(status + tile, (tile ? TS_AGG : TS_INCL) | (unsigned)total);
+        if (mm_keys) {
+            uint32_t lo = wlo[0], hi = whi[0];
+            for (int k = 1; k < 8; k++) { lo = min(lo, wlo[k]); hi = max(hi, whi[k]); }
+            // a stale (larger / smaller) value only costs an atomic that changes nothing
+            if (lo < mm_keys[0]) atomicMin(&mm_keys[0], lo);
+            if (hi > mm_keys[1]) atomicMax(&mm_keys[1], hi);
+        }
+    }
+    for (unsigned b = minbits; b; b &= b - 1) tgt[tid + 256 * (__ffs(b) - 1)] = ++rank;
     tile_pointer_double(sp);
-    int mine[16], cnt = 0;
+    if (w == 0) {
+        int excl = tile_lookback(status, tile);
+        if (tid == 0) {
+            base_s = excl;
+            if (tile) st_release_u64(status + tile, TS_INCL | (unsigned)(excl + total));
+        }
+    }
+    __syncthreads();
+    const int base = base_s;
+    int mine[16], nl = 0;
 #pragma unroll 4
     for (int u = 0; u < 16; u++) {
         int k = tid + 256 * u;
@@ -172,20 +265,15 @@ __global__ void __launch_bounds__(256) k_descent_tile(const float *__restrict__ 
         if (r < rows && c < cols) {
             int t = tgt[sp[k]];
             int i = r * cols + c;
-            if (t < 0) { t = -(t + 1); mine[u] = i; cnt++; }
-            ptr[i] = t;
+            if (t > 0) t += base;
+            else if (t < 0) { mine[u] = i; nl++; }
+            lab[i] = t;
         }
     }
-    int pos = block_append_pos(cnt, n_list);
+    int pos = block_append_pos(nl, n_list);
 #pragma unroll 4
     for (int u = 0; u < 16; u++)
         if (mine[u] >= 0) list[pos++] = mine[u];
-}
-
-// lab[i] = cid[ptr[i]], written over ptr (each thread only overwrites its own slot; cid is separate)
-__global__ void __launch_bounds__(256) k_catchment_ids(int *ptr_lab, const int *cid, int64_t n) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) ptr_lab[i] = cid[ptr_lab[i]];
 }
 
 __global__ void __launch_bounds__(256) k_boruvka_init(int *comp, uint32_t *E, int nC) {
@@ -384,26 +472,31 @@ __global__ void __launch_bounds__(256) k_fill_final(const float *__restrict__ z,
     if (depths) depths[i] = __fsub_rn(w, zc);
 }
 
-// every cell -> the local minimum ("catchment") it drains to: tile-local compression, then pointer jumping over the
-// cells whose path leaves their tile.  `scratch` (n ints) holds that list.
+// every cell -> the id of the catchment it drains to (0 = outside), tile-local compression, then pointer jumping over
+// the cells whose path leaves their tile.  `scratch` (n ints) holds that list.  *nC: catchments + 1 (for "outside").
 static int descent_resolve(const float *dem, int *lab, int *scratch, int64_t rows, int64_t cols, int open,
-                           int64_t *rounds_out, cudaStream_t s) {
-    DevBuf<int> cnt;
-    MS_TRY(cnt.alloc(1, s));
-    MS_CUDA(cudaMemsetAsync(cnt.p, 0, sizeof(int), s));
-    int tiles_x = (int)cdiv(cols, FT), tiles_y = (int)cdiv(rows, FT);
+                           uint32_t *mm_keys, int *nC, int64_t *rounds_out, cudaStream_t s) {
+    int tiles_x = (int)cdiv(cols, FT), tiles = tiles_x * (int)cdiv(rows, FT);
+    // the tiles' status words, then {ticket, list length}
+    DevBuf<unsigned long long> st;
+    MS_TRY(st.alloc((size_t)tiles + 1, s));
+    MS_CUDA(cudaMemsetAsync(st.p, 0, ((size_t)tiles + 1) * sizeof(unsigned long long), s));
+    int *ctl = (int *)(st.p + tiles);
     prof_units(rows * cols);
     CUtensorMap zmap;
     memset(&zmap, 0, sizeof(zmap));
     // (a band's rows sit inside a raster with halo rows: it keeps the LDG -> STS form)
     if (!open && tma_map_2d(&zmap, dem, rows, cols, FT + 2, DT_LD_TMA, true, true))
-        MS_LAUNCH(k_descent_tile<true>, tiles_x * tiles_y, 256, 0, s, dem, lab, (int)rows, (int)cols, tiles_x, open, scratch, cnt.p, zmap);
+        MS_LAUNCH(k_descent_tile<true>, tiles, 256, 0, s, dem, lab, (int)rows, (int)cols, tiles_x, open, scratch, ctl + 1,
+                  st.p, ctl, mm_keys, zmap);
     else
-        MS_LAUNCH(k_descent_tile<false>, tiles_x * tiles_y, 256, 0, s, dem, lab, (int)rows, (int)cols, tiles_x, open, scratch, cnt.p, zmap);
+        MS_LAUNCH(k_descent_tile<false>, tiles, 256, 0, s, dem, lab, (int)rows, (int)cols, tiles_x, open, scratch, ctl + 1,
+                  st.p, ctl, mm_keys, zmap);
     int64_t *h = host_flags().h;
-    MS_TRY(ms::readback(h, cnt.p, sizeof(int), s));
+    MS_TRY(ms::readback(h, st.p + tiles - 1, 2 * sizeof(unsigned long long), s));
     MS_TRY(ms::stream_sync(s));
-    return forest_resolve_list(lab, scratch, *(int *)h, rounds_out, s);
+    *nC = 1 + (int)(unsigned)h[0];
+    return forest_resolve_ids(lab, scratch, ((int *)(h + 1))[1], rounds_out, s);
 }
 
 // The Boruvka rounds of the row-band fill, on the band's cells.  comp / E initialised by k_boruvka_init, `frozen`
@@ -475,15 +568,12 @@ static int boruvka_rounds_band(const float *dem, const int *lab, int *comp, uint
 }
 
 // ---- single GPU: Boruvka on an explicit catchment edge list -------------------------------------------------------
-// The tile pass numbers the catchments and collects, per 64x64 tile, the lowest cell-pair edge between every pair of
+// The tile pass collects, per 64x64 tile, the lowest cell-pair edge between every pair of
 // catchments that touch inside it (or across its right / lower edge); later rounds work on that list only.  At
 // 32768^2 (fractal DEM) it holds 68.8 M entries for 20.3 M catchments, where the cell-list rounds visited ~650 M
 // boundary cells in round 2 alone; the list and the vertex arrays shrink every round (DESIGN.md §K1).
-constexpr int TE_SLOTS = 1024;       // shared hash slots per tile: a tile of a DEM holds ~80 catchments, white noise ~450
+constexpr int TE_SLOTS = 512;        // shared hash slots per tile: a tile of a DEM holds ~80 catchments, white noise ~450
 constexpr int TE_PROBES = 32;        // a candidate that finds no slot within this many goes straight to the global list
-constexpr int TE_LD = FT + 2;        // catchment ids of rows r0 .. r0 + 64, columns c0 - 1 .. c0 + 64
-constexpr int TE_N = (FT + 1) * TE_LD;
-constexpr int TE_LOADS = (TE_N + 255) / 256;
 
 // list entry `pos` = edge (a < b, ordered weight w); Boruvka's key of the entry for both endpoints is (w, pos), a strict
 // total order over the list, so the same pair listed by two tiles cannot form a hook cycle.  Vertex 0 ("outside")
@@ -519,33 +609,34 @@ __device__ __forceinline__ void tile_edge_insert(unsigned long long *hk, uint32_
     if (pos < cap) edge_put(ea, eb, ew, best, pos, a, b, w);
 }
 
-// One CTA per 64x64 tile (the tiling of k_descent_tile, and its TMA box of z).  lab = cid[ptr] for the tile's cells;
-// every cell pair is looked at from its lower cell (directions E, SW, S, SE); a pair of different catchments a < b is
-// an edge of weight max(z_i, z_j) (a = 0: an edge to "outside"), aggregated per pair in shared memory (minimum weight),
-// then appended to the list with one atomic per CTA, which also does round 1's lowest-edge search.  Past `cap` the
-// entries are counted but not written (the caller re-runs the pass with the counted size).
+// One CTA per 64x64 tile (the tiling of k_descent_tile, and its TMA box of z): every cell pair is looked at from its
+// lower cell (directions E, SW, S, SE); a pair of different catchments a < b is an edge of weight max(z_i, z_j) (a = 0:
+// an edge to "outside"), aggregated per pair in shared memory (minimum weight), then appended to the list with one
+// atomic per CTA, which also does round 1's lowest-edge search.  Past `cap` the entries are counted but not written
+// (the caller re-runs the pass with the counted size).
+// TMA = true: the catchment ids of rows r0 .. r0 + 64, columns c0 - 1 .. c0 + 64 come in as a second box (65 x 72 from
+// column c0 - 4, like z's), cells outside the raster as 0; no pair with such a cell is looked at.
 template <bool TMA>
-__global__ void __launch_bounds__(256) k_tile_edges(const float *__restrict__ z, const int *__restrict__ ptr,
-                                                    const int *__restrict__ cid, int *__restrict__ lab, int rows,
+__global__ void __launch_bounds__(256) k_tile_edges(const float *__restrict__ z, const int *__restrict__ lab, int rows,
                                                     int cols, int tiles_x, int *ea, int *eb, uint32_t *ew, int cap,
                                                     int *n_edges, unsigned long long *best,
-                                                    const __grid_constant__ CUtensorMap zmap) {
+                                                    const __grid_constant__ CUtensorMap zmap,
+                                                    const __grid_constant__ CUtensorMap lmap) {
     constexpr int LD = TMA ? DT_LD_TMA : FT + 2;
     constexpr int X0 = TMA ? DT_X0_TMA : 1;
     __shared__ __align__(128) float sz[(FT + 2) * LD];
-    __shared__ int sl[TE_N];
+    __shared__ __align__(128) int sl[(FT + 1) * LD];
     __shared__ unsigned long long hk[TE_SLOTS];
     __shared__ uint32_t hw[TE_SLOTS];
     __shared__ uint64_t bar;
     int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
     int r0 = ty * FT, c0 = tx * FT, tid = threadIdx.x;
-    for (int k = tid; k < TE_SLOTS; k += 256) { hk[k] = HASH_EMPTY; hw[k] = 0xffffffffu; }
     if (TMA) {
-        if (tid == 0) mbar_init(&bar, 1);
-        __syncthreads();
         if (tid == 0) {
-            mbar_expect_tx(&bar, (unsigned)sizeof(sz));
+            mbar_init(&bar, 1);
+            mbar_expect_tx(&bar, (unsigned)(sizeof(sz) + sizeof(sl)));
             tma_load_2d(sz, &zmap, &bar, c0 - DT_X0_TMA, r0 - 1);
+            tma_load_2d(sl, &lmap, &bar, c0 - DT_X0_TMA, r0);
         }
     } else {
         for (int k = tid; k < (FT + 2) * (FT + 2); k += 256) {
@@ -553,25 +644,15 @@ __global__ void __launch_bounds__(256) k_tile_edges(const float *__restrict__ z,
             int r = r0 + lr - 1, c = c0 + lc - 1;
             sz[k] = (r >= 0 && r < rows && c >= 0 && c < cols) ? z[(size_t)r * cols + c] : INFINITY;
         }
+        for (int k = tid; k < (FT + 1) * (FT + 2); k += 256) {
+            int lr = k / (FT + 2), lc = k - lr * (FT + 2);
+            int r = r0 + lr, c = c0 + lc - 1;
+            sl[k] = (r < rows && c >= 0 && c < cols) ? lab[(size_t)r * cols + c] : 0;
+        }
     }
-    // catchment ids while the copy engine brings z: all root pointers first, then their ids
-    int pv[TE_LOADS];
-#pragma unroll
-    for (int u = 0; u < TE_LOADS; u++) {
-        int k = tid + 256 * u, lr = k / TE_LD, lc = k - lr * TE_LD;
-        int r = r0 + lr, c = c0 + lc - 1;
-        pv[u] = (k < TE_N && r < rows && c >= 0 && c < cols) ? __ldg(ptr + (size_t)r * cols + c) : -1;
-    }
-#pragma unroll
-    for (int u = 0; u < TE_LOADS; u++) {
-        int k = tid + 256 * u, lr = k / TE_LD, lc = k - lr * TE_LD;
-        if (k >= TE_N) break;
-        int l = pv[u] >= 0 ? __ldg(cid + pv[u]) : -1;
-        sl[k] = l;
-        if (l >= 0 && lr < FT && lc >= 1 && lc <= FT) lab[(size_t)(r0 + lr) * cols + c0 + lc - 1] = l;
-    }
-    if (TMA) mbar_wait(&bar, 0);
+    for (int k = tid; k < TE_SLOTS; k += 256) { hk[k] = HASH_EMPTY; hw[k] = 0xffffffffu; }
     __syncthreads();
+    if (TMA) mbar_wait(&bar, 0);
     // a thread walks 16 cells down one column: the pairs of a catchment border repeat along it, so consecutive
     // candidates of the same pair are merged in registers before they reach the table
     const int lc = tid & 63, lr0 = (tid >> 6) * 16, c = c0 + lc;
@@ -581,13 +662,13 @@ __global__ void __launch_bounds__(256) k_tile_edges(const float *__restrict__ z,
         for (int u = 0; u < 16; u++) {
             const int lr = lr0 + u, r = r0 + lr;
             if (r >= rows) break;
-            const int l = sl[lr * TE_LD + lc + 1];
+            const int l = sl[lr * LD + lc + X0];
             const float zc = sz[(lr + 1) * LD + lc + X0];
 #pragma unroll
             for (int d = 0; d < 4; d++) {
                 const int dr = d == 0 ? 0 : 1, dc = d == 0 ? 1 : d - 2;
                 if (r + dr >= rows || c + dc < 0 || c + dc >= cols) continue;
-                const int m = sl[(lr + dr) * TE_LD + lc + 1 + dc];
+                const int m = sl[(lr + dr) * LD + lc + X0 + dc];
                 if (m == l) continue;
                 const uint32_t w = okey32(fmaxf(zc, sz[(lr + 1 + dr) * LD + lc + X0 + dc]));
                 const int a = min(l, m), b = max(l, m);
@@ -677,27 +758,31 @@ __global__ void __launch_bounds__(256) k_spill_down(uint32_t *wk, const int *__r
 }
 
 int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_t rows, int64_t cols,
-                          int64_t *stats, cudaStream_t s) {
+                          int64_t *stats, cudaStream_t s, float *minmax_out) {
     if (!dtm || !filled) { set_error("fill_terrain: null pointer"); return MS_ERR_ARG; }
     if (rows < 3 || cols < 3 || rows * cols > (1ll << 30)) {
         set_error("fill_terrain: unsupported shape %lld x %lld", (long long)rows, (long long)cols);
         return MS_ERR_SHAPE;
     }
     int64_t n = rows * cols;
-    DevBuf<int> lab, ptr, cid;
     DevBuf<int64_t> ctr;
-    MS_TRY(lab.alloc((size_t)n, s));
-    MS_TRY(ptr.alloc((size_t)n, s));
-    MS_TRY(cid.alloc((size_t)n, s));
+    DevBuf<uint32_t> mm_keys;
+    DevBuf<int> lab, list;
     MS_TRY(ctr.alloc(2, s));
+    if (minmax_out) {
+        MS_TRY(mm_keys.alloc(2, s));
+        MS_CUDA(cudaMemsetAsync(mm_keys.p, 0xff, sizeof(uint32_t), s));
+        MS_CUDA(cudaMemsetAsync(mm_keys.p + 1, 0, sizeof(uint32_t), s));
+    }
+    MS_TRY(lab.alloc((size_t)n, s));
+    MS_TRY(list.alloc((size_t)n, s));
     int64_t *h = host_flags().h;
 
     int64_t jump_rounds = 0;
-    MS_TRY(descent_resolve(dtm, ptr.p, cid.p, rows, cols, 0, &jump_rounds, s));
-    MS_TRY(exclusive_scan_selfptr(ptr.p, cid.p, n, ctr.p, s));
-    MS_TRY(ms::readback(h, ctr.p, sizeof(int64_t), s));
-    MS_TRY(ms::stream_sync(s));
-    const int nC = (int)h[0];
+    int nC = 0;
+    MS_TRY(descent_resolve(dtm, lab.p, list.p, rows, cols, 0, mm_keys.p, &nC, &jump_rounds, s));
+    list.release();
+    if (minmax_out) MS_LAUNCH(k_minmax_finish, 1, 1, 0, s, mm_keys.p, minmax_out);
 
     // per vertex: the lowest edge and the parent / flags of the current level; wk and map of every level (the live
     // vertices at least halve per round, so all levels together hold < 2 nC + rounds)
@@ -720,9 +805,11 @@ int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_
     if (cap > cap_max) cap = cap_max;
     DevBuf<int> ea[2], eb[2];
     DevBuf<uint32_t> ew[2];
-    CUtensorMap zmap;
+    CUtensorMap zmap, lmap;
     memset(&zmap, 0, sizeof(zmap));
-    const bool tma = tma_map_2d(&zmap, dtm, rows, cols, FT + 2, DT_LD_TMA, true, true);
+    memset(&lmap, 0, sizeof(lmap));
+    const bool tma = tma_map_2d(&zmap, dtm, rows, cols, FT + 2, DT_LD_TMA, true, true) &&
+                     tma_map_2d(&lmap, lab.p, rows, cols, FT + 1, DT_LD_TMA, false, false);
     const int tiles_x = (int)cdiv(cols, FT), tiles = tiles_x * (int)cdiv(rows, FT);
     int64_t m = 0;
     for (int attempt = 0;; attempt++) {
@@ -733,11 +820,11 @@ int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_
         MS_CUDA(cudaMemsetAsync(ctr.p + 1, 0, sizeof(int64_t), s));
         prof_units(n);
         if (tma)
-            MS_LAUNCH(k_tile_edges<true>, tiles, 256, 0, s, dtm, ptr.p, cid.p, lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
-                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap);
+            MS_LAUNCH(k_tile_edges<true>, tiles, 256, 0, s, dtm, (const int *)lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
+                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap, lmap);
         else
-            MS_LAUNCH(k_tile_edges<false>, tiles, 256, 0, s, dtm, ptr.p, cid.p, lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
-                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap);
+            MS_LAUNCH(k_tile_edges<false>, tiles, 256, 0, s, dtm, (const int *)lab.p, (int)rows, (int)cols, tiles_x, ea[0].p,
+                      eb[0].p, ew[0].p, (int)cap, (int *)(ctr.p + 1), best.p, zmap, lmap);
         MS_TRY(ms::readback(h, ctr.p + 1, sizeof(int), s));
         MS_TRY(ms::stream_sync(s));
         m = (int64_t)(unsigned)((int *)h)[0];
@@ -751,8 +838,6 @@ int fill_terrain_dev_impl(const float *dtm, float *filled, float *depths, int64_
         ea[0].release();
         cap = m + m / 4 < cap_max ? m + m / 4 : cap_max;
     }
-    cid.release();
-    ptr.release();
     MS_TRY(ea[1].alloc((size_t)m, s));
     MS_TRY(eb[1].alloc((size_t)m, s));
     MS_TRY(ew[1].alloc((size_t)m, s));
@@ -953,19 +1038,13 @@ int fill_band_local(ms_band *B, const float *dem, int64_t *n_frozen, cudaStream_
     int64_t rows = B->rows, cols = B->cols, n = rows * cols;
     int *lab = (int *)band_buf(B, BB_LAB, (size_t)n * sizeof(int));
     if (!lab) return MS_ERR_CUDA;
-    DevBuf<int> tmp;
     DevBuf<int64_t> total;
-    MS_TRY(tmp.alloc((size_t)n, s));
+    DevBuf<int> tmp;
     MS_TRY(total.alloc(1, s));
-    dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
-    unsigned g1 = cdiv(n, 256);
+    MS_TRY(tmp.alloc((size_t)n, s));
     int64_t *h = host_flags().h;
-    MS_TRY(descent_resolve(dem, lab, tmp.p, rows, cols, B->open, nullptr, s));
-    MS_TRY(exclusive_scan_selfptr(lab, tmp.p, n, total.p, s));
-    MS_LAUNCH(k_catchment_ids, g1, 256, 0, s, lab, tmp.p, n);
-    MS_TRY(ms::readback(h, total.p, sizeof(int64_t), s));
-    MS_TRY(ms::stream_sync(s));
-    int nC = (int)h[0];
+    int nC = 0;
+    MS_TRY(descent_resolve(dem, lab, tmp.p, rows, cols, B->open, nullptr, &nC, nullptr, s));
     tmp.release();
     B->nC = nC;
     int *comp = (int *)band_buf(B, BB_COMP, (size_t)nC * sizeof(int));

@@ -11,7 +11,6 @@
 #include "common.cuh"
 
 namespace ms {
-int minmax_dev(const float *z, int64_t n, float *out2, cudaStream_t s);
 int fill_no_flats_dev_impl(const float *dtm, const float *filled, double sh, double dg, double *out, int64_t rows,
                            int64_t cols, int64_t *stats, cudaStream_t s, uint8_t *flowdir_out, int *flowdir_done);
 int flowdir_dev_impl(const double *t, uint8_t *out, int64_t rows, int64_t cols, int edges, cudaStream_t s, int open);
@@ -113,14 +112,12 @@ extern "C" int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, voi
     for (int k = 0; k < 8; k++) io->stats[k] = 0;
     int64_t *h = host_flags().h;
 
-    // dem.py:67-72
-    MS_TRY(fill_terrain_dev_impl(io->dem, io->filled, io->depths, rows, cols, io->stats, s));
-    MS_TRY(ship(host->filled, io->filled, (size_t)n * sizeof(float), s));
-    MS_TRY(ship(host->depths, io->depths, (size_t)n * sizeof(float), s));
-    // dem.py:79 (fill.py:235-250)
+    // dem.py:67-72, and dem.py:79's min / max of the DEM (fill.py:235-250), which the fill's tile pass reduces
     DevBuf<float> mm;
     MS_TRY(mm.alloc(2, s));
-    MS_TRY(minmax_dev(io->dem, n, mm.p, s));
+    MS_TRY(fill_terrain_dev_impl(io->dem, io->filled, io->depths, rows, cols, io->stats, s, mm.p));
+    MS_TRY(ship(host->filled, io->filled, (size_t)n * sizeof(float), s));
+    MS_TRY(ship(host->depths, io->depths, (size_t)n * sizeof(float), s));
     MS_TRY(ms::readback(h + 24, mm.p, 2 * sizeof(float), s));
     MS_TRY(ms::stream_sync(s));
     float lo = ((float *)(h + 24))[0], hi = ((float *)(h + 24))[1];

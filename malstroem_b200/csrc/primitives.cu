@@ -1,5 +1,5 @@
-// primitives.cu — device-wide exclusive scan and forest pointer jumping, shared by the fill (catchment
-// numbering), connected components (scipy numbering) and watershed stages.
+// primitives.cu — device-wide exclusive scan and forest pointer jumping, shared by the fill (catchment ids),
+// connected components (scipy numbering) and watershed stages.
 #include "common.cuh"
 
 namespace ms {
@@ -223,6 +223,45 @@ int forest_resolve_list(int *ptr, const int *list, int n_list, int64_t *rounds_o
             if (*(int *)h == 0) break;
             if (rounds >= 64) {
                 set_error("forest_resolve: no convergence after %d rounds (cyclic pointers)", rounds);
+                return MS_ERR_NOCONV;
+            }
+        }
+    }
+    if (rounds_out) *rounds_out = rounds;
+    return MS_OK;
+}
+
+// The same jumping on catchment ids (the fill): lab[i] >= 0 is final, lab[i] < 0 links cell i to cell -(1 + lab[i])
+// further down its path.  Only the cells in `list` hold links; each round they hop up to JUMP_HOPS links and write the
+// last value back (a concurrent reader sees the old or the new value, both lie on the cell's path).
+__global__ void __launch_bounds__(256) k_forest_jump_ids(int *lab, const int *__restrict__ list, int n, int *changed) {
+    int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    int i = list[k];
+    int v = lab[i];
+    if (v >= 0) return;
+#pragma unroll 1
+    for (int h = 0; h < JUMP_HOPS && v < 0; h++) v = lab[-(v + 1)];
+    lab[i] = v;
+    if (v < 0) *changed = 1;
+}
+
+int forest_resolve_ids(int *lab, const int *list, int n_list, int64_t *rounds_out, cudaStream_t s) {
+    int rounds = 0;
+    if (n_list > 0) {
+        DevBuf<int> flag;
+        MS_TRY(flag.alloc(1, s));
+        int64_t *h = host_flags().h;
+        for (;;) {
+            MS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), s));
+            prof_units(n_list);
+            MS_LAUNCH(k_forest_jump_ids, cdiv(n_list, 256), 256, 0, s, lab, list, n_list, flag.p);
+            MS_TRY(ms::readback(h, flag.p, sizeof(int), s));
+            MS_TRY(ms::stream_sync(s));
+            rounds++;
+            if (*(int *)h == 0) break;
+            if (rounds >= 64) {
+                set_error("forest_resolve_ids: no convergence after %d rounds (cyclic links)", rounds);
                 return MS_ERR_NOCONV;
             }
         }
