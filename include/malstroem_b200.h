@@ -442,6 +442,49 @@ int ms_water_depth_dev(const float *dem, const float *filled, const int32_t *lab
 int ms_water_depth(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
                    int64_t nlabels, const double *level, float *out_depth);
 
+/* The same levels on a raster split by rows (malstroem_b200/bands.py BandPipeline.flood), one band per call, all
+ * pointers device memory, dem / filled / labels the band's own rows.  Band g owns the labels it numbered, lo < l <= hi
+ * (lo = the sum of the earlier bands' counts); a label of the band at or below lo is "foreign": its owner is a lower
+ * band.  Per-label arrays: cnt and off nlabels + 2 entries, lkey nlabels + 1, kept between the phases; cnt and off
+ * must start on 16-byte boundaries (the scans load and store 16-byte vectors).
+ *   count:   the band's cells per label, checks (labels in [0, hi], F uniform within the band), send offsets in off
+ *            and the foreign list: (label, count, F key) int32 triples in label order, at most `capacity` (a foreign
+ *            label touches the band's first or last row, so 2 * cols suffice); *n_send = cells of foreign labels.
+ *   layout:  the owner's received triples (every sender's list part for the owner, any order): counts added, F keys
+ *            checked against its own, segment offsets of its labels in off; recv_pos[i] = where run i starts in its
+ *            label's segment.  *n_cells = cells of its segments (the seg buffer to allocate).
+ *   scatter: z keys of the band's cells: owned labels' into seg, foreign labels' into send (n_send keys, label
+ *            order, so the part for each owner is contiguous).
+ *   solve:   the received key runs (concatenated in the order of the received triples, n_recv_keys = the sum of
+ *            their counts, else MS_ERR_ARG) into their segments, then the
+ *            levels and wet counts of the owned labels into out_level / out_wet [n_events][nlabels + 1] (other
+ *            columns untouched), bitwise those of ms_flood_levels_dev on the whole raster with the same st_sum and v.
+ * The return value reports bad arguments and CUDA errors only.  Errors of the data come back in *flags (combine them
+ * across the bands, then stop): MS_FLOOD_LABEL a label outside [0, hi] or a triple outside the owner's range,
+ * MS_FLOOD_UNIFORM F not uniform over a label (within the band or across bands), MS_FLOOD_VOLUME a negative v,
+ * MS_FLOOD_SIZE an owner's segments reaching 2^31 cells, MS_FLOOD_CAPACITY more foreign labels than `capacity` (labels
+ * that are not connected components).  Each phase synchronises the stream. */
+#define MS_FLOOD_LABEL 1
+#define MS_FLOOD_UNIFORM 2
+#define MS_FLOOD_VOLUME 4
+#define MS_FLOOD_SIZE 8
+#define MS_FLOOD_CAPACITY 16
+int ms_band_flood_count_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                            int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, uint32_t *lkey, int32_t *off,
+                            int32_t *foreign, int64_t capacity, int64_t *n_foreign, int64_t *n_send, int *flags,
+                            void *stream);
+int ms_band_flood_layout_dev(int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, const uint32_t *lkey, int32_t *off,
+                             const int32_t *recv, int64_t n_recv, int32_t *recv_pos, int64_t *n_cells, int *flags,
+                             void *stream);
+int ms_band_flood_scatter_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                              int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, const uint32_t *lkey,
+                              const int32_t *off, uint32_t *seg, uint32_t *send, int *flags, void *stream);
+int ms_band_flood_solve_dev(int64_t nlabels, int64_t lo, int64_t hi, const int32_t *off, const uint32_t *lkey,
+                            uint32_t *seg, const int32_t *recv, int64_t n_recv, const int32_t *recv_pos,
+                            const uint32_t *recv_keys, int64_t n_recv_keys, const double *st_sum, double cell_area,
+                            int64_t n_events, const double *v, double *out_level, int64_t *out_wet, int *flags,
+                            void *stream);
+
 #ifdef __cplusplus
 }
 #endif

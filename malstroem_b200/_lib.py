@@ -17,6 +17,7 @@ DTYPE_CODE = {np.dtype(np.float32): MS_F32, np.dtype(np.float64): MS_F64, np.dty
               np.dtype(np.bool_): MS_U8, np.dtype(np.int32): MS_I32, np.dtype(np.int64): MS_I64}
 
 ERR_CUDA, ERR_ARG, ERR_SHAPE, ERR_LABEL, ERR_NOCONV = -1, -2, -3, -4, -5
+MS_FLOOD_LABEL, MS_FLOOD_UNIFORM, MS_FLOOD_VOLUME, MS_FLOOD_SIZE, MS_FLOOD_CAPACITY = 1, 2, 4, 8, 16   # ms_band_flood_*_dev
 
 c_i64 = ctypes.c_int64
 c_int = ctypes.c_int
@@ -123,6 +124,13 @@ SIGNATURES = {
     "ms_flood_levels": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_dbl, c_i64, c_p, c_p, c_p]),
     "ms_water_depth_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p, c_p]),
     "ms_water_depth": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p]),
+    "ms_band_flood_count_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_i64,
+                                        c_p, c_p, c_p, c_p]),
+    "ms_band_flood_layout_dev": (c_int, [c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p]),
+    "ms_band_flood_scatter_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_p,
+                                          c_p, c_p]),
+    "ms_band_flood_solve_dev": (c_int, [c_i64, c_i64, c_i64, c_p, c_p, c_p, c_p, c_i64, c_p, c_p, c_i64, c_p, c_dbl,
+                                        c_i64, c_p, c_p, c_p, c_p, c_p]),
 }
 
 

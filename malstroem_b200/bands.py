@@ -78,6 +78,11 @@ class ThreadComm(object):
         t.copy_(r.to(t.dtype))
         return t
 
+    def all_to_all_var(self, chunks):
+        """chunks[j] goes to rank j; returns what every rank sent to this one (tensors of one dtype, any first dim)."""
+        got = self._swap(list(chunks))
+        return [x[self.rank].clone() for x in got]
+
     def exchange(self, up, down):
         got = self._swap((up, down))
         a = got[self.rank - 1][1].clone() if self.rank > 0 else None
@@ -107,6 +112,19 @@ class DistComm(object):
         pad[: t.shape[0]] = t
         got = self.all_gather(pad)
         return [got[i, : ns[i]] for i in range(self.size)]
+
+    def all_to_all_var(self, chunks):
+        n = torch.tensor([c.shape[0] for c in chunks], dtype=torch.int64, device=chunks[0].device)
+        got = torch.empty_like(n)
+        self.dist.all_to_all_single(got, n, group=self.group)
+        ns = got.tolist()
+        tail = tuple(chunks[0].shape[1:])
+        row = int(np.prod(tail))
+        send = torch.cat([c.reshape(-1) for c in chunks])
+        out = torch.empty(sum(ns) * row, dtype=send.dtype, device=send.device)
+        self.dist.all_to_all_single(out, send, output_split_sizes=[k * row for k in ns],
+                                    input_split_sizes=[c.shape[0] * row for c in chunks], group=self.group)
+        return [x.view((-1,) + tail) for x in out.split([k * row for k in ns])]
 
     def all_reduce(self, t, op):
         d = self.dist
@@ -175,6 +193,12 @@ def exit_targets(exit_to, cols, g):
     ok = (e >= 0) & (gn >= 0) & (gn < G)
     node = (gn.clamp(0, G - 1) * 2 + (1 - s)) * cols + e.clamp(0, cols - 1)
     return node.reshape(-1), ok.reshape(-1)
+
+
+def label_owner(labels, offsets):
+    """The band that owns each label (ascending `offsets`: the label offsets of the bands, band g numbering offsets[g]
+    + 1 ... offsets[g] + count[g]): the last band whose offset lies below the label."""
+    return torch.searchsorted(offsets, labels, right=False) - 1
 
 
 def cc_plan(roots, globals_, cell_lo, cell_hi):
@@ -587,6 +611,8 @@ class BandPipeline(object):
         counts = comm.all_gather(torch.tensor([cnt.value], dtype=torch.int64, device=dev)).view(-1)
         label_offset = int(counts[: comm.rank].sum())
         self.nlabels = int(counts.sum())
+        cl = counts.tolist()
+        self.label_ranges = [(sum(cl[:g]), c) for g, c in enumerate(cl)]      # (offset, count) of every band
         # labels of the component roots that touch a band edge, published by their owners
         ncomp = len(plan["comp_roots"])
         lab_of = torch.zeros(max(ncomp, 1), dtype=torch.int64, device=dev)
@@ -682,6 +708,121 @@ class BandPipeline(object):
                        _network.SUM_MODE if sum_mode is None else sum_mode, _p(res["rainv"]), _p(res["spillv"]),
                        _p(res["v"]), _p(res["pctv"]), None, st)
         return res
+
+    # ---- water levels and depth rasters after the rain events (csrc/flood.cu) -------------------------------------
+    _FLOOD_LOCAL = 1 << 30          # this rank's library call or allocation failed (not a data error)
+
+    def _flood_phase(self, name, *args):
+        """One phase's library call; a failure on this rank becomes a flag, so that no rank is left waiting in the
+        collective that follows.  Returns _FLOOD_LOCAL or 0."""
+        try:
+            self._call(name, *args)
+            return 0
+        except (RuntimeError, ValueError, IndexError) as e:
+            self._flood_error = e
+            return self._FLOOD_LOCAL
+
+    def _flood_flags(self, flags):
+        """Combine the error flags of a flood phase over all ranks; every rank raises."""
+        bits = (self._FLOOD_LOCAL, _lib.MS_FLOOD_LABEL, _lib.MS_FLOOD_CAPACITY, _lib.MS_FLOOD_UNIFORM,
+                _lib.MS_FLOOD_VOLUME, _lib.MS_FLOOD_SIZE)
+        got = self.comm.all_reduce(torch.tensor([1 if flags & b else 0 for b in bits], dtype=torch.int32,
+                                                device=self.device), "max").tolist()
+        if got[0]:
+            if flags & self._FLOOD_LOCAL:
+                raise self._flood_error
+            raise RuntimeError("flood: the phase failed on another band")
+        if got[1]:
+            raise IndexError("flood: a label outside [0, %d] or outside its band's range" % self.nlabels)
+        if got[2]:
+            raise ValueError("flood: a band holds more labels of lower bands than its first and last rows can carry "
+                             "(labels must be the connected bluespot labels of this run)")
+        if got[3]:
+            raise ValueError("flood: the fill is not uniform over a label (labels must be bluespots of this fill)")
+        if got[4]:
+            raise ValueError("flood: a negative volume")
+        if got[5]:
+            raise ValueError("flood: the bluespots owned by one band hold 2^31 cells or more")
+
+    def flood(self, net, cell_area):
+        """RasterPipeline.flood for a banded run: every rank returns the complete `level` float64 and `wet` int64
+        [n_events, nlabels+1], bitwise what RasterPipeline.flood gives on the whole raster with the same st_sum and v.
+        The band that numbered a label owns it; every other band sends it its cells' z keys (keys travel only
+        towards lower ranks), the owner solves its labels, and the owned column ranges are gathered."""
+        comm, dev, st, n = self.comm, self.device, self._stream(), self.nlabels + 1
+        v = net["v"].contiguous()
+        if v.dim() != 2 or v.shape[1] != n or v.dtype != torch.float64 or v.device != self.device:
+            raise ValueError("flood: net['v'] must be a float64 tensor [n_events, %d] on %s" % (n, self.device))
+        ca = float(cell_area)
+        if not (ca > 0.0 and np.isfinite(ca)):
+            raise ValueError("flood: cell_area must be > 0 (%g)" % ca)
+        ne = int(v.shape[0])
+        level = torch.full((ne, n), float("nan"), dtype=torch.float64, device=dev)
+        wet = torch.zeros((ne, n), dtype=torch.int64, device=dev)
+        if ne == 0 or self.nlabels == 0:
+            return {"level": level, "wet": wet}
+        lo, cnt_g = self.label_ranges[comm.rank]
+        hi = lo + cnt_g
+        i64, cint = ctypes.c_int64, ctypes.c_int
+        rasters = (_p(self.dem), _p(self.out["filled"]), _p(self.out["labels"]), self.rows, self.cols, self.nlabels,
+                   lo, hi)
+        cnt = torch.empty(n + 1, dtype=torch.int32, device=dev)
+        off = torch.empty(n + 1, dtype=torch.int32, device=dev)
+        lkey = torch.empty(n, dtype=torch.int32, device=dev)
+        # a foreign label reaches the band's first or last row, where at most cols / 2 labels fit in each
+        cap = 2 * self.cols
+        foreign = torch.empty((cap, 3), dtype=torch.int32, device=dev)
+        nf, nsend, flags = i64(0), i64(0), cint(0)
+        err = self._flood_phase("ms_band_flood_count_dev", *rasters, _p(cnt), _p(lkey), _p(off), _p(foreign), cap,
+                                ctypes.byref(nf), ctypes.byref(nsend), ctypes.byref(flags), st)
+        self._flood_flags(flags.value | err)
+        # every foreign run to its owner: the list is in label order, so each owner's part is contiguous
+        foreign = foreign[: nf.value]
+        starts = torch.tensor([o for o, _ in self.label_ranges], dtype=torch.int64, device=dev)
+        dest = label_owner(foreign[:, 0].long(), starts)
+        runs = torch.bincount(dest, minlength=comm.size).tolist()
+        keys = torch.zeros(comm.size, dtype=torch.int64, device=dev).index_add_(0, dest, foreign[:, 1].long()).tolist()
+        recv = torch.cat(comm.all_to_all_var(list(foreign.split(runs)))).contiguous()
+        recv_pos = torch.empty(recv.shape[0], dtype=torch.int32, device=dev)
+        ncells = i64(0)
+        err = self._flood_phase("ms_band_flood_layout_dev", self.nlabels, lo, hi, _p(cnt), _p(lkey), _p(off), _p(recv),
+                                recv.shape[0], _p(recv_pos), ctypes.byref(ncells), ctypes.byref(flags), st)
+        self._flood_flags(flags.value | err)
+        self.stats.update(flood_keys_sent=nsend.value, flood_crossing_labels=int(torch.unique(recv[:, 0]).numel()))
+        try:
+            seg = torch.empty(ncells.value, dtype=torch.int32, device=dev)
+            send = torch.empty(nsend.value, dtype=torch.int32, device=dev)
+        except RuntimeError as e:                       # out of device memory on this rank
+            self._flood_error, seg, send = e, None, None
+        err = self._FLOOD_LOCAL if seg is None else self._flood_phase(
+            "ms_band_flood_scatter_dev", *rasters, _p(cnt), _p(lkey), _p(off), _p(seg), _p(send), ctypes.byref(flags), st)
+        self._flood_flags(flags.value | err)
+        recv_keys = torch.cat(comm.all_to_all_var(list(send.split(keys)))).contiguous()
+        err = self._flood_phase("ms_band_flood_solve_dev", self.nlabels, lo, hi, _p(off), _p(lkey), _p(seg), _p(recv),
+                                recv.shape[0], _p(recv_pos), _p(recv_keys), recv_keys.numel(),
+                                _p(self.tables["st_sum"]), ca, ne, _p(v), _p(level), _p(wet), ctypes.byref(flags), st)
+        self._flood_flags(flags.value | err)
+        own = torch.cat([level[:, lo + 1:hi + 1].T, wet[:, lo + 1:hi + 1].T.view(torch.float64)], 1).contiguous()
+        got = torch.cat(comm.all_gather_var(own)).T
+        level[:, 1:] = got[:ne]
+        wet[:, 1:] = got[ne:].contiguous().view(torch.int64)
+        return {"level": level, "wet": wet}
+
+    def water_depth(self, level_row, out=None):
+        """RasterPipeline.water_depth for the band's rows: level_row is one row of flood()'s `level`."""
+        n = self.nlabels + 1
+        level_row = level_row.contiguous()
+        if level_row.shape != (n,) or level_row.dtype != torch.float64 or level_row.device != self.device:
+            raise ValueError("water_depth: level_row must be a float64 tensor [%d] on %s" % (n, self.device))
+        if out is None:
+            out = torch.empty((self.rows, self.cols), dtype=torch.float32, device=self.device)
+        elif (out.shape != (self.rows, self.cols) or out.dtype != torch.float32 or not out.is_contiguous()
+              or out.device != self.device):
+            raise ValueError("water_depth: out must be a contiguous float32 tensor of the band's shape on %s"
+                             % self.device)
+        self._call("ms_water_depth_dev", _p(self.dem), _p(self.out["filled"]), _p(self.out["labels"]), self.rows,
+                   self.cols, self.nlabels, _p(level_row), _p(out), self._stream())
+        return out
 
     # ---- host-buffer front end (bench `e2e`): H2D of the band's DEM rows, the run, D2H of every raster + table
     def host_buffers(self):

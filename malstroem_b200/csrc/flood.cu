@@ -28,7 +28,7 @@ constexpr int SEG_CTA = 8192;     // up to this size: one CTA each; larger: glob
 constexpr int WARPS_A = 4;        // warps per CTA of the one-warp-per-segment kernel
 constexpr int T_B = 256;          // threads of the one-CTA-per-segment kernels
 constexpr int CHUNK_C = T_B * 16; // cells per scan chunk of a large segment
-enum { FE_LABEL = 1, FE_UNIFORM = 2, FE_VOLUME = 4 };
+enum { FE_LABEL = MS_FLOOD_LABEL, FE_UNIFORM = MS_FLOOD_UNIFORM, FE_VOLUME = MS_FLOOD_VOLUME };
 enum { CTL_ERR, CTL_NA, CTL_NB, CTL_NC, CTL_CELLS_C, CTL_N };
 
 __device__ inline double zval(uint32_t k) { return (double)okey32_inv(k); }
@@ -37,11 +37,13 @@ __device__ inline double qnan() { return __longlong_as_double(0x7ff8000000000000
 // Pass 1 (SCATTER = false): cnt[l] += cells of l (one atomic per run of one label among a thread's 16 cells), lkey[l]
 // = okey32(F) of the label (a plain store: all writers of a uniform label store the same bits).  Pass 2 (SCATTER =
 // true, cnt zeroed again): every cell of l > 0 writes okey32(z) into segment l, and is checked against lkey[l].
+// Labels above `nlabels` are errors.  On a band, labels l <= lo belong to a lower band: pass 2 writes their cells to
+// `send` at off[l] instead (the whole raster: lo = 0).
 template <bool SCATTER>
 __global__ void __launch_bounds__(256) k_flood_group(const int32_t *__restrict__ lab, const float *__restrict__ fil,
                                                      const float *__restrict__ dem, int64_t n, int64_t nlabels,
                                                      int *cnt, uint32_t *lkey, const int *__restrict__ off,
-                                                     uint32_t *seg, int *ctl) {
+                                                     uint32_t *seg, int64_t lo, uint32_t *send, int *ctl) {
     const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * FL_CELLS;
     if (i0 >= n) return;
     const int m = n - i0 < FL_CELLS ? (int)(n - i0) : FL_CELLS;
@@ -61,7 +63,7 @@ __global__ void __launch_bounds__(256) k_flood_group(const int32_t *__restrict__
                 lkey[a] = k0;
             } else {
                 const uint32_t L = lkey[a];
-                uint32_t *dst = seg + off[a] + atomicAdd(cnt + a, e - j) - j;
+                uint32_t *dst = (a > lo ? seg : send) + off[a] + atomicAdd(cnt + a, e - j) - j;
                 for (int q = j; q < e; q++) {
                     if (okey32(__ldg(fil + i0 + q)) != L) err |= FE_UNIFORM;
                     dst[q] = okey32(__ldg(dem + i0 + q));
@@ -74,15 +76,15 @@ __global__ void __launch_bounds__(256) k_flood_group(const int32_t *__restrict__
     if (err) atomicOr(ctl + CTL_ERR, err);
 }
 
-// Labels every event of which is answered without the values (v NaN, full, or no cells; label 0) get their levels
-// here; the rest go to the list of their size class.
+// Labels l0 <= l < l1 every event of which is answered without the values (v NaN, full, or no cells; label 0) get
+// their levels here; the rest go to the list of their size class.
 __global__ void __launch_bounds__(256) k_flood_classify(const int *__restrict__ off, const uint32_t *__restrict__ lkey,
                                                         const double *__restrict__ st_sum, double ca,
-                                                        const double *__restrict__ v, int nl1, int ne, double *level,
-                                                        int64_t *wet, int *list_a, int *list_b, int *list_c,
-                                                        int *size_c, int *ctl) {
-    const int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= nl1) return;
+                                                        const double *__restrict__ v, int nl1, int ne, int l0, int l1,
+                                                        double *level, int64_t *wet, int *list_a, int *list_b,
+                                                        int *list_c, int *size_c, int *ctl) {
+    const int l = l0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (l >= l1) return;
     const int cnt = off[l + 1] - off[l];
     const double L = cnt ? zval(lkey[l]) : qnan();
     const double cap = __dmul_rn(st_sum[l], ca);
@@ -375,52 +377,35 @@ static int flood_check(const void *dem, const void *fil, const void *lab, int64_
     return MS_OK;
 }
 
-static int flood_levels_impl(const float *dem, const float *fil, const int32_t *lab, int64_t rows, int64_t cols,
-                             int64_t nlabels, const double *st_sum, double ca, int64_t ne64, const double *v,
-                             double *level, int64_t *wet, cudaStream_t s) {
-    const int64_t n = rows * cols;
-    const int nl1 = (int)nlabels + 1, ne = (int)ne64;
-    DevBuf<int> cnt, off, ctl, list_a, list_b, list_c, size_c;
-    DevBuf<uint32_t> lkey, seg;
+// Levels and wet counts of the labels l0 <= l < l1 from their segments: seg[off[l], off[l+1]) holds label l's z keys
+// (any order), lkey[l] its fill key.  Labels outside the range are not touched.  ctl: CTL_N ints, counters zero,
+// ctl[CTL_ERR] the grouping's flags.  *err: the flags after the classification (FE_VOLUME added); when they are not
+// zero nothing else runs.
+static int flood_solve(const int *off, const uint32_t *lkey, const uint32_t *seg, int l0, int l1,
+                       const double *st_sum, double ca, const double *v, int nl1, int ne, double *level, int64_t *wet,
+                       int *ctl, int *err, cudaStream_t s) {
+    const int nr = l1 - l0;
+    *err = 0;
+    if (nr <= 0) return MS_OK;
+    DevBuf<int> list_a, list_b, list_c, size_c;
     DevBuf<int64_t> total;
-    MS_TRY(cnt.alloc((size_t)nl1 + 1, s));
-    MS_TRY(off.alloc((size_t)nl1 + 1, s));
-    MS_TRY(lkey.alloc((size_t)nl1, s));
-    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_TRY(list_a.alloc((size_t)nr, s));
+    MS_TRY(list_b.alloc((size_t)nr, s));
+    MS_TRY(list_c.alloc((size_t)nr, s));
+    MS_TRY(size_c.alloc((size_t)nr, s));
     MS_TRY(total.alloc(1, s));
-    MS_CUDA(cudaMemsetAsync(cnt.p, 0, ((size_t)nl1 + 1) * sizeof(int), s));
-    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
-    const unsigned g = cdiv(n, 256 * FL_CELLS);
-    prof_units(n);
-    MS_LAUNCH(k_flood_group<false>, g, 256, 0, s, lab, fil, dem, n, nlabels, cnt.p, lkey.p, off.p, seg.p, ctl.p);
-    MS_TRY(exclusive_scan_i32(cnt.p, off.p, (int64_t)nl1 + 1, total.p, s));
+    MS_LAUNCH(k_flood_classify, cdiv(nr, 256), 256, 0, s, off, lkey, st_sum, ca, v, nl1, ne, l0, l1, level, wet,
+              list_a.p, list_b.p, list_c.p, size_c.p, ctl);
     int64_t *h = host_flags().h;
-    MS_TRY(readback(h, total.p, sizeof(int64_t), s));
-    MS_TRY(stream_sync(s));
-    const int64_t ncells = h[0];
-    MS_TRY(seg.alloc((size_t)ncells, s));
-    MS_CUDA(cudaMemsetAsync(cnt.p, 0, ((size_t)nl1 + 1) * sizeof(int), s));
-    prof_units(n);
-    MS_LAUNCH(k_flood_group<true>, g, 256, 0, s, lab, fil, dem, n, nlabels, cnt.p, lkey.p, off.p, seg.p, ctl.p);
-    MS_TRY(list_a.alloc((size_t)nl1, s));
-    MS_TRY(list_b.alloc((size_t)nl1, s));
-    MS_TRY(list_c.alloc((size_t)nl1, s));
-    MS_TRY(size_c.alloc((size_t)nl1, s));
-    MS_LAUNCH(k_flood_classify, cdiv(nl1, 256), 256, 0, s, off.p, lkey.p, st_sum, ca, v, nl1, ne, level, wet,
-              list_a.p, list_b.p, list_c.p, size_c.p, ctl.p);
-    MS_TRY(readback(h, ctl.p, CTL_N * sizeof(int), s));
+    MS_TRY(readback(h, ctl, CTL_N * sizeof(int), s));
     MS_TRY(stream_sync(s));
     int c[CTL_N];
     for (int k = 0; k < CTL_N; k++) c[k] = ((int *)h)[k];
-    if (c[CTL_ERR] & FE_LABEL) { set_error("flood_levels: a label outside [0, %lld]", (long long)nlabels); return MS_ERR_LABEL; }
-    if (c[CTL_ERR] & FE_UNIFORM) {
-        set_error("flood_levels: the fill is not uniform over a label (labels must be bluespots of this fill)");
-        return MS_ERR_ARG;
-    }
-    if (c[CTL_ERR] & FE_VOLUME) { set_error("flood_levels: a negative volume"); return MS_ERR_ARG; }
+    *err = c[CTL_ERR];
+    if (*err) return MS_OK;
     if (c[CTL_NA]) {
         prof_units(c[CTL_NA]);
-        MS_LAUNCH(k_flood_seg_warp, cdiv(c[CTL_NA], WARPS_A), WARPS_A * 32, 0, s, seg.p, off.p, lkey.p, list_a.p,
+        MS_LAUNCH(k_flood_seg_warp, cdiv(c[CTL_NA], WARPS_A), WARPS_A * 32, 0, s, seg, off, lkey, list_a.p,
                   c[CTL_NA], st_sum, ca, v, nl1, ne, level, wet);
     }
     if (c[CTL_NB]) {
@@ -431,7 +416,7 @@ static int flood_levels_impl(const float *dem, const float *fil, const int32_t *
             attr = true;
         }
         prof_units(c[CTL_NB]);
-        MS_LAUNCH(k_flood_seg_cta, c[CTL_NB], T_B, smem, s, seg.p, off.p, lkey.p, list_b.p, c[CTL_NB], st_sum, ca, v,
+        MS_LAUNCH(k_flood_seg_cta, c[CTL_NB], T_B, smem, s, seg, off, lkey, list_b.p, c[CTL_NB], st_sum, ca, v,
                   nl1, ne, level, wet);
     }
     if (c[CTL_NC]) {
@@ -455,7 +440,7 @@ static int flood_levels_impl(const float *dem, const float *fil, const int32_t *
         MS_LAUNCH(k_flood_nchunks, cdiv(nc, 256), 256, 0, s, size_c.p, nc, flag.p);
         MS_TRY(exclusive_scan_i32(flag.p, choff.p, nc, nchunks.p, s));
         prof_units(m);
-        MS_LAUNCH(k_flood_gather, cdiv(m, 256), 256, 0, s, seg.p, off.p, list_c.p, coff.p, nc, m, ka.p, va.p);
+        MS_LAUNCH(k_flood_gather, cdiv(m, 256), 256, 0, s, seg, off, list_c.p, coff.p, nc, m, ka.p, va.p);
         // LSD: stable by z key (32 bits), then stable by segment rank -> (segment, z) order
         int *k1 = ka.p, *v1 = va.p, *k2 = kb.p, *v2 = vb.p;
         MS_TRY(radix_sort_split(&k1, &v1, &k2, &v2, flag.p, total.p, m, 32, s));
@@ -467,9 +452,228 @@ static int flood_levels_impl(const float *dem, const float *fil, const int32_t *
                   prefix.p, ctot.p);
         MS_LAUNCH(k_flood_big_carry, cdiv(nc, 128), 128, 0, s, choff.p, size_c.p, nc, ctot.p, carry.p);
         MS_LAUNCH(k_flood_big_solve, cdiv((int64_t)nc * ne, 128), 128, 0, s, (const uint32_t *)k1, list_c.p,
-                  size_c.p, coff.p, choff.p, nc, prefix.p, carry.p, lkey.p, st_sum, ca, v, nl1, ne, level, wet);
+                  size_c.p, coff.p, choff.p, nc, prefix.p, carry.p, lkey, st_sum, ca, v, nl1, ne, level, wet);
     }
     return MS_OK;
+}
+
+static int flood_levels_impl(const float *dem, const float *fil, const int32_t *lab, int64_t rows, int64_t cols,
+                             int64_t nlabels, const double *st_sum, double ca, int64_t ne64, const double *v,
+                             double *level, int64_t *wet, cudaStream_t s) {
+    const int64_t n = rows * cols;
+    const int nl1 = (int)nlabels + 1, ne = (int)ne64;
+    DevBuf<int> cnt, off, ctl;
+    DevBuf<uint32_t> lkey, seg;
+    DevBuf<int64_t> total;
+    MS_TRY(cnt.alloc((size_t)nl1 + 1, s));
+    MS_TRY(off.alloc((size_t)nl1 + 1, s));
+    MS_TRY(lkey.alloc((size_t)nl1, s));
+    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_TRY(total.alloc(1, s));
+    MS_CUDA(cudaMemsetAsync(cnt.p, 0, ((size_t)nl1 + 1) * sizeof(int), s));
+    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
+    const unsigned g = cdiv(n, 256 * FL_CELLS);
+    prof_units(n);
+    MS_LAUNCH(k_flood_group<false>, g, 256, 0, s, lab, fil, dem, n, nlabels, cnt.p, lkey.p, off.p, seg.p, 0,
+              nullptr, ctl.p);
+    MS_TRY(exclusive_scan_i32(cnt.p, off.p, (int64_t)nl1 + 1, total.p, s));
+    int64_t *h = host_flags().h;
+    MS_TRY(readback(h, total.p, sizeof(int64_t), s));
+    MS_TRY(stream_sync(s));
+    const int64_t ncells = h[0];
+    MS_TRY(seg.alloc((size_t)ncells, s));
+    MS_CUDA(cudaMemsetAsync(cnt.p, 0, ((size_t)nl1 + 1) * sizeof(int), s));
+    prof_units(n);
+    MS_LAUNCH(k_flood_group<true>, g, 256, 0, s, lab, fil, dem, n, nlabels, cnt.p, lkey.p, off.p, seg.p, 0, nullptr,
+              ctl.p);
+    int err = 0;
+    MS_TRY(flood_solve(off.p, lkey.p, seg.p, 0, nl1, st_sum, ca, v, nl1, ne, level, wet, ctl.p, &err, s));
+    if (err & FE_LABEL) { set_error("flood_levels: a label outside [0, %lld]", (long long)nlabels); return MS_ERR_LABEL; }
+    if (err & FE_UNIFORM) {
+        set_error("flood_levels: the fill is not uniform over a label (labels must be bluespots of this fill)");
+        return MS_ERR_ARG;
+    }
+    if (err & FE_VOLUME) { set_error("flood_levels: a negative volume"); return MS_ERR_ARG; }
+    return MS_OK;
+}
+
+// ---- the same on a band of a raster split by rows (BandPipeline.flood).  Band g owns the labels lo < l <= hi
+// (the labels it numbered; their first cells lie in it); a label it sees at or below lo is owned by a lower band.  The
+// owner of a label gathers every band's z keys of it into its own segment and solves it there with flood_solve, so the
+// label's sorted keys, its count and with them the summation order are those of the whole-raster call.
+
+// foreign labels: flag[l] = label l (1 <= l <= lo) has cells in this band
+__global__ void __launch_bounds__(256) k_flood_foreign_flag(const int *__restrict__ cnt, int64_t lo, int *flag) {
+    const int64_t l = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (l <= lo) flag[l] = l > 0 && cnt[l] > 0;
+}
+
+// the foreign list in label order: (label, count, fill key); res[0] = flags, res[2] = cells to send (off[lo + 1])
+__global__ void __launch_bounds__(256) k_flood_foreign_list(const int *__restrict__ cnt,
+                                                            const uint32_t *__restrict__ lkey,
+                                                            const int *__restrict__ flag, const int *__restrict__ pos,
+                                                            const int *__restrict__ off, int64_t lo, int32_t *list,
+                                                            int64_t cap, int *ctl, int64_t *res) {
+    const int64_t l = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (l <= lo && flag[l]) {
+        const int64_t p = pos[l];
+        if (p < cap) {
+            list[3 * p] = (int32_t)l;
+            list[3 * p + 1] = cnt[l];
+            list[3 * p + 2] = (int32_t)lkey[l];
+        } else {
+            atomicOr(ctl + CTL_ERR, MS_FLOOD_CAPACITY);
+        }
+    }
+    if (l == 0) res[2] = off[lo + 1];
+}
+
+// received runs: check the owner range and the fill key, reserve a place in the segment (after the owner's own
+// cells: their count is in cnt[l] already).  res[0] = received cells, res[1] = the owner's own cells of its labels.
+__global__ void __launch_bounds__(256) k_flood_recv(const int32_t *__restrict__ recv, int64_t nrecv, int64_t lo,
+                                                    int64_t hi, int *cnt, const uint32_t *__restrict__ lkey,
+                                                    const int *__restrict__ off, int *pos, int *ctl,
+                                                    unsigned long long *res) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) res[1] = (unsigned long long)(off[hi + 1] - off[lo + 1]);
+    if (i >= nrecv) return;
+    const int64_t l = recv[3 * i];
+    const int c = recv[3 * i + 1];
+    if (l <= lo || l > hi || c <= 0) { atomicOr(ctl + CTL_ERR, FE_LABEL); return; }
+    if ((uint32_t)recv[3 * i + 2] != lkey[l]) atomicOr(ctl + CTL_ERR, FE_UNIFORM);
+    pos[i] = atomicAdd(cnt + l, c);
+    atomicAdd(res, (unsigned long long)c);
+}
+
+// received keys: key j of run i goes to seg[off[l_i] + pos[i] + j]
+__global__ void __launch_bounds__(256) k_flood_recv_copy(const int32_t *__restrict__ recv, int nrecv,
+                                                         const int *__restrict__ roff, const int *__restrict__ pos,
+                                                         const int *__restrict__ off,
+                                                         const uint32_t *__restrict__ keys, int64_t nkeys,
+                                                         uint32_t *seg) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= nkeys) return;
+    const int r = rank_of(roff, nrecv, (int)k);
+    seg[off[recv[3 * r]] + pos[r] + (int)k - roff[r]] = keys[k];
+}
+
+__global__ void __launch_bounds__(256) k_flood_recv_counts(const int32_t *__restrict__ recv, int nrecv, int *c) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < nrecv) c[i] = recv[3 * i + 1];
+}
+
+static int band_flood_count(const float *dem, const float *fil, const int32_t *lab, int64_t n, int64_t lo, int64_t hi,
+                            int *cnt, uint32_t *lkey, int *off, int32_t *foreign, int64_t cap, int64_t *n_foreign,
+                            int64_t *n_send, int *flags, cudaStream_t s) {
+    DevBuf<int> ctl, flag, pos;
+    DevBuf<int64_t> res;
+    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_TRY(flag.alloc((size_t)lo + 1, s));
+    MS_TRY(pos.alloc((size_t)lo + 1, s));
+    MS_TRY(res.alloc(3, s));
+    MS_CUDA(cudaMemsetAsync(cnt, 0, ((size_t)hi + 2) * sizeof(int), s));
+    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
+    prof_units(n);
+    MS_LAUNCH(k_flood_group<false>, cdiv(n, 256 * FL_CELLS), 256, 0, s, lab, fil, dem, n, hi, cnt, lkey, off,
+              nullptr, 0, nullptr, ctl.p);
+    // send offsets of the foreign labels (off[0 .. lo]), off[lo + 1] = their cells, off[hi + 1] - off[lo + 1] = the
+    // cells of the band's own labels; no sum reaches 2^31 (a band holds at most 2^30 cells)
+    MS_TRY(exclusive_scan_i32(cnt, off, hi + 2, res.p + 1, s));
+    MS_LAUNCH(k_flood_foreign_flag, cdiv(lo + 1, 256), 256, 0, s, cnt, lo, flag.p);
+    MS_TRY(exclusive_scan_i32(flag.p, pos.p, lo + 1, res.p + 1, s));
+    MS_LAUNCH(k_flood_foreign_list, cdiv(lo + 1, 256), 256, 0, s, cnt, lkey, flag.p, pos.p, off, lo, foreign, cap,
+              ctl.p, res.p);
+    int64_t *h = host_flags().h;
+    MS_TRY(readback(h, res.p + 1, 2 * sizeof(int64_t), s));
+    MS_TRY(readback(h + 2, ctl.p, sizeof(int), s));
+    MS_TRY(stream_sync(s));
+    *n_foreign = h[0] < cap ? h[0] : cap;
+    *n_send = h[1];
+    *flags = *(int *)(h + 2);
+    return MS_OK;
+}
+
+static int band_flood_layout(int64_t lo, int64_t hi, int *cnt, const uint32_t *lkey, int *off, const int32_t *recv,
+                             int64_t nrecv, int *recv_pos, int64_t *n_cells, int *flags, cudaStream_t s) {
+    DevBuf<int> ctl;
+    DevBuf<unsigned long long> res;
+    DevBuf<int64_t> total;
+    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_TRY(res.alloc(2, s));
+    MS_TRY(total.alloc(1, s));
+    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
+    MS_CUDA(cudaMemsetAsync(res.p, 0, 2 * sizeof(unsigned long long), s));
+    MS_LAUNCH(k_flood_recv, cdiv(nrecv > 0 ? nrecv : 1, 256), 256, 0, s, recv, nrecv, lo, hi, cnt, lkey, off,
+              recv_pos, ctl.p, res.p);
+    // segment offsets of the owned labels (off[lo + 1] = 0); wrong if the sum reaches 2^31, which is refused below.
+    // The scan loads and stores 16-byte vectors, so it runs on copies that start on an allocation.
+    const int64_t m = hi - lo + 1;
+    DevBuf<int> a, b;
+    MS_TRY(a.alloc((size_t)m, s));
+    MS_TRY(b.alloc((size_t)m, s));
+    MS_CUDA(cudaMemcpyAsync(a.p, cnt + lo + 1, (size_t)m * sizeof(int), cudaMemcpyDeviceToDevice, s));
+    MS_TRY(exclusive_scan_i32(a.p, b.p, m, total.p, s));
+    MS_CUDA(cudaMemcpyAsync(off + lo + 1, b.p, (size_t)m * sizeof(int), cudaMemcpyDeviceToDevice, s));
+    int64_t *h = host_flags().h;
+    MS_TRY(readback(h, res.p, 2 * sizeof(int64_t), s));
+    MS_TRY(readback(h + 2, ctl.p, sizeof(int), s));
+    MS_TRY(stream_sync(s));
+    *n_cells = h[0] + h[1];
+    *flags = *(int *)(h + 2);
+    if (*n_cells >= (1ll << 31)) {
+        set_error("band_flood_layout: the labels of a band hold %lld cells with those of the other bands; at most "
+                  "2^31 - 1 are supported", (long long)*n_cells);
+        *flags |= MS_FLOOD_SIZE;
+    }
+    return MS_OK;
+}
+
+static int band_flood_scatter(const float *dem, const float *fil, const int32_t *lab, int64_t n, int64_t lo,
+                              int64_t hi, int *cnt, const uint32_t *lkey, const int *off, uint32_t *seg,
+                              uint32_t *send, int *flags, cudaStream_t s) {
+    DevBuf<int> ctl;
+    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
+    MS_CUDA(cudaMemsetAsync(cnt, 0, ((size_t)hi + 2) * sizeof(int), s));
+    prof_units(n);
+    MS_LAUNCH(k_flood_group<true>, cdiv(n, 256 * FL_CELLS), 256, 0, s, lab, fil, dem, n, hi, cnt, (uint32_t *)lkey,
+              off, seg, lo, send, ctl.p);
+    int64_t *h = host_flags().h;
+    MS_TRY(readback(h, ctl.p, sizeof(int), s));
+    MS_TRY(stream_sync(s));
+    *flags = *(int *)h;
+    return MS_OK;
+}
+
+static int band_flood_solve(int64_t nlabels, int64_t lo, int64_t hi, const int *off, const uint32_t *lkey,
+                            uint32_t *seg, const int32_t *recv, int64_t nrecv, const int *recv_pos,
+                            const uint32_t *recv_keys, int64_t n_recv_keys, const double *st_sum, double ca,
+                            int64_t ne, const double *v, double *level, int64_t *wet, int *flags, cudaStream_t s) {
+    if (nrecv > 0) {
+        DevBuf<int> c, roff;
+        DevBuf<int64_t> total;
+        MS_TRY(c.alloc((size_t)nrecv, s));
+        MS_TRY(roff.alloc((size_t)nrecv, s));
+        MS_TRY(total.alloc(1, s));
+        MS_LAUNCH(k_flood_recv_counts, cdiv(nrecv, 256), 256, 0, s, recv, (int)nrecv, c.p);
+        MS_TRY(exclusive_scan_i32(c.p, roff.p, nrecv, total.p, s));
+        int64_t *h = host_flags().h;
+        MS_TRY(readback(h, total.p, sizeof(int64_t), s));
+        MS_TRY(stream_sync(s));
+        if (h[0] != n_recv_keys) {
+            set_error("band_flood_solve: %lld received keys for runs of %lld cells", (long long)n_recv_keys,
+                      (long long)h[0]);
+            return MS_ERR_ARG;
+        }
+        prof_units(n_recv_keys);
+        MS_LAUNCH(k_flood_recv_copy, cdiv(n_recv_keys, 256), 256, 0, s, recv, (int)nrecv, roff.p, recv_pos, off,
+                  recv_keys, n_recv_keys, seg);
+    }
+    DevBuf<int> ctl;
+    MS_TRY(ctl.alloc(CTL_N, s));
+    MS_CUDA(cudaMemsetAsync(ctl.p, 0, CTL_N * sizeof(int), s));
+    return flood_solve(off, lkey, seg, (int)lo + 1, (int)hi + 1, st_sum, ca, v, (int)nlabels + 1, (int)ne, level, wet,
+                       ctl.p, flags, s);
 }
 
 static int water_depth_impl(const float *dem, const float *fil, const int32_t *lab, int64_t rows, int64_t cols,
@@ -575,6 +779,75 @@ int ms_water_depth(const float *dem, const float *filled, const int32_t *labels,
     MS_TRY(ms::stream_sync(s));
     ms::cache_bind_host(o, out_depth, n * sizeof(float));
     return MS_OK;
+}
+
+static int band_flood_range(int64_t nlabels, int64_t lo, int64_t hi, const char *what) {
+    if (nlabels < 0 || nlabels >= (1ll << 31) - 2 || lo < 0 || lo > hi || hi > nlabels) {
+        ms::set_error("%s: the owned labels (%lld, %lld] are not a range of [1, %lld]", what, (long long)lo,
+                      (long long)hi, (long long)nlabels);
+        return MS_ERR_ARG;
+    }
+    return MS_OK;
+}
+
+int ms_band_flood_count_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                            int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, uint32_t *lkey, int32_t *off,
+                            int32_t *foreign, int64_t capacity, int64_t *n_foreign, int64_t *n_send, int *flags,
+                            void *stream) {
+    MS_TRY(ms::flood_check(dem, filled, labels, rows, cols, nlabels, "band_flood_count"));
+    MS_TRY(band_flood_range(nlabels, lo, hi, "band_flood_count"));
+    if (!cnt || !lkey || !off || !foreign || capacity < 1 || !n_foreign || !n_send || !flags ||
+        ((uintptr_t)cnt & 15) || ((uintptr_t)off & 15)) {
+        ms::set_error("band_flood_count: null pointer, cnt / off not on a 16-byte boundary or capacity < 1");
+        return MS_ERR_ARG;
+    }
+    MS_TRY(ms::ensure_init());
+    return ms::band_flood_count(dem, filled, labels, rows * cols, lo, hi, cnt, lkey, off, foreign, capacity, n_foreign,
+                                n_send, flags, (cudaStream_t)stream);
+}
+
+int ms_band_flood_layout_dev(int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, const uint32_t *lkey, int32_t *off,
+                             const int32_t *recv, int64_t n_recv, int32_t *recv_pos, int64_t *n_cells, int *flags,
+                             void *stream) {
+    MS_TRY(band_flood_range(nlabels, lo, hi, "band_flood_layout"));
+    if (!cnt || !lkey || !off || n_recv < 0 || n_recv >= (1ll << 31) || (n_recv && (!recv || !recv_pos)) ||
+        !n_cells || !flags) {
+        ms::set_error("band_flood_layout: null pointer or bad count of received runs (%lld)", (long long)n_recv);
+        return MS_ERR_ARG;
+    }
+    MS_TRY(ms::ensure_init());
+    return ms::band_flood_layout(lo, hi, cnt, lkey, off, recv, n_recv, recv_pos, n_cells, flags, (cudaStream_t)stream);
+}
+
+int ms_band_flood_scatter_dev(const float *dem, const float *filled, const int32_t *labels, int64_t rows, int64_t cols,
+                              int64_t nlabels, int64_t lo, int64_t hi, int32_t *cnt, const uint32_t *lkey,
+                              const int32_t *off, uint32_t *seg, uint32_t *send, int *flags, void *stream) {
+    MS_TRY(ms::flood_check(dem, filled, labels, rows, cols, nlabels, "band_flood_scatter"));
+    MS_TRY(band_flood_range(nlabels, lo, hi, "band_flood_scatter"));
+    if (!cnt || !lkey || !off || !flags) { ms::set_error("band_flood_scatter: null pointer"); return MS_ERR_ARG; }
+    MS_TRY(ms::ensure_init());
+    return ms::band_flood_scatter(dem, filled, labels, rows * cols, lo, hi, cnt, lkey, off, seg, send, flags,
+                                  (cudaStream_t)stream);
+}
+
+int ms_band_flood_solve_dev(int64_t nlabels, int64_t lo, int64_t hi, const int32_t *off, const uint32_t *lkey,
+                            uint32_t *seg, const int32_t *recv, int64_t n_recv, const int32_t *recv_pos,
+                            const uint32_t *recv_keys, int64_t n_recv_keys, const double *st_sum, double cell_area,
+                            int64_t n_events, const double *v, double *out_level, int64_t *out_wet, int *flags,
+                            void *stream) {
+    MS_TRY(band_flood_range(nlabels, lo, hi, "band_flood_solve"));
+    if (!off || !lkey || !st_sum || !v || !out_level || !out_wet || !flags || n_recv < 0 || n_recv >= (1ll << 31) ||
+        n_recv_keys < 0 || n_recv_keys >= (1ll << 31) || (n_recv && (!recv || !recv_pos)) ||
+        (n_recv_keys && (!recv_keys || !seg)) || (!n_recv && n_recv_keys) || n_events < 0 ||
+        n_events >= (1ll << 31) || !(cell_area > 0.0) || !isfinite(cell_area)) {
+        ms::set_error("band_flood_solve: null pointer, bad count or cell_area not > 0 (%g)", cell_area);
+        return MS_ERR_ARG;
+    }
+    MS_TRY(ms::ensure_init());
+    *flags = 0;
+    if (n_events == 0) return MS_OK;
+    return ms::band_flood_solve(nlabels, lo, hi, off, lkey, seg, recv, n_recv, recv_pos, recv_keys, n_recv_keys, st_sum,
+                                cell_area, n_events, v, out_level, out_wet, flags, (cudaStream_t)stream);
 }
 
 }  // extern "C"
