@@ -325,6 +325,48 @@ typedef struct ms_host_out {
 int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, void *stream);
 int ms_copies_wait(void);
 
+/* ---- the bluespot filter of BluespotTool.process (bluespots.py:158-170: raw labels -> raw stats -> filterbluespots ->
+ * keep_labels -> connected_components) ------------------------------------------------------------------------------
+ * A filter is a postfix program over three per-label variables (malstroem_b200/bluespot_filter.py compiles the CLI's
+ * `-filter` text into it): area = (double)count * cell_area, maxdepth = max, volume = sum * cell_area, from the raw
+ * label_stats of the depths.  Every operation is one IEEE float64 operation (the library builds with -fmad=false), so
+ * decisions are bitwise numpy's.  Comparisons push 1.0 / 0.0; truthiness is x != 0 (NaN is true, as in Python); the
+ * program keeps a label when its result is true.  Label 0 is never kept.  At most MS_BF_MAX_OPS operations and a stack
+ * of MS_BF_MAX_STACK values; a malformed program is MS_ERR_ARG before any device work. */
+#define MS_BF_MAX_OPS 64
+#define MS_BF_MAX_STACK 16
+enum {
+    MS_BF_AREA = 1, MS_BF_MAXDEPTH, MS_BF_VOLUME, MS_BF_CONST, /* push a variable, or imm[k]                 */
+    MS_BF_NEG, MS_BF_NOT,                                       /* -x, (x == 0)                              */
+    MS_BF_ADD, MS_BF_SUB, MS_BF_MUL, MS_BF_DIV,                 /* a op b (b on top of the stack)            */
+    MS_BF_LT, MS_BF_LE, MS_BF_GT, MS_BF_GE, MS_BF_EQ, MS_BF_NE, /* a op b -> 1.0 / 0.0                       */
+    MS_BF_AND, MS_BF_OR                                         /* (a != 0) op (b != 0) -> 1.0 / 0.0         */
+};
+typedef struct ms_bluespot_filter {
+    int32_t n_ops;
+    int32_t op[MS_BF_MAX_OPS];
+    double imm[MS_BF_MAX_OPS]; /* the constant of an MS_BF_CONST at the same position */
+    double cell_area;
+} ms_bluespot_filter;
+
+/* keep decisions of labels 1..nlabels from their raw stats (device tables of nlabels + 1 entries; only max, sum and
+ * count are read) as a rank-compaction table: lut_out[l] = rank of l among the kept labels (1, 2, ...), 0 for a
+ * dropped label and for label 0.  *nkept comes back to the host (synchronises the stream).  `filter` is a HOST
+ * pointer. */
+int ms_bluespot_filter_dev(const ms_bluespot_filter *filter, int64_t nlabels, const double *st_max,
+                           const double *st_sum, const int64_t *st_count, int32_t *lut_out, int64_t *nkept,
+                           void *stream);
+/* labels[c] = lut[labels[c]] in place, lut with nlabels + 1 entries: the second connected_components of
+ * bluespots.py:170, which only renumbers the kept components (SURVEY.md A.6).  MS_ERR_LABEL for a label outside
+ * [0, nlabels] (synchronises the stream). */
+int ms_relabel_dev(int32_t *labels, int64_t n, int64_t nlabels, const int32_t *lut, void *stream);
+/* ms_pipeline_host_dev with the bluespot filter between the labels and the watersheds: raw labels, raw label_stats of
+ * the depths, keep decisions, relabel; io->nlabels = the kept bluespots, every raster and table after the labels is
+ * the filtered one (the labels are shipped after the relabel).  *nlabels_raw (may be NULL) = the raw bluespots.
+ * filter == NULL is ms_pipeline_host_dev. */
+int ms_pipeline_filtered_host_dev(ms_rasters *io, const ms_host_out *host, const ms_bluespot_filter *filter,
+                                  int64_t *nlabels_raw, void *stream);
+
 /* ---- SURVEY.md §8(f): the bluespot network on device ------------------------------------------------ */
 /* net.pourpoint_network / net.next_downstream_label (malstroem/algorithms/net.py:142-192; the walk is
  * flow.trace_downstream, flow.py:279-301).  For each of the n_pp start cells (pp_row, pp_col): out_down = the first

@@ -103,6 +103,9 @@ SIGNATURES = {
     "ms_band_tables_b_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_p, c_p, c_i64, c_p, c_p, c_p]),
     "ms_pipeline_dev": (c_int, [c_p, c_p]),
     "ms_pipeline_host_dev": (c_int, [c_p, c_p, c_p]),
+    "ms_pipeline_filtered_host_dev": (c_int, [c_p, c_p, c_p, c_p, c_p]),
+    "ms_bluespot_filter_dev": (c_int, [c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ms_relabel_dev": (c_int, [c_p, c_i64, c_i64, c_p, c_p]),
     "ms_copies_wait": (c_int, []),
     "ms_synth_fractal_dev": (c_int, [c_p, c_i64, c_i64, c_i64, c_i64, c_int, c_p]),
     "ms_pourpoint_network": (c_int, [c_p, c_p, c_int, c_i64, c_i64, c_i64, c_p, c_p, c_i64, c_int, c_p, c_p, c_p, c_p,
@@ -150,6 +153,15 @@ class MsHostOut(ctypes.Structure):
     """struct ms_host_out of include/malstroem_b200.h"""
     _fields_ = [("filled", c_p), ("depths", c_p), ("fnf", c_p), ("flowdir", c_p), ("accum", c_p), ("labels", c_p),
                 ("wsheds", c_p)]
+
+
+MS_BF_MAX_OPS, MS_BF_MAX_STACK = 64, 16
+
+
+class MsBluespotFilter(ctypes.Structure):
+    """struct ms_bluespot_filter of include/malstroem_b200.h (malstroem_b200.bluespot_filter builds it)"""
+    _fields_ = [("n_ops", ctypes.c_int32), ("op", ctypes.c_int32 * MS_BF_MAX_OPS), ("imm", c_dbl * MS_BF_MAX_OPS),
+                ("cell_area", c_dbl)]
 
 
 _lib = None

@@ -11,6 +11,7 @@ Every stage of the hot path runs as "band-local kernel phase -> small exchange -
     K4 accumulation           per edge cell: where it leaves / which exit it ends at / the count it carries;
                               totals over the forest of all band exits
     K5/6 bluespot labels      roots of the edge rows; merged on the host (CPU, O(cols)); per-band counts
+    bluespot filter           all-reduces of the raw per-label stats the filter reads; every rank relabels alike
     K7 watersheds             per edge cell what it resolves to; chains followed across bands
     K8-K10 tables             all-reduces of the per-label tables (min / max / sum)
 
@@ -26,6 +27,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import bluespot_filter as _bf
 
 OPEN_TOP, OPEN_BOTTOM = 1, 2
 BAND_ALIGN = 64
@@ -309,10 +311,14 @@ class BandPipeline(object):
         self.timing[name] = self.timing.get(name, 0.0) + (now - self._t_last) * 1e3
         self._t_last = now
 
-    def run(self, ship=None):
-        """ship(names), if given, is called after the stage that finishes the rasters `names` (run_host: D2H copies)."""
+    def run(self, ship=None, bluespot_filter=None, cell_area=1.0):
+        """ship(names), if given, is called after the stage that finishes the rasters `names` (run_host: D2H copies).
+        bluespot_filter, cell_area: as for RasterPipeline.run — the bands keep the labels the single-GPU run keeps,
+        numbered alike; stats["bluespots_raw"] holds the raw count."""
         import os
         import time
+        prog = _bf.compile_filter(bluespot_filter)
+        filt = prog.struct(cell_area) if prog is not None else None
         ship = ship or (lambda names: None)
         L, comm, dev, cols, rows, n = _lib.lib(), self.comm, self.device, self.cols, self.rows, self.rows * self.cols
         st = self._stream()
@@ -387,6 +393,8 @@ class BandPipeline(object):
         self._tick("accum")
         # K5/K6 bluespot labels, K8 stats
         self._labels(st)
+        if prog is not None:
+            self._filter(st, filt, prog.reads)
         ship(("labels",))
         self._tick("labels")
         # K7 watersheds, then every per-label table (K8, K10, K8', K8'') in two fused passes and three all-reduces
@@ -630,6 +638,33 @@ class BandPipeline(object):
                    label_offset, _p(self.out["labels"]), st)
         self.stats["cc_boundary_roots"] = int(k.value)
 
+    def _filter(self, st, filt, reads):
+        """The bluespot filter (bluespots.py:160-170) across the bands: partial raw label_stats of the band, all-reduced
+        in the fields the program reads (max as a min over -max, as _tables does; count and sum added), so every rank
+        holds the same bits and computes the same keep decisions and rank table; then each band relabels its rows."""
+        comm, dev, n, m = self.comm, self.device, self.rows * self.cols, self.nlabels + 1
+        f64 = torch.float64
+        mn, mx, sm = (torch.empty(m, dtype=f64, device=dev) for _ in range(3))
+        cnt = torch.empty(m, dtype=torch.int64, device=dev)
+        self._call("ms_label_stats_dev", _p(self.out["depths"]), _lib.MS_F32, _p(self.out["labels"]), n, self.nlabels,
+                   _p(mn), _p(mx), _p(sm), _p(cnt), st)
+        if _bf.MAXDEPTH in reads:
+            mx.neg_()
+            comm.all_reduce(mx, "min")
+            mx.neg_()
+        if _bf.AREA in reads:
+            comm.all_reduce(cnt, "sum")
+        if _bf.VOLUME in reads:
+            comm.all_reduce(sm, "sum")
+        lut = torch.empty(m, dtype=torch.int32, device=dev)
+        nkept = ctypes.c_int64(0)
+        self._call("ms_bluespot_filter_dev", ctypes.byref(filt), self.nlabels, _p(mx), _p(sm), _p(cnt), _p(lut),
+                   ctypes.byref(nkept), st)
+        self._call("ms_relabel_dev", _p(self.out["labels"]), n, self.nlabels, _p(lut), st)
+        self.label_ranges = _bf.label_ranges_after_filter(self.label_ranges, (lut > 0).cpu().numpy())
+        self.stats["bluespots_raw"] = self.nlabels
+        self.nlabels = int(nkept.value)
+
     def _tables(self, st):
         """label_stats(depths, labels), label_count(wsheds), label_min_index(fnf, labels), label_max_index(accum,
         labels) (bluespots.py:160-205) for the whole raster, complete on every rank."""
@@ -834,11 +869,12 @@ class BandPipeline(object):
             self._host = h
         return self._host
 
-    def run_host(self, dem_host=None):
+    def run_host(self, dem_host=None, bluespot_filter=None, cell_area=1.0):
         """Pinned host DEM rows -> H2D -> the staged run -> D2H.  Every rank brings back its own rows of the rasters,
         each over a copy stream as soon as the stage that produces it is done (so the copies overlap the later stages,
         as in RasterPipeline.run_host); the per-label tables are replicated on every rank, so rank 0 alone ships
-        them, into pinned buffers.  Returns the dict of pinned host tensors (`tables` only on rank 0)."""
+        them, into pinned buffers.  Returns the dict of pinned host tensors (`tables` only on rank 0).
+        bluespot_filter, cell_area: as for run()."""
         h = self.host_buffers()
         if dem_host is not None:
             h["dem"].copy_(torch.from_numpy(dem_host) if isinstance(dem_host, np.ndarray) else dem_host)
@@ -859,7 +895,7 @@ class BandPipeline(object):
                         for a in range(0, src.shape[0], step):
                             dst[a:a + step].copy_(src[a:a + step], non_blocking=True)
 
-        self.run(ship=ship)
+        self.run(ship=ship, bluespot_filter=bluespot_filter, cell_area=cell_area)
         tabs = {}
         if self.comm.rank == 0:
             m = self.nlabels + 1
@@ -889,10 +925,11 @@ class BandPipeline(object):
         return self.rows * self.cols * per_cell + (self.nlabels + 1) * per_label
 
 
-def run_threaded(dem, nbands, device=0, after=None, eps=None):
+def run_threaded(dem, nbands, device=0, after=None, eps=None, bluespot_filter=None, cell_area=1.0):
     """One process, one GPU, `nbands` bands as threads (the decomposition without NCCL): returns the BandPipelines
     after the run.  `dem`: cuda float32 tensor [rows, cols].  `after(pipeline)`, if given, runs in every band's
-    thread after the run (for calls that communicate, like `network`); its result is kept in `p.after_result`."""
+    thread after the run (for calls that communicate, like `network`); its result is kept in `p.after_result`.
+    bluespot_filter, cell_area: as for BandPipeline.run."""
     rows, cols = dem.shape
     grp = ThreadGroup(nbands)
     pipes, errs = [None] * nbands, []
@@ -903,7 +940,7 @@ def run_threaded(dem, nbands, device=0, after=None, eps=None):
             p = BandPipeline(rows, cols, ThreadComm(grp, rank), device=device, eps=eps)
             pipes[rank] = p
             p.dem.copy_(dem[p.r0:p.r1])
-            p.run()
+            p.run(bluespot_filter=bluespot_filter, cell_area=cell_area)
             if after is not None:
                 p.after_result = after(p)
         except BaseException as e:      # noqa: BLE001 - report and release the other threads

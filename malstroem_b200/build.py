@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 TAG = os.environ.get("MS_BUILD_TAG", "")
 OBJ = os.path.join(HERE, "csrc", "_obj" + TAG)
 LIB = os.path.join(HERE, "libmalstroem_b200%s.so" % TAG)
-SOURCES = ["core.cu", "primitives.cu", "fill.cu", "noflats.cu", "flow.cu", "accum.cu", "labels.cu", "pipeline.cu", "synth.cu", "network.cu", "cache.cu", "tiff.cu", "polygon.cu", "flood.cu"]
+SOURCES = ["core.cu", "primitives.cu", "fill.cu", "noflats.cu", "flow.cu", "accum.cu", "labels.cu", "pipeline.cu", "synth.cu", "network.cu", "cache.cu", "tiff.cu", "polygon.cu", "flood.cu", "bfilter.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 # no --use_fast_math: denormals (ftz=false), exact division and no FMA contraction are part of the contract
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-fmad=false",

@@ -1,8 +1,9 @@
 // pipeline.cu — the whole raster hot path on device-resident data (what bench.py times):
 // DEM -> fill (+depths) -> short/diag -> no-flats fill -> D8 -> accumulation -> bluespot labels ->
-// label stats -> watersheds (+counts) -> pour points.  Order and operands follow DemTool.process
-// (malstroem/dem.py:53-93) and BluespotTool.process (malstroem/bluespots.py:138-216) without the
-// bluespot filter (bench: no filter; the tool layer applies its filter on the host between the stages).
+// [bluespot filter] -> label stats -> watersheds (+counts) -> pour points.  Order and operands follow DemTool.process
+// (malstroem/dem.py:53-93) and BluespotTool.process (malstroem/bluespots.py:138-216).  The bluespot filter
+// (bluespots.py:160-170) runs when the caller gives one (ms_pipeline_filtered_host_dev): raw label stats, keep
+// decisions and a relabel of the kept labels by rank (bfilter.cu); bench.py runs without a filter.
 #include <math.h>
 
 #include <stdio.h>
@@ -29,6 +30,10 @@ int pipeline_tables_dev_impl(const float *depths, const int32_t *lab, const doub
                              double *st_max, double *st_sum, int64_t *st_count, int64_t *ws_count, double *pmin_v,
                              int64_t *pmin_r, int64_t *pmin_c, double *pmax_v, int64_t *pmax_r, int64_t *pmax_c,
                              int *err_dev, cudaStream_t s);
+int bluespot_filter_dev_impl(const ms_bluespot_filter *f, int64_t nlabels, const double *st_max, const double *st_sum,
+                             const int64_t *st_count, int32_t *lut, int64_t *nkept, cudaStream_t s);
+int relabel_dev_impl(int32_t *lab, int64_t n, int64_t nlabels, const int32_t *lut, int *err_dev, cudaStream_t s);
+int check_bluespot_filter(const ms_bluespot_filter *f);
 }  // namespace ms
 
 namespace {
@@ -92,9 +97,41 @@ extern "C" int ms_copies_wait(void) {
     return MS_OK;
 }
 
+namespace {
+// bluespots.py:160-170: raw label_stats(depths, labels) -> filterbluespots -> keep_labels -> connected_components,
+// the last two as one relabel by rank.  The raw stats go into the pipeline's own tables when it has all four (the
+// table passes overwrite them with the filtered ones), into scratch otherwise.
+int filter_labels(ms_rasters *io, const ms_bluespot_filter *filter, int *err_dev, cudaStream_t s) {
+    using namespace ms;
+    const int64_t n = io->rows * io->cols, m = io->nlabels + 1;
+    DevBuf<double> smin, smax, ssum;
+    DevBuf<int64_t> scnt;
+    double *tmin = io->st_min, *tmax = io->st_max, *tsum = io->st_sum;
+    int64_t *tcnt = io->st_count;
+    if (!tmin || !tmax || !tsum || !tcnt) {
+        MS_TRY(smin.alloc((size_t)m, s)); MS_TRY(smax.alloc((size_t)m, s));
+        MS_TRY(ssum.alloc((size_t)m, s)); MS_TRY(scnt.alloc((size_t)m, s));
+        tmin = smin.p; tmax = smax.p; tsum = ssum.p; tcnt = scnt.p;
+    }
+    MS_TRY(label_stats_dev_impl(io->depths, MS_F32, io->labels, n, io->nlabels, tmin, tmax, tsum, tcnt, err_dev, s));
+    DevBuf<int32_t> lut;
+    MS_TRY(lut.alloc((size_t)m, s));
+    int64_t nkept = 0;
+    MS_TRY(bluespot_filter_dev_impl(filter, io->nlabels, tmax, tsum, tcnt, lut.p, &nkept, s));
+    MS_TRY(relabel_dev_impl(io->labels, n, io->nlabels, lut.p, err_dev, s));
+    io->nlabels = nkept;
+    return MS_OK;
+}
+}  // namespace
+
 extern "C" int ms_pipeline_dev(ms_rasters *io, void *stream) { return ms_pipeline_host_dev(io, nullptr, stream); }
 
 extern "C" int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, void *stream) {
+    return ms_pipeline_filtered_host_dev(io, host, nullptr, nullptr, stream);
+}
+
+extern "C" int ms_pipeline_filtered_host_dev(ms_rasters *io, const ms_host_out *host, const ms_bluespot_filter *filter,
+                                             int64_t *nlabels_raw, void *stream) {
     using namespace ms;
     if (host && g_trace_on > 0) {
         if (!g_trace_origin) cudaEventCreate(&g_trace_origin);
@@ -108,6 +145,7 @@ extern "C" int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, voi
         set_error("pipeline: null raster pointer");
         return MS_ERR_ARG;
     }
+    if (filter) MS_TRY(check_bluespot_filter(filter));
     int64_t rows = io->rows, cols = io->cols, n = rows * cols;
     for (int k = 0; k < 8; k++) io->stats[k] = 0;
     int64_t *h = host_flags().h;
@@ -148,12 +186,14 @@ extern "C" int ms_pipeline_host_dev(ms_rasters *io, const ms_host_out *host, voi
     MS_TRY(ms::readback(h, tot.p, sizeof(int64_t), s));
     MS_TRY(ms::stream_sync(s));
     io->nlabels = h[0];
-    MS_TRY(ship(host->labels, io->labels, (size_t)n * sizeof(int32_t), s));
+    if (nlabels_raw) *nlabels_raw = io->nlabels;
     if (io->nlabels + 1 > io->table_capacity) {
         set_error("pipeline: %lld labels do not fit table_capacity %lld", (long long)io->nlabels,
                   (long long)io->table_capacity);
         return MS_ERR_ARG;
     }
+    if (filter) MS_TRY(filter_labels(io, filter, err.p, s));
+    MS_TRY(ship(host->labels, io->labels, (size_t)n * sizeof(int32_t), s));
     // every table asked for (the usual case): two fused passes over the rasters (labels.cu: k_tables_a2 / k_tables_b)
     const bool fused = io->st_min && io->st_max && io->st_sum && io->st_count && io->ws_count && io->ppmin_value &&
                        io->ppmin_row && io->ppmin_col;

@@ -65,21 +65,35 @@ class RasterPipeline(object):
         self._host = None
 
     # ---- device-resident run (bench `value`) ---------------------------------------------------------
-    def run(self, dem=None, host_out=None):
+    def run(self, dem=None, host_out=None, bluespot_filter=None, cell_area=1.0):
         """dem: optional cuda float32 tensor of the pipeline's shape (else self.dem is used as is).
         host_out: optional _lib.MsHostOut of pinned host buffers the finished rasters are shipped to while the later
-        stages run (complete after ms_copies_wait)."""
+        stages run (complete after ms_copies_wait).
+        bluespot_filter: optional `-filter` text of the reference's CLI (malstroem_b200.bluespot_filter), evaluated on
+        the raw bluespots with `cell_area` (the area of one cell, for `area` and `volume`); every raster and table
+        from the labels on is then the filtered one (bluespots.py:158-206), and stats["bluespots_raw"] holds the raw
+        count.  None or "" runs without a filter."""
+        from . import bluespot_filter as _bf
+        prog = _bf.compile_filter(bluespot_filter)
+        filt = prog.struct(cell_area) if prog is not None else None
         if dem is not None and dem.data_ptr() != self.dem.data_ptr():
             self.dem.copy_(dem)
         stream = torch.cuda.current_stream(self.device).cuda_stream
+        nraw = ctypes.c_int64(0)
         with _lib.lock:
-            if host_out is None:
+            if filt is not None:
+                _lib.check(_lib.lib().ms_pipeline_filtered_host_dev(
+                    ctypes.byref(self.io), ctypes.byref(host_out) if host_out is not None else None, ctypes.byref(filt),
+                    ctypes.byref(nraw), ctypes.c_void_p(stream)), "ms_pipeline_filtered_host_dev")
+            elif host_out is None:
                 _lib.check(_lib.lib().ms_pipeline_dev(ctypes.byref(self.io), ctypes.c_void_p(stream)), "ms_pipeline_dev")
             else:
                 _lib.check(_lib.lib().ms_pipeline_host_dev(ctypes.byref(self.io), ctypes.byref(host_out),
                                                            ctypes.c_void_p(stream)), "ms_pipeline_host_dev")
         self.nlabels = int(self.io.nlabels)
         self.stats = dict(zip(STAT_NAMES, [int(v) for v in self.io.stats]))
+        if filt is not None:
+            self.stats["bluespots_raw"] = int(nraw.value)
         self.short, self.diag = float(self.io.short_eps), float(self.io.diag_eps)
         return self
 
@@ -166,9 +180,10 @@ class RasterPipeline(object):
             self._host = h
         return self._host
 
-    def run_host(self, dem_host=None):
+    def run_host(self, dem_host=None, bluespot_filter=None, cell_area=1.0):
         """dem_host: pinned (or pageable) float32 CPU tensor / ndarray.  Returns the dict of pinned host
-        tensors holding the output rasters (HOST_RASTERS) and the first nlabels+1 entries of every table."""
+        tensors holding the output rasters (HOST_RASTERS) and the first nlabels+1 entries of every table.
+        bluespot_filter, cell_area: as for run()."""
         h = self.host_buffers()
         if dem_host is not None:
             src = torch.from_numpy(dem_host) if isinstance(dem_host, np.ndarray) else dem_host
@@ -178,7 +193,7 @@ class RasterPipeline(object):
         ho = _lib.MsHostOut()
         for name in self.host_rasters():
             setattr(ho, name, h[name].data_ptr())
-        self.run(host_out=ho)          # rasters leave through the copy stream while the later stages run
+        self.run(host_out=ho, bluespot_filter=bluespot_filter, cell_area=cell_area)          # rasters leave through the copy stream while the later stages run
         m = self.nlabels + 1
         for name, t in self.tables.items():
             h[name][:m].copy_(t[:m], non_blocking=True)
