@@ -139,3 +139,85 @@ def pathological_spiral_dem(rows, cols, seed=3):
     # the outer end drains off the right border
     mm[py[-1], px[-1]:] = lo - 1000
     return (mm.astype(np.float32) * np.float32(0.001)).astype(np.float32)
+
+
+def serpentine_path(rows, cols, pitch):
+    """Cells (rows, cols index arrays, in flow order) of a one-cell channel that runs down column 1, along row rows-2,
+    up column 1 + pitch, along row 1, ... every `pitch` columns, and then along its last row to the right border."""
+    if pitch < 2 or rows < 5 or cols < pitch + 6:
+        raise ValueError("serpentine: needs pitch >= 2, rows >= 5 and cols >= pitch + 6")
+    xs = list(range(1, cols - 5, pitch))
+    pr, pc = [], []
+    down = np.arange(1, rows - 1)
+    for k, x in enumerate(xs):
+        seg = down if k % 2 == 0 else down[::-1]
+        pr.append(seg)
+        pc.append(np.full(seg.size, x))
+        end = seg[-1]
+        stop = xs[k + 1] if k + 1 < len(xs) else cols
+        run = np.arange(x + 1, stop)
+        pr.append(np.full(run.size, end))
+        pc.append(run)
+    return np.concatenate(pr), np.concatenate(pc)
+
+
+def serpentine_dem(rows, cols, pitch=4, pit=False):
+    """Walls of 100 and a serpentine channel (serpentine_path) whose bed falls by one step per cell to the right
+    border: the whole raster drains down one path that crosses every row-band edge once per column of the channel
+    (about cols / pitch times), with a flow accumulation that reaches nearly rows * cols there.  With `pit`, the third-last channel cell is a
+    one-cell pit two steps below the channel cell after it: the only bluespot, whose watershed is nearly the whole
+    raster.  The bed is an integer times a power of two, exact in float32 and below 64."""
+    pr, pc = serpentine_path(rows, cols, pitch)
+    n = pr.size
+    scale = np.float32(2.0 ** -max(0, int(n).bit_length() - 6))
+    bed = (n - np.arange(n)).astype(np.float32) * scale
+    if pit:
+        bed[n - 3] = bed[n - 1] - scale
+    dem = np.full((rows, cols), 100.0, np.float32)
+    dem[pr, pc] = bed
+    return dem
+
+
+def mask_dem(mask):
+    """0 on the cells of `mask`, 10 elsewhere and on the raster border: every 8-connected component of the mask away
+    from the border is one bluespot of depth 10, and the filled raster is one flat at 10."""
+    dem = np.where(mask, np.float32(0.0), np.float32(10.0)).astype(np.float32)
+    dem[0, :] = dem[-1, :] = dem[:, 0] = dem[:, -1] = 10.0
+    return dem
+
+
+def comb_mask(rows, cols):
+    """Teeth in every third column from row 1 to row rows-2, joined in pairs by row rows-2 alone: two pieces of one
+    component in every band but the last, which has at least two rows in any row-band split."""
+    m = np.zeros((rows, cols), bool)
+    teeth = list(range(3, cols - 1, 3))
+    for x in teeth:
+        m[1:rows - 1, x] = True
+    for a, b in zip(teeth[0::2], teeth[1::2]):
+        m[rows - 2, a:b + 1] = True
+    return m
+
+
+def speckle_mask(rows, cols, density=0.39, seed=1):
+    """Independent cells at `density`: just below the 8-connected site-percolation threshold (0.407), many components,
+    some hundreds of rows tall with long, thin branches."""
+    return np.random.default_rng(seed).random((rows, cols)) < density
+
+
+def pit_chain_dem(rows, cols, period=64):
+    """Walls of 100 and one channel down column cols // 2: a pit in the middle of every `period` rows, a rim of two
+    cells on every multiple of `period` rows, the rims falling by one per period away from the outlet at row 0 (so
+    every pit spills over the rim below it into the next pit, away from the outlet, and the chain drains out over the
+    60 of row 1).  With row bands of `period` rows each pit lies in its own band and spills across a band edge."""
+    c = cols // 2
+    r = np.arange(rows)
+    mid = (r // period) * period + period // 2
+    z = 10.0 + 0.25 * np.abs(r - mid)
+    edge = (r % period == 0) | (r % period == period - 1)
+    k = (r + 1) // period                              # the rim on rows k*period - 1, k*period
+    z = np.where(edge & (r >= period - 1), 50.0 - k, z)
+    dem = np.full((rows, cols), 100.0, np.float32)
+    dem[1:rows - 1, c] = z[1:rows - 1]
+    dem[1, c] = 60.0
+    dem[0, c] = 5.0
+    return dem

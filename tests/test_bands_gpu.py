@@ -5,43 +5,11 @@ import numpy as np
 import pytest
 import torch
 
+from band_cases import check, oracle_all
 from malstroem_b200 import bands, synth
 from oracle import port
 
 pytestmark = pytest.mark.gpu
-
-
-def oracle_all(dem):
-    filled = port.fill_terrain(dem)
-    short, diag = port.minimum_safe_short_and_diag(dem)
-    fnf = port.fill_terrain_no_flats(dem, short, diag)
-    fd = port.terrain_flowdirection(fnf)
-    acc = port.accumulated_flow(fd, fast=True)
-    depths = filled - dem
-    lab, n = port.connected_components(depths)
-    ws = lab.copy()
-    port.watersheds_from_labels(fd, ws, 0)
-    return dict(filled=filled, depths=depths, fnf=fnf, flowdir=fd, accum=acc, labels=lab, wsheds=ws, n=n,
-                stats=port.label_stats(depths, lab, n), count=port.label_count(ws),
-                ppmin=port.label_min_index(fnf, lab, n), ppmax=port.label_max_index(acc, lab, n))
-
-
-def check(pipes, want):
-    for name in ("filled", "depths", "fnf", "flowdir", "accum", "labels", "wsheds"):
-        got = torch.cat([p.out[name] for p in pipes]).cpu().numpy()
-        assert np.array_equal(got, want[name]), name
-    for p in pipes:                                   # every rank holds the same, complete tables
-        assert p.nlabels == want["n"]
-        t = {k: v.cpu().numpy() for k, v in p.tables.items()}
-        for k in ("min", "max", "count"):
-            assert np.array_equal(t["st_" + k], want["stats"][k]), k
-        np.testing.assert_allclose(t["st_sum"], want["stats"]["sum"], rtol=1e-6, atol=1e-300)
-        m = len(want["count"])
-        assert np.array_equal(t["ws_count"][:m], want["count"]) and not t["ws_count"][m:].any()
-        for key in ("ppmin", "ppmax"):
-            assert np.array_equal(t[key + "_row"], want[key]["row"]), key
-            assert np.array_equal(t[key + "_col"], want[key]["col"]), key
-            assert np.array_equal(t[key + "_value"], want[key]["value"]), key
 
 
 @pytest.mark.parametrize("shape,nbands,seed", [((320, 256), 2, 11), ((448, 200), 3, 12), ((512, 384), 4, 13),
