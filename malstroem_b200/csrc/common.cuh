@@ -181,8 +181,6 @@ __device__ inline int d8_border(int code, bool top, bool bot, int c, int cols) {
 // ---- shared device primitives (scan.cu, forest.cu) ----------------------------------------------
 // exclusive scan of int32 flags; out may alias flags; *total_dev receives the sum (int64 on device)
 int exclusive_scan_i32(const int *flags, int *out, int64_t n, int64_t *total_dev, cudaStream_t s);
-// the same over the flags "ptr[i] == i" (roots of a parent-pointer array); out must not alias ptr
-int exclusive_scan_selfptr(const int *ptr, int *out, int64_t n, int64_t *total_dev, cudaStream_t s);
 // stable LSD sort of int (key, val) pairs on key bits [0, bits), one binary split per bit (network.cu: the network's
 // upstream lists, flood.cu's large segments).  The passes ping-pong between the buffers; on return *key / *val point
 // at the sorted pairs and *key_alt / *val_alt at the other pair of buffers.  flag: n ints of scratch.

@@ -81,13 +81,16 @@ __global__ void __launch_bounds__(256) k_ws_ptr(const uint8_t *__restrict__ fd, 
 }
 
 // Tile form of k_ws_ptr + most of the pointer jumping (see k_descent_tile): in-tile paths are compressed in shared
-// memory; a cell whose path leaves its tile gets the cell it enters next and goes on `list` for the global jumps.
-template <typename L>
-__global__ void __launch_bounds__(256) k_ws_tile(const uint8_t *__restrict__ fd, const L *__restrict__ lab, int *ptr,
+// memory; a cell whose path leaves its tile goes on `list` for the global jumps.
+// LABELS = false: out = ptr, the first labelled / terminal cell on the path; a listed cell holds the cell it enters
+// next.  LABELS = true (labels >= 0, unassigned 0): out = the watershed raster itself - the in-tile root's label, or,
+// for a listed cell, -(1 + the cell it enters next), the link encoding of forest_resolve_ids.
+template <typename L, bool LABELS>
+__global__ void __launch_bounds__(256) k_ws_tile(const uint8_t *__restrict__ fd, const L *__restrict__ lab, int *out,
                                                  int *interior_nodir, L unassigned, int rows, int cols, int tiles_x,
                                                  int *list, int *n_list) {
     __shared__ unsigned short sp[FT * FT];
-    __shared__ int tgt[FT * FT];          // per tile-local root: >= 0 final global index, < 0: -(1 + cell in another tile)
+    __shared__ int tgt[FT * FT];          // per tile-local root: >= 0 final (cell index or label), < 0: -(1 + cell in another tile)
     int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
     int r0 = ty * FT, c0 = tx * FT, tid = threadIdx.x;
 #pragma unroll 4
@@ -99,10 +102,11 @@ __global__ void __launch_bounds__(256) k_ws_tile(const uint8_t *__restrict__ fd,
         int t = 0;
         if (r < rows && c < cols) {
             int i = r * cols + c;
-            t = i;
+            const L v = lab[i];
+            t = LABELS ? (int)v : i;
             int d = fd[i], nr, nc;
             if (interior_nodir && d > 7 && r > 0 && c > 0 && r < rows - 1 && c < cols - 1) *interior_nodir = 1;
-            if (lab[i] == unassigned && d8_next(r, c, d, rows, cols, &nr, &nc)) {
+            if (v == unassigned && d8_next(r, c, d, rows, cols, &nr, &nc)) {
                 int tr = nr - r0, tc = nc - c0;
                 if (tr >= 0 && tr < FT && tc >= 0 && tc < FT) p = (unsigned short)(tr * FT + tc);
                 else t = -(1 + nr * cols + nc);
@@ -123,8 +127,12 @@ __global__ void __launch_bounds__(256) k_ws_tile(const uint8_t *__restrict__ fd,
         if (r < rows && c < cols) {
             int t = tgt[sp[k]];
             int i = r * cols + c;
-            if (t < 0) { t = -(t + 1); mine[u] = i; cnt++; }
-            ptr[i] = t;
+            if (t < 0) {
+                mine[u] = i;
+                cnt++;
+                if (!LABELS) t = -(t + 1);
+            }
+            out[i] = t;
         }
     }
     int pos = block_append_pos(cnt, n_list);
@@ -133,9 +141,10 @@ __global__ void __launch_bounds__(256) k_ws_tile(const uint8_t *__restrict__ fd,
         if (mine[u] >= 0) list[pos++] = mine[u];
 }
 
-// ptr[i] = the first labelled / terminal cell on i's path.  `scratch_list`: n ints.
-template <typename L>
-static int ws_resolve(const uint8_t *fd, const L *lab, int *ptr, int *nodir_flag, L unassigned, int64_t rows,
+// LABELS = false: ptr[i] = the first labelled / terminal cell on i's path.  LABELS = true: out = the watershed labels
+// (see k_ws_tile).  `nodir_flag` (optional) comes back in host_flags().h[8].
+template <typename L, bool LABELS>
+static int ws_resolve(const uint8_t *fd, const L *lab, int *out, int *nodir_flag, L unassigned, int64_t rows,
                       int64_t cols, int64_t *rounds_out, cudaStream_t s) {
     int64_t n = rows * cols;
     DevBuf<int> list, cnt;
@@ -144,13 +153,14 @@ static int ws_resolve(const uint8_t *fd, const L *lab, int *ptr, int *nodir_flag
     MS_CUDA(cudaMemsetAsync(cnt.p, 0, sizeof(int), s));
     int tiles_x = (int)cdiv(cols, FT), tiles_y = (int)cdiv(rows, FT);
     prof_units(n);
-    MS_LAUNCH(k_ws_tile<L>, tiles_x * tiles_y, 256, 0, s, fd, lab, ptr, nodir_flag, unassigned, (int)rows, (int)cols,
-              tiles_x, list.p, cnt.p);
+    MS_LAUNCH((k_ws_tile<L, LABELS>), tiles_x * tiles_y, 256, 0, s, fd, lab, out, nodir_flag, unassigned, (int)rows,
+              (int)cols, tiles_x, list.p, cnt.p);
     int64_t *h = host_flags().h;
     MS_TRY(ms::readback(h, cnt.p, sizeof(int), s));
     if (nodir_flag) MS_TRY(ms::readback(h + 8, nodir_flag, sizeof(int), s));
     MS_TRY(ms::stream_sync(s));
-    return forest_resolve_list(ptr, list.p, *(int *)h, rounds_out, s);
+    if (LABELS) return forest_resolve_ids(out, list.p, *(int *)h, rounds_out, s);
+    return forest_resolve_list(out, list.p, *(int *)h, rounds_out, s);
 }
 
 template <typename L>
@@ -179,7 +189,7 @@ int watersheds_dev_t(const uint8_t *fd, L *lab, int64_t rows, int64_t cols, L un
     dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
     int64_t *h = host_flags().h;
     int64_t rounds = 0;
-    MS_TRY(ws_resolve<L>(fd, lab, ptr.p, flag.p, unassigned, rows, cols, &rounds, s));     // synchronises: h[8] is valid
+    MS_TRY((ws_resolve<L, false>(fd, lab, ptr.p, flag.p, unassigned, rows, cols, &rounds, s)));     // synchronises: h[8] is valid
     bool general = *(int *)(h + 8) != 0;
     if (general) {
         MS_TRY(ptr_full.alloc((size_t)n, s));
@@ -204,6 +214,30 @@ int watersheds_dev_impl(const uint8_t *fd, void *lab, int label_bytes, int64_t r
     if (label_bytes == 8) return watersheds_dev_t<int64_t>(fd, (int64_t *)lab, rows, cols, unassigned, stats, s);
     set_error("watersheds_from_labels: label_bytes must be 4 or 8");
     return MS_ERR_ARG;
+}
+
+// The pipeline's K7 (labels int32 >= 0, unassigned 0): the tile pass reads `lab` and writes the watershed raster `ws`
+// directly, and only the cells whose path leaves their tile are resolved afterwards - no copy of the labels, no ptr
+// raster and no pass over every cell to gather lab[root].  A path can only end at an interior cell without a flow
+// direction on a DEM with NaNs (the fallback D8); then the general form runs again from the untouched labels.
+int watersheds_labels_dev_impl(const uint8_t *fd, const int32_t *lab, int32_t *ws, int64_t rows, int64_t cols,
+                               int64_t *stats, cudaStream_t s) {
+    if (!fd || !lab || !ws) { set_error("watersheds: null pointer"); return MS_ERR_ARG; }
+    if (rows < 1 || cols < 1 || rows * cols > (1ll << 30)) {
+        set_error("watersheds: unsupported shape %lld x %lld", (long long)rows, (long long)cols);
+        return MS_ERR_SHAPE;
+    }
+    DevBuf<int> flag;
+    MS_TRY(flag.alloc(1, s));
+    MS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), s));
+    int64_t rounds = 0;
+    MS_TRY((ws_resolve<int32_t, true>(fd, lab, ws, flag.p, 0, rows, cols, &rounds, s)));     // h[8] is valid
+    if (*(int *)(host_flags().h + 8)) {
+        MS_CUDA(cudaMemcpyAsync(ws, lab, (size_t)(rows * cols) * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+        return watersheds_dev_t<int32_t>(fd, ws, rows, cols, 0, stats, s);
+    }
+    if (stats) stats[6] = rounds;
+    return MS_OK;
 }
 
 
@@ -289,7 +323,7 @@ int ms_band_ws_local_dev(ms_band *B, const uint8_t *fd, const int32_t *labelled,
     MS_TRY(flag.alloc(1, s));
     MS_CUDA(cudaMemsetAsync(flag.p, 0, sizeof(int), s));
     int64_t *h = host_flags().h;
-    MS_TRY(ws_resolve<int32_t>(fd, labelled, ptr, flag.p, unassigned, rows, cols, nullptr, s));
+    MS_TRY((ws_resolve<int32_t, false>(fd, labelled, ptr, flag.p, unassigned, rows, cols, nullptr, s)));
     if (*(int *)(h + 8)) {
         set_error("band watersheds: an interior cell without flow direction (band mode needs every path to end on "
                   "the raster border)");
@@ -468,7 +502,7 @@ static int pp_network_t(const uint8_t *fd, const L *lab, int64_t rows, int64_t c
         bool forest = has_bg && !path_len && np >= 64;
         if (forest) {
             MS_TRY(ptr.alloc((size_t)n, s));
-            MS_TRY(ws_resolve<L>(fd, lab, ptr.p, nullptr, (L)bg, rows, cols, nullptr, s));
+            MS_TRY((ws_resolve<L, false>(fd, lab, ptr.p, nullptr, (L)bg, rows, cols, nullptr, s)));
             prof_units(np);
             MS_LAUNCH((k_pp_downstream<L, true>), grid, 128, 0, s, fd, lab, ptr.p, (int)rows, (int)cols, np, pp_row,
                       pp_col, (L)bg, has_bg, down, found, path_len, (const int64_t *)nullptr, (int64_t *)nullptr,

@@ -10,8 +10,11 @@ namespace ms {
 // K5/K6.  label.connected_components (label.py:19-40 -> scipy.ndimage.label, full 3x3 structure):
 // foreground = value != 0 (NaN and denormals are foreground, -0.0 is not), 8-connectivity, int32 labels
 // numbered 1..n by each component's first cell in row-major order.  Union-find over cell indices where a
-// union always hangs the larger root under the smaller, so every component's root is its minimum index;
-// an exclusive scan of the root flags in raster order then gives scipy's numbering.
+// union always hangs the larger root under the smaller, so every component's root is its minimum index, and
+// numbering the roots in raster order gives scipy's numbering.  The roots are kept as one 64-bit mask per 64-cell
+// row segment of a tile (`roots`, rows x tiles_x words): the tile pass sets a bit for each tile-local root, the
+// border pass clears it when the root is hung under another.  A scan of the masks' popcounts gives every
+// segment's first number, and a root's number is that plus the roots left of it in its segment.
 // ------------------------------------------------------------------------------------------------
 template <typename T>
 __device__ inline bool is_fg(T v) { return v != (T)0; }
@@ -22,14 +25,23 @@ __device__ inline int cc_find(const int *parent, int x) {
     return x;
 }
 
-__device__ inline void cc_union(int *parent, int a, int b) {
+constexpr int CT = 64;
+
+// roots (optional): b's bit goes when b stops being a root, which happens at most once (parents only decrease)
+__device__ inline void cc_union(int *parent, int a, int b, unsigned long long *roots, int cols, int tiles_x) {
     for (;;) {
         a = cc_find(parent, a);
         b = cc_find(parent, b);
         if (a == b) return;
         if (a > b) { int t = a; a = b; b = t; }
         int old = atomicMin(parent + b, a);      // b was a root: hang it under the smaller root a
-        if (old == b) return;
+        if (old == b) {
+            if (roots) {
+                int r = b / cols, c = b - r * cols;
+                atomicAnd(roots + (size_t)r * tiles_x + c / CT, ~(1ull << (c % CT)));
+            }
+            return;
+        }
         b = old;                                  // somebody re-parented b meanwhile: retry from there
     }
 }
@@ -37,7 +49,6 @@ __device__ inline void cc_union(int *parent, int a, int b) {
 // Tile-local phase: one CTA labels a 64x64 tile in shared memory with the same union-find (row runs pre-linked,
 // atomicMin hooking, smaller index wins), then writes each cell's tile-local root as a GLOBAL cell index.  Only the
 // cells on tile edges are merged through global memory afterwards (k_cc_border): 3 % of the raster instead of all.
-constexpr int CT = 64;
 
 // Shared-memory layout of the tile forest: one pad word per 16 cells.  A thread owns 16 consecutive cells, so with
 // the plain layout the lanes of a warp would sit 16 words apart (2 banks in use, 16-way conflicts on every access);
@@ -62,8 +73,11 @@ __device__ inline void cc_union_s(int *p, int a, int b) {
     }
 }
 
+// roots (optional): the row-segment root masks.  Six CTAs per SM: with the mask loop ptxas would take 58 registers
+// (four CTAs); capped, it keeps the 40 of the form without it and does not spill.
 template <typename T>
-__global__ void __launch_bounds__(256) k_cc_tile(const T *__restrict__ data, int *__restrict__ parent, int rows, int cols,
+__global__ void __launch_bounds__(256, 6) k_cc_tile(const T *__restrict__ data, int *__restrict__ parent,
+                                                 unsigned long long *__restrict__ roots, int rows, int cols,
                                                  int tiles_x) {
     __shared__ int sp[CT * CT + CT * CT / 16];
     int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
@@ -142,12 +156,22 @@ __global__ void __launch_bounds__(256) k_cc_tile(const T *__restrict__ data, int
         int rr = r0 + (k >> 6), cc = c0 + (k & 63);
         if (rr < rows && cc < cols) parent[(size_t)rr * cols + cc] = sp[cpad(k)];
     }
+    if (!roots) return;
+    // a warp holds half a row of the tile: its ballot of the tile-local roots is that half of the row's root mask
+#pragma unroll 1
+    for (int u = 0; u < 16; u++) {
+        int k = tid + 256 * u;
+        int rr = r0 + (k >> 6), cc = c0 + (k & 63);
+        unsigned b = __ballot_sync(0xffffffffu, rr < rows && cc < cols && sp[cpad(k)] == rr * cols + cc);
+        if ((tid & 31) == 0 && rr < rows) ((unsigned *)roots)[((size_t)rr * tiles_x + tx) * 2 + ((k >> 5) & 1)] = b;
+    }
 }
 
 // merges across tile edges: cells of a tile's first row look up (3 neighbours), cells of its first column look left.
 // One CTA of 128 threads per tile: threads 0..63 are the tile's first row, 64..127 its first column (the raster is not
 // swept for the 3 % of cells that have something to do).
-__global__ void __launch_bounds__(128) k_cc_border(int *parent, int rows, int cols, int tiles_x) {
+__global__ void __launch_bounds__(128) k_cc_border(int *parent, unsigned long long *roots, int rows, int cols,
+                                                   int tiles_x) {
     int ty = blockIdx.x / tiles_x, tx = blockIdx.x - ty * tiles_x;
     int t = threadIdx.x & 63;
     bool top = threadIdx.x < 64;
@@ -158,14 +182,14 @@ __global__ void __launch_bounds__(128) k_cc_border(int *parent, int rows, int co
     if (top) {
         if (r == 0) return;
         int up = i - cols;
-        if (c > 0 && parent[up - 1] >= 0) cc_union(parent, i, up - 1);
-        if (parent[up] >= 0) cc_union(parent, i, up);
-        if (c < cols - 1 && parent[up + 1] >= 0) cc_union(parent, i, up + 1);
+        if (c > 0 && parent[up - 1] >= 0) cc_union(parent, i, up - 1, roots, cols, tiles_x);
+        if (parent[up] >= 0) cc_union(parent, i, up, roots, cols, tiles_x);
+        if (c < cols - 1 && parent[up + 1] >= 0) cc_union(parent, i, up + 1, roots, cols, tiles_x);
     } else {
         if (c == 0) return;
-        if (r > 0 && parent[i - cols - 1] >= 0) cc_union(parent, i, i - cols - 1);
-        if (parent[i - 1] >= 0) cc_union(parent, i, i - 1);
-        if (r < rows - 1 && parent[i + cols - 1] >= 0) cc_union(parent, i, i + cols - 1);
+        if (r > 0 && parent[i - cols - 1] >= 0) cc_union(parent, i, i - cols - 1, roots, cols, tiles_x);
+        if (parent[i - 1] >= 0) cc_union(parent, i, i - 1, roots, cols, tiles_x);
+        if (r < rows - 1 && parent[i + cols - 1] >= 0) cc_union(parent, i, i + cols - 1, roots, cols, tiles_x);
     }
 }
 
@@ -182,30 +206,47 @@ __global__ void __launch_bounds__(256) k_cc_flatten(int *parent, int *flag, int6
     if (flag) flag[i] = f;
 }
 
-__global__ void __launch_bounds__(256) k_cc_number(const int *__restrict__ parent, const int *__restrict__ rank,
-                                                   int32_t *__restrict__ labels, int64_t n) {
+__global__ void __launch_bounds__(256) k_cc_seg_count(const unsigned long long *__restrict__ roots, int *cnt,
+                                                      int64_t nseg) {
+    int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < nseg) cnt[k] = __popcll(roots[k]);
+}
+
+// label of a root = roots in the segments before its own (base) + roots left of it in its segment + 1
+__global__ void __launch_bounds__(256) k_cc_number(const int *__restrict__ parent,
+                                                   const unsigned long long *__restrict__ roots,
+                                                   const int *__restrict__ base, int32_t *__restrict__ labels,
+                                                   int64_t n, int cols, int tiles_x) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     int p = parent[i];
-    labels[i] = p < 0 ? 0 : rank[cc_find(parent, p)] + 1;
+    int32_t v = 0;
+    if (p >= 0) {
+        int root = cc_find(parent, p);
+        int r = root / cols, c = root - r * cols;
+        size_t seg = (size_t)r * tiles_x + c / CT;
+        v = base[seg] + __popcll(roots[seg] & ((1ull << (c % CT)) - 1ull)) + 1;
+    }
+    labels[i] = v;
 }
 
 template <typename T>
 int cc_dev_t(const T *data, int32_t *labels, int64_t rows, int64_t cols, int64_t *nlabels_dev, cudaStream_t s) {
     int64_t n = rows * cols;
-    DevBuf<int> parent, flag;
-    MS_TRY(parent.alloc((size_t)n, s));
-    MS_TRY(flag.alloc((size_t)n, s));
-    dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
-    unsigned g1 = cdiv(n, 256);
     int tiles_x = (int)cdiv(cols, CT), tiles_y = (int)cdiv(rows, CT);
+    int64_t nseg = rows * tiles_x;
+    DevBuf<int> parent, base;
+    DevBuf<unsigned long long> roots;
+    MS_TRY(parent.alloc((size_t)n, s));
+    MS_TRY(roots.alloc((size_t)nseg, s));
+    MS_TRY(base.alloc((size_t)nseg, s));
     prof_units(n);
-    MS_LAUNCH(k_cc_tile<T>, tiles_x * tiles_y, 256, 0, s, data, parent.p, (int)rows, (int)cols, tiles_x);
-    MS_LAUNCH(k_cc_border, tiles_x * tiles_y, 128, 0, s, parent.p, (int)rows, (int)cols, tiles_x);
-    // roots are the cells that point at themselves, flattened or not: number them in raster order, then every cell
-    // walks its (2-4 hop) chain once and takes its root's number — no separate flattening pass
-    MS_TRY(exclusive_scan_selfptr(parent.p, flag.p, n, nlabels_dev, s));
-    MS_LAUNCH(k_cc_number, g1, 256, 0, s, parent.p, flag.p, labels, n);
+    MS_LAUNCH(k_cc_tile<T>, tiles_x * tiles_y, 256, 0, s, data, parent.p, roots.p, (int)rows, (int)cols, tiles_x);
+    MS_LAUNCH(k_cc_border, tiles_x * tiles_y, 128, 0, s, parent.p, roots.p, (int)rows, (int)cols, tiles_x);
+    // every cell walks its (2-4 hop) chain once and takes its root's number — no separate flattening pass
+    MS_LAUNCH(k_cc_seg_count, cdiv(nseg, 256), 256, 0, s, roots.p, base.p, nseg);
+    MS_TRY(exclusive_scan_i32(base.p, base.p, nseg, nlabels_dev, s));
+    MS_LAUNCH(k_cc_number, cdiv(n, 256), 256, 0, s, parent.p, roots.p, base.p, labels, n, (int)cols, tiles_x);
     return MS_OK;
 }
 
@@ -276,8 +317,10 @@ int cc_band_local_t(ms_band *B, const T *data, int64_t cell_offset, int64_t *roo
     if (!parent || !rank) return MS_ERR_CUDA;
     dim3 g2(cdiv(cols, 64), cdiv(rows, 4));
     int tiles_x = (int)cdiv(cols, CT), tiles_y = (int)cdiv(rows, CT);
-    MS_LAUNCH(k_cc_tile<T>, tiles_x * tiles_y, 256, 0, s, data, parent, (int)rows, (int)cols, tiles_x);
-    MS_LAUNCH(k_cc_border, tiles_x * tiles_y, 128, 0, s, parent, (int)rows, (int)cols, tiles_x);
+    MS_LAUNCH(k_cc_tile<T>, tiles_x * tiles_y, 256, 0, s, data, parent, (unsigned long long *)nullptr, (int)rows,
+              (int)cols, tiles_x);
+    MS_LAUNCH(k_cc_border, tiles_x * tiles_y, 128, 0, s, parent, (unsigned long long *)nullptr, (int)rows, (int)cols,
+              tiles_x);
     MS_LAUNCH(k_cc_flatten, cdiv(n, 256), 256, 0, s, parent, rank, n);
     MS_LAUNCH(k_cc_edge_roots, cdiv(cols, 256), 256, 0, s, parent, cell_offset, (int)rows, (int)cols, root_top, root_bot);
     return MS_OK;

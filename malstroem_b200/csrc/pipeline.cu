@@ -16,8 +16,8 @@ int fill_no_flats_dev_impl(const float *dtm, const float *filled, double sh, dou
                            int64_t cols, int64_t *stats, cudaStream_t s, uint8_t *flowdir_out, int *flowdir_done);
 int flowdir_dev_impl(const double *t, uint8_t *out, int64_t rows, int64_t cols, int edges, cudaStream_t s, int open);
 int accum_dev_impl(const uint8_t *fd, double *acc, int64_t rows, int64_t cols, cudaStream_t s);
-int watersheds_dev_impl(const uint8_t *fd, void *lab, int label_bytes, int64_t rows, int64_t cols, int64_t unassigned,
-                        int64_t *stats, cudaStream_t s);
+int watersheds_labels_dev_impl(const uint8_t *fd, const int32_t *lab, int32_t *ws, int64_t rows, int64_t cols,
+                               int64_t *stats, cudaStream_t s);
 int cc_dev_impl(const void *data, int dtype, int32_t *labels, int64_t rows, int64_t cols, int64_t *nlabels_dev,
                 cudaStream_t s);
 int label_stats_dev_impl(const void *data, int dtype, const int32_t *lab, int64_t n, int64_t nlabels, double *omin,
@@ -201,8 +201,7 @@ extern "C" int ms_pipeline_filtered_host_dev(ms_rasters *io, const ms_host_out *
         MS_TRY(label_stats_dev_impl(io->depths, MS_F32, io->labels, n, io->nlabels, io->st_min, io->st_max, io->st_sum,
                                     io->st_count, err.p, s));
     // bluespots.py:183-186
-    MS_CUDA(cudaMemcpyAsync(io->wsheds, io->labels, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
-    MS_TRY(watersheds_dev_impl(io->flowdir, io->wsheds, 4, rows, cols, 0, io->stats, s));
+    MS_TRY(watersheds_labels_dev_impl(io->flowdir, io->labels, io->wsheds, rows, cols, io->stats, s));
     MS_TRY(ship(host->wsheds, io->wsheds, (size_t)n * sizeof(int32_t), s));
     if (fused) {
         // bluespots.py:160, 186, 195-206 (both pour-point variants)

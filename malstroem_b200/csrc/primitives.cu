@@ -12,9 +12,6 @@ constexpr int SCAN_T = 256;
 constexpr int SCAN_I = 16;
 constexpr int SCAN_CH = SCAN_T * SCAN_I;
 
-// SELF = false: the values themselves.  SELF = true: the flag "p[i] == i" (roots of a parent-pointer array), so that
-// the fill's and the labelling's numbering scans read the pointers directly instead of a materialised flag raster.
-template <bool SELF>
 __device__ inline void load16(const int *p, int64_t base, int64_t n, int v[SCAN_I]) {
     if (base + SCAN_I <= n) {
         const int4 *q = reinterpret_cast<const int4 *>(p + base);
@@ -27,10 +24,7 @@ __device__ inline void load16(const int *p, int64_t base, int64_t n, int v[SCAN_
 #pragma unroll
         for (int k = 0; k < SCAN_I; k++) v[k] = (base + k < n) ? p[base + k] : -1;
     }
-    if (SELF) {
-#pragma unroll
-        for (int k = 0; k < SCAN_I; k++) v[k] = (v[k] == (int)(base + k)) ? 1 : 0;
-    } else if (base + SCAN_I > n) {
+    if (base + SCAN_I > n) {
 #pragma unroll
         for (int k = 0; k < SCAN_I; k++) if (base + k >= n) v[k] = 0;
     }
@@ -66,11 +60,10 @@ __device__ inline int block_exclusive_scan(int x, int *total) {
     return r;
 }
 
-template <bool SELF>
 __global__ void __launch_bounds__(SCAN_T) k_scan_reduce(const int *in, int64_t n, int *bsum) {
     int64_t base = (int64_t)blockIdx.x * SCAN_CH + (int64_t)threadIdx.x * SCAN_I;
     int v[SCAN_I];
-    load16<SELF>(in, base, n, v);
+    load16(in, base, n, v);
     int s = 0;
 #pragma unroll
     for (int k = 0; k < SCAN_I; k++) s += v[k];
@@ -116,11 +109,10 @@ __global__ void __launch_bounds__(1024) k_scan_bsums(int *bsum, int nb, int64_t 
     if (threadIdx.x == 0) *total = (int64_t)carry_s;
 }
 
-template <bool SELF>
 __global__ void __launch_bounds__(SCAN_T) k_scan_final(const int *in, int *out, int64_t n, const int *bsum) {
     int64_t base = (int64_t)blockIdx.x * SCAN_CH + (int64_t)threadIdx.x * SCAN_I;
     int v[SCAN_I];
-    load16<SELF>(in, base, n, v);
+    load16(in, base, n, v);
     int s = 0;
 #pragma unroll
     for (int k = 0; k < SCAN_I; k++) s += v[k];
@@ -146,19 +138,9 @@ int exclusive_scan_i32(const int *flags, int *out, int64_t n, int64_t *total_dev
     int nb = (int)cdiv(n, SCAN_CH);
     DevBuf<int> bsum;
     MS_TRY(bsum.alloc((size_t)nb, s));
-    MS_LAUNCH(k_scan_reduce<false>, nb, SCAN_T, 0, s, flags, n, bsum.p);
+    MS_LAUNCH(k_scan_reduce, nb, SCAN_T, 0, s, flags, n, bsum.p);
     MS_LAUNCH(k_scan_bsums, 1, 1024, 0, s, bsum.p, nb, total_dev);
-    MS_LAUNCH(k_scan_final<false>, nb, SCAN_T, 0, s, flags, out, n, bsum.p);
-    return MS_OK;
-}
-
-int exclusive_scan_selfptr(const int *ptr, int *out, int64_t n, int64_t *total_dev, cudaStream_t s) {
-    int nb = (int)cdiv(n, SCAN_CH);
-    DevBuf<int> bsum;
-    MS_TRY(bsum.alloc((size_t)nb, s));
-    MS_LAUNCH(k_scan_reduce<true>, nb, SCAN_T, 0, s, ptr, n, bsum.p);
-    MS_LAUNCH(k_scan_bsums, 1, 1024, 0, s, bsum.p, nb, total_dev);
-    MS_LAUNCH(k_scan_final<true>, nb, SCAN_T, 0, s, ptr, out, n, bsum.p);
+    MS_LAUNCH(k_scan_final, nb, SCAN_T, 0, s, flags, out, n, bsum.p);
     return MS_OK;
 }
 
