@@ -616,7 +616,8 @@ int label_stats_dev_impl(const void *data, int dtype, const int32_t *lab, int64_
 // ------------------------------------------------------------------------------------------------
 // K8' / K8''.  label.label_min_index / label_max_index (label.py:101-166; speedups/_label.pyx:99-128):
 // strict comparison while scanning in raster order, so among equal extreme values the smallest flat
-// index wins; NaN never wins; labels never seen keep (+-inf, -1, -1).  Two passes: the extreme ordered
+// index wins; NaN never wins, and neither does the start value itself (+inf for the minimum, -inf for the
+// maximum); labels never seen, or seen only with such values, keep (+-inf, -1, -1).  Two passes: the extreme ordered
 // key per label, then the smallest index among the cells that hold it.  (-0.0 and +0.0 share a key, as
 // they compare equal; the reported value is read back from the winning cell.)
 // ------------------------------------------------------------------------------------------------
@@ -629,7 +630,7 @@ __global__ void __launch_bounds__(256) k_extreme_key(const double *__restrict__ 
         int lbl = lab[i];
         double v = data[i];
         if (lbl < 0 || lbl > nlabels) { *err = 1; continue; }
-        if (v != v) continue;
+        if (!(MAX ? v > -INFINITY : v < INFINITY)) continue;      // NaN or the start value: never wins
         unsigned long long k = okey64(v);
         if (lbl == 0) {
             bg = MAX ? (k > bg ? k : bg) : (k < bg ? k : bg);
@@ -838,10 +839,10 @@ __global__ void __launch_bounds__(256) k_tables_a2(const float *__restrict__ dep
                 if (vok) { rmin = k < rmin ? k : rmin; rmax = k > rmax ? k : rmax; }
                 rsum += (double)v;
                 rcnt++;
-                const unsigned long long fk = (f == f) ? okey64(f) : ~0ull;
+                const unsigned long long fk = (f < INFINITY) ? okey64(f) : ~0ull;     // NaN and +inf never win (K8')
                 rkmin = fk < rkmin ? fk : rkmin;
                 if (ACC) {
-                    const unsigned long long ak = (a == a) ? okey64(a) : 0ull;
+                    const unsigned long long ak = (a > -INFINITY) ? okey64(a) : 0ull;
                     rkmax = ak > rkmax ? ak : rkmax;
                 }
             }
@@ -913,10 +914,11 @@ __global__ void __launch_bounds__(256) k_tables_b(const int32_t *__restrict__ la
         int lbl = lab[i];
         if (lbl < 0 || lbl > nlabels) continue;
         double f = fnf[i];
-        if (f == f && okey64(f) == kmin[lbl] && (int)i < imin[lbl]) atomicMin(imin + lbl, (int)i);
+        // infinities stay out as in pass A: ms_band_tables_b_dev hands a label without an extreme the key of +inf / -inf
+        if (f < INFINITY && okey64(f) == kmin[lbl] && (int)i < imin[lbl]) atomicMin(imin + lbl, (int)i);
         if (ACC) {
             double a = accum[i];
-            if (a == a && okey64(a) == kmax[lbl] && (int)i < imax[lbl]) atomicMin(imax + lbl, (int)i);
+            if (a > -INFINITY && okey64(a) == kmax[lbl] && (int)i < imax[lbl]) atomicMin(imax + lbl, (int)i);
         }
     }
 }

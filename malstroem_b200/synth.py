@@ -204,6 +204,16 @@ def speckle_mask(rows, cols, density=0.39, seed=1):
     return np.random.default_rng(seed).random((rows, cols)) < density
 
 
+def pit_lattice_dem(rows, cols, seed=1):
+    """Level ground at 10 with a one-cell pit on every cell of odd row and odd column away from the border.  No two
+    pits touch, even diagonally, so each is a bluespot of its own: 1024 in a 64 x 64 tile, more than the 256-slot
+    per-tile tables of the label-table pass hold.  Pit floors are 1 .. 9, seeded."""
+    dem = np.full((rows, cols), 10.0, np.float32)
+    pits = dem[1:rows - 1:2, 1:cols - 1:2]
+    pits[...] = np.random.default_rng(seed).integers(1, 10, pits.shape).astype(np.float32)
+    return dem
+
+
 def pit_chain_dem(rows, cols, period=64):
     """Walls of 100 and one channel down column cols // 2: a pit in the middle of every `period` rows, a rim of two
     cells on every multiple of `period` rows, the rims falling by one per period away from the outlet at row 0 (so

@@ -134,6 +134,16 @@ def cross_band_ties(want, nbands):
     return out
 
 
+def labels_per_tile(lab, tile=64):
+    """The number of distinct nonzero labels in each tile x tile tile (flat, row-major over the tiles)."""
+    rows, cols = lab.shape
+    tiles_x = -(-cols // tile)
+    r, c = np.nonzero(lab)
+    top = int(lab.max()) + 1
+    key = ((r // tile) * tiles_x + c // tile) * top + lab[r, c]
+    return np.bincount(np.unique(key) // top, minlength=tiles_x * -(-rows // tile))
+
+
 def chain_spills_on_edges(dem, depths, nbands):
     """Pits (cells lower than all eight neighbours, inside a bluespot) whose spill along their column - the lower of
     the two crests met walking up and down the column from the pit - lies on one of the two rows of a band edge."""
@@ -182,6 +192,7 @@ CASES = {
     "serpentine_pit": (lambda: synth.serpentine_dem(1024, 512, 4, pit=True), (3, 8)),
     "comb": (lambda: synth.mask_dem(synth.comb_mask(960, 515)), (2, 5, 8)),
     "speckle": (lambda: synth.mask_dem(synth.speckle_mask(960, 515)), (2, 5, 8)),
+    "pit_lattice": (lambda: synth.pit_lattice_dem(320, 258), (2, 3)),
 }
 CASE_BANDS = [(name, nb) for name, (_, nbs) in CASES.items() for nb in nbs]
 
@@ -223,3 +234,7 @@ def assert_reach(name, nb):
             assert split_in_first_band(lab, nb)
         else:
             assert (band_presence(lab, nb).sum(1) >= 2).sum() >= 15 * (nb - 1)     # 17 / 87 / 179
+    elif name == "pit_lattice":
+        # more bluespots (and watersheds) in a 64 x 64 tile than the per-tile tables of the label-table pass hold
+        # (1024 in a full tile)
+        assert labels_per_tile(lab).max() > 256 and labels_per_tile(want["wsheds"]).max() > 256

@@ -189,6 +189,11 @@ def test_label_functions_edge_cases():
     data = rng.standard_normal((77, 131))
     data[rng.random((77, 131)) < 0.2] = 0.5          # ties: first cell in raster order must win
     data[3, 4] = -0.0
+    # a label whose only values are +inf has no arg-min, one whose only values are -inf no arg-max (strict comparison
+    # against the +inf / -inf start value); elsewhere the infinities are extremes
+    data[lab == 5] = np.inf
+    data[lab == 6] = -np.inf
+    data[7, 8], data[9, 10] = np.inf, -np.inf
     for nl in (None, 39, 60):                         # tables longer than the labels present
         check_index(label.label_min_index(data, lab, nl), port.label_min_index(data, lab, nl))
         check_index(label.label_max_index(data, lab, nl), port.label_max_index(data, lab, nl))
@@ -254,12 +259,15 @@ def test_pipeline_matches_functions():
     m = n + 1
     st = port.label_stats(dep, lab)
     assert np.array_equal(h["st_min"].numpy()[:m], st["min"]) and np.array_equal(h["st_count"].numpy()[:m], st["count"])
+    assert np.array_equal(h["st_max"].numpy()[:m], st["max"])
     np.testing.assert_allclose(h["st_sum"].numpy()[:m], st["sum"], rtol=SUM_RTOL)
     assert np.array_equal(h["ws_count"].numpy()[:m], port.label_count(ws))
     mi = port.label_min_index(fnf, lab, n)
     assert np.array_equal(h["ppmin_row"].numpy()[:m], mi["row"]) and np.array_equal(h["ppmin_col"].numpy()[:m], mi["col"])
+    assert np.array_equal(h["ppmin_value"].numpy()[:m], mi["value"])
     ma = port.label_max_index(acc, lab, n)
     assert np.array_equal(h["ppmax_row"].numpy()[:m], ma["row"]) and np.array_equal(h["ppmax_col"].numpy()[:m], ma["col"])
+    assert np.array_equal(h["ppmax_value"].numpy()[:m], ma["value"])
 
 
 # ---------------------------------------------------------------- sizes beyond the CPU oracle: certificates
