@@ -441,6 +441,15 @@ int ms_tiff_decode_dev(const void *in, const uint64_t *in_off, const uint32_t *i
                        int block_h, int sample_bytes, int sample_format, int predictor, void *scratch, void *raster,
                        int64_t rows, int64_t cols, int subst_mode, double nodata, double subst, int compressed,
                        void *stream);
+/* ms_tiff_decode_rows_dev: one window of file rows, for a row band (RasterReader.read_rows).  The nblocks streams are
+ * the whole block rows from block row block_row0 on (k * blocks_x tiles, or k strips) and must cover file rows
+ * [out_row0, out_row0 + out_rows); `raster` is out_rows x cols and receives them, file row r at raster row
+ * r - out_row0; `rows` stays the file's row count.  The short last strip of a striped file is accepted only when the
+ * window's block rows include the file's last one.  ms_tiff_decode_dev is the window (0, 0, rows). */
+int ms_tiff_decode_rows_dev(const void *in, const uint64_t *in_off, const uint32_t *in_len, int64_t nblocks,
+                            int block_w, int block_h, int sample_bytes, int sample_format, int predictor, void *scratch,
+                            void *raster, int64_t rows, int64_t cols, int64_t block_row0, int64_t out_row0,
+                            int64_t out_rows, int subst_mode, double nodata, double subst, int compressed, void *stream);
 
 /* ---- SURVEY.md 8(f4): label polygonisation.  Replaces vector.py:42-87 (vectorize_labels_file), i.e.
  * gdal.Polygonize(band, band.GetMaskBand(), layer, 0, ['8CONNECTED=8']): one polygon per 8-connected (connect8 = 0:

@@ -119,6 +119,8 @@ SIGNATURES = {
     "ms_tiff_pack_dev": (c_int, [c_p, c_i64, c_p, c_p, c_i64, c_p, c_p]),
     "ms_tiff_decode_dev": (c_int, [c_p, c_p, c_p, c_i64, c_int, c_int, c_int, c_int, c_int, c_p, c_p, c_i64, c_i64,
                                    c_int, c_dbl, c_dbl, c_int, c_p]),
+    "ms_tiff_decode_rows_dev": (c_int, [c_p, c_p, c_p, c_i64, c_int, c_int, c_int, c_int, c_int, c_p, c_p, c_i64,
+                                        c_i64, c_i64, c_i64, c_i64, c_int, c_dbl, c_dbl, c_int, c_p]),
     "ms_polygonize_dev": (c_int, [c_p, c_i64, c_i64, c_int, c_int, ctypes.c_int32, c_p, c_p]),
     "ms_polygonize": (c_int, [c_p, c_i64, c_i64, c_int, c_int, ctypes.c_int32, c_p]),
     "ms_polygonize_fetch": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p, c_p]),

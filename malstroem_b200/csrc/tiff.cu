@@ -445,20 +445,23 @@ __global__ void __launch_bounds__(128) k_tiff_inflate(const unsigned char *__res
 }
 
 // Undo the predictor per block row, crop into the raster, substitute nodata (io.py:69-71).  block = bw x bh samples
-// (tiles: 256 x 256; strips: image width x rows per strip), one thread per block row.
+// (tiles: 256 x 256; strips: image width x rows per strip), one thread per block row.  Block k of the call sits in
+// block row block_row0 + k / blocks_x of the file; only file rows [out_row0, out_row0 + out_rows) are written, file row
+// r to raster row r - out_row0.
 template <int ES>
 __global__ void __launch_bounds__(128) k_tiff_unpack(const unsigned char *__restrict__ blocks, size_t block_stride, int bw, int bh,
                                                      int blocks_x, int nblocks, int predictor, unsigned char *raster, int rows,
-                                                     int cols, int fmt, int subst_mode, double nodata, double subst) {
+                                                     int cols, int block_row0, int out_row0, int out_rows, int fmt,
+                                                     int subst_mode, double nodata, double subst) {
     typedef typename SampleT<ES>::T T;
     long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= (long long)nblocks * bh) return;
     int blk = (int)(g / bh), br = (int)(g - (long long)blk * bh);
     int by = blk / blocks_x, bx = blk - by * blocks_x;
-    int r = by * bh + br, c0 = bx * bw;
-    if (r >= rows) return;
+    int r = (block_row0 + by) * bh + br, c0 = bx * bw;
+    if (r >= rows || r < out_row0 || r >= out_row0 + out_rows) return;
     const T *src = reinterpret_cast<const T *>(blocks + (size_t)blk * block_stride) + (size_t)br * bw;
-    T *dst = reinterpret_cast<T *>(raster) + (size_t)r * cols + c0;
+    T *dst = reinterpret_cast<T *>(raster) + (size_t)(r - out_row0) * cols + c0;
     int n = min(bw, cols - c0);
     T acc = 0;
     for (int x = 0; x < n; x++) {
@@ -543,16 +546,14 @@ int ms_tiff_encode_dev(const void *raster, int sample_bytes, int64_t rows, int64
     return MS_OK;
 }
 
-/* RasterReader.read (io.py:52-72), the part that touches every byte: nblocks zlib streams (`in` + in_off[k], in_len[k]
- * bytes; all device) of blocks of block_w x block_h samples (tiles, or strips with block_w = cols) are inflated into
- * `scratch` (nblocks * block_w * block_h * sample_bytes bytes), the predictor is undone, the blocks are cropped into
- * the rows x cols raster and samples that are the file's nodata value (subst_mode 1: isclose(nodata); 2: isnan) are
- * replaced by `subst` (subst_mode 0: none).  sample_format: 1 unsigned, 2 signed, 3 float.  MS_ERR_ARG with the
- * index of the stream in the message when a stream is malformed. */
-int ms_tiff_decode_dev(const void *in, const uint64_t *in_off, const uint32_t *in_len, int64_t nblocks, int block_w,
-                       int block_h, int sample_bytes, int sample_format, int predictor, void *scratch, void *raster,
-                       int64_t rows, int64_t cols, int subst_mode, double nodata, double subst, int compressed,
-                       void *stream) {
+/* RasterReader.read_rows: the window of file rows [out_row0, out_row0 + out_rows) of ms_tiff_decode_dev.  The nblocks
+ * streams are the whole block rows from block row block_row0 on (k * blocks_x tiles, or k strips) and must cover the
+ * window; `raster` is out_rows x cols and receives the window, `rows` is the file's row count.  The last strip of a
+ * striped file may be short only when the call holds the file's last block row. */
+int ms_tiff_decode_rows_dev(const void *in, const uint64_t *in_off, const uint32_t *in_len, int64_t nblocks,
+                            int block_w, int block_h, int sample_bytes, int sample_format, int predictor, void *scratch,
+                            void *raster, int64_t rows, int64_t cols, int64_t block_row0, int64_t out_row0,
+                            int64_t out_rows, int subst_mode, double nodata, double subst, int compressed, void *stream) {
     using namespace ms;
     MS_TRY(ensure_init());
     if (!in || !in_off || !in_len || !scratch || !raster || nblocks < 1 || block_w < 1 || block_h < 1 || rows < 1 ||
@@ -560,17 +561,26 @@ int ms_tiff_decode_dev(const void *in, const uint64_t *in_off, const uint32_t *i
         set_error("tiff decode: bad argument");
         return MS_ERR_ARG;
     }
+    const int64_t blocks_x = cdiv(cols, block_w), block_rows = cdiv(rows, block_h), k = nblocks / blocks_x;
+    if (nblocks % blocks_x || block_row0 < 0 || block_row0 + k > block_rows || out_rows < 1 || out_row0 < block_row0 * block_h ||
+        out_row0 + out_rows > min(rows, (block_row0 + k) * block_h)) {
+        set_error("tiff decode: %lld blocks from block row %lld do not cover rows [%lld, %lld) of %lld",
+                  (long long)nblocks, (long long)block_row0, (long long)out_row0, (long long)(out_row0 + out_rows),
+                  (long long)rows);
+        return MS_ERR_ARG;
+    }
     cudaStream_t s = (cudaStream_t)stream;
     size_t block_bytes = (size_t)block_w * block_h * sample_bytes;
-    // strips (block_w == cols): the last one holds the remaining rows only; tiles are always whole
-    int64_t last_rows = rows - (cdiv(rows, block_h) - 1) * block_h;
-    size_t last_bytes = block_w >= cols ? (size_t)block_w * (size_t)last_rows * sample_bytes : block_bytes;
+    // strips (block_w == cols): the file's last one holds the remaining rows only; tiles are always whole
+    int64_t last_rows = rows - (block_rows - 1) * block_h;
+    size_t last_bytes = block_w >= cols && block_row0 + k == block_rows ? (size_t)block_w * (size_t)last_rows * sample_bytes
+                                                                        : block_bytes;
     const unsigned char *blocks = (const unsigned char *)scratch;
     if (compressed) {
         DevBuf<int> err;
         MS_TRY(err.alloc(1, s));
         MS_CUDA(cudaMemsetAsync(err.p, 0, sizeof(int), s));
-        prof_units(rows * cols);
+        prof_units(out_rows * cols);
         MS_LAUNCH(k_tiff_inflate, cdiv(nblocks, 4), 128, 0, s, (const unsigned char *)in, (const unsigned long long *)in_off,
                   in_len, (int)nblocks, (unsigned char *)scratch, block_bytes, (unsigned)block_bytes, (unsigned)last_bytes, err.p);
         int *h = (int *)host_flags().h;
@@ -578,17 +588,36 @@ int ms_tiff_decode_dev(const void *in, const uint64_t *in_off, const uint32_t *i
         MS_TRY(ms::stream_sync(s));
         if (*h) { set_error("tiff decode: stream %d is not a valid zlib stream of %zu bytes", *h - 1, block_bytes); return MS_ERR_ARG; }
     }
-    int blocks_x = (int)cdiv(cols, block_w);
     int64_t nthreads = nblocks * block_h;
     unsigned char *r8 = (unsigned char *)raster;
+#define MS_UNPACK(ES)                                                                                                    \
+    MS_LAUNCH(k_tiff_unpack<ES>, cdiv(nthreads, 128), 128, 0, s, blocks, block_bytes, block_w, block_h, (int)blocks_x,     \
+              (int)nblocks, predictor, r8, (int)rows, (int)cols, (int)block_row0, (int)out_row0, (int)out_rows,          \
+              sample_format, subst_mode, nodata, subst)
     switch (sample_bytes) {
-        case 1: MS_LAUNCH(k_tiff_unpack<1>, cdiv(nthreads, 128), 128, 0, s, blocks, block_bytes, block_w, block_h, blocks_x, (int)nblocks, predictor, r8, (int)rows, (int)cols, sample_format, subst_mode, nodata, subst); break;
-        case 2: MS_LAUNCH(k_tiff_unpack<2>, cdiv(nthreads, 128), 128, 0, s, blocks, block_bytes, block_w, block_h, blocks_x, (int)nblocks, predictor, r8, (int)rows, (int)cols, sample_format, subst_mode, nodata, subst); break;
-        case 4: MS_LAUNCH(k_tiff_unpack<4>, cdiv(nthreads, 128), 128, 0, s, blocks, block_bytes, block_w, block_h, blocks_x, (int)nblocks, predictor, r8, (int)rows, (int)cols, sample_format, subst_mode, nodata, subst); break;
-        case 8: MS_LAUNCH(k_tiff_unpack<8>, cdiv(nthreads, 128), 128, 0, s, blocks, block_bytes, block_w, block_h, blocks_x, (int)nblocks, predictor, r8, (int)rows, (int)cols, sample_format, subst_mode, nodata, subst); break;
+        case 1: MS_UNPACK(1); break;
+        case 2: MS_UNPACK(2); break;
+        case 4: MS_UNPACK(4); break;
+        case 8: MS_UNPACK(8); break;
         default: set_error("tiff decode: sample size %d", sample_bytes); return MS_ERR_ARG;
     }
+#undef MS_UNPACK
     return MS_OK;
+}
+
+/* RasterReader.read (io.py:52-72), the part that touches every byte: nblocks zlib streams (`in` + in_off[k], in_len[k]
+ * bytes; all device) of blocks of block_w x block_h samples (tiles, or strips with block_w = cols) are inflated into
+ * `scratch` (nblocks * block_w * block_h * sample_bytes bytes), the predictor is undone, the blocks are cropped into
+ * the rows x cols raster and samples that are the file's nodata value (subst_mode 1: isclose(nodata); 2: isnan) are
+ * replaced by `subst` (subst_mode 0: none).  sample_format: 1 unsigned, 2 signed, 3 float.  MS_ERR_ARG with the
+ * index of the stream in the message when a stream is malformed.  The whole file: the window (0, 0, rows) of
+ * ms_tiff_decode_rows_dev. */
+int ms_tiff_decode_dev(const void *in, const uint64_t *in_off, const uint32_t *in_len, int64_t nblocks, int block_w,
+                       int block_h, int sample_bytes, int sample_format, int predictor, void *scratch, void *raster,
+                       int64_t rows, int64_t cols, int subst_mode, double nodata, double subst, int compressed,
+                       void *stream) {
+    return ms_tiff_decode_rows_dev(in, in_off, in_len, nblocks, block_w, block_h, sample_bytes, sample_format, predictor,
+                                   scratch, raster, rows, cols, 0, 0, rows, subst_mode, nodata, subst, compressed, stream);
 }
 
 }  // extern "C"

@@ -10,7 +10,9 @@ the GeoTIFF citation string (written to and read from GTCitationGeoKey) instead 
 readers without GDAL's WKT parser (cv2, tifffile) are unaffected.  The vector half of io.py (OGR) is out of scope.
 There is no CPU fallback: read() / write() need the CUDA library.
 """
+import bisect
 import ctypes
+import os
 import struct
 
 import numpy as np
@@ -62,14 +64,19 @@ def _pack_value(typ, values):
     return struct.pack("<%d%s" % (len(vals), _TYPE_FMT[typ]), *vals), len(vals)
 
 
+def tiff_head_len(tile_sizes):
+    """Bytes before the first tile in build_tiff's file: 8 (classic TIFF) or 16 (BigTIFF, for 4 GB of data and up)."""
+    total = int(sum(int(s) for s in tile_sizes))
+    return 16 if total + 65536 + 16 * len(tile_sizes) >= (1 << 32) - (1 << 20) else 8
+
+
 def build_tiff(rows, cols, dtype, predictor, tile_sizes, transform=None, crs=None, nodata=None):
     """Header and tag directory of a tiled, deflate-compressed single-band TIFF whose tile data (the zlib streams, in
     tile order, one after the other) follows the header directly.  Returns (head bytes, tail bytes): the file is
     head + data + tail.  Classic TIFF below 4 GB, BigTIFF above (the reference's bigtiff='if_safer')."""
     fmt, bits = _DTYPES[np.dtype(dtype)]
-    total = int(sum(int(s) for s in tile_sizes))
-    big = total + 65536 + 16 * len(tile_sizes) >= (1 << 32) - (1 << 20)
-    head_len = 16 if big else 8
+    head_len = tiff_head_len(tile_sizes)
+    big = head_len == 16
     offsets, pos = [], head_len
     for s in tile_sizes:
         offsets.append(pos)
@@ -105,6 +112,44 @@ def build_tiff(rows, cols, dtype, predictor, tile_sizes, transform=None, crs=Non
     head = (b"II" + struct.pack("<HHHQ", 43, 8, 0, ifd_off)) if big else (b"II" + struct.pack("<HI", 42, ifd_off))
     tail = (b"\0" if (pos & 1) else b"") + ifd + extra
     return head, tail
+
+
+# ---------------------------------------------------------------------------------------- container: row bands
+def band_tile_plan(bands, rows):
+    """How row bands share the 256-row tile rows of one file.  bands: [(r0, r1)] in rank order, tiling [0, rows).
+    Tile row t belongs to the band that holds its first row 256 t.  Per rank a dict:
+      own    (t0, t1): the tile rows the band encodes;
+      inner  (t0, t1): those of `own` whose rows all lie in the band (encoded straight from the band's rows);
+      cross  the last tile row of `own` when it runs past the band's last row, else None;
+      send   (dest, a, b): rows [a, b) of the band, which the owner `dest` of the tile row that crosses the band's
+             first row lacks; None when the band starts on a tile row;
+      recv   [(src, a, b)] in rank order: the `send`s addressed to this band, together the rows of `cross` past the
+             band's last row.
+    Rows only travel towards lower ranks and may skip bands that own no tile row."""
+    ends = [int(b) for _, b in bands]
+    plans = []
+    for r0, r1 in bands:
+        t0, t1 = -(-r0 // TILE), -(-r1 // TILE)
+        cross = t1 - 1 if t1 > t0 and min(t1 * TILE, rows) > r1 else None
+        send = None
+        first = (r0 // TILE) * TILE
+        if r1 > r0 and first < r0:
+            send = (bisect.bisect_right(ends, first), r0, min(r1, first + TILE))
+        plans.append({"own": (t0, t1), "inner": (t0, t1 if cross is None else cross), "cross": cross, "send": send,
+                      "recv": []})
+    for g, p in enumerate(plans):
+        if p["send"] is not None:
+            plans[p["send"][0]]["recv"].append((g,) + p["send"][1:])
+    return plans
+
+
+def band_file_offsets(tile_sizes, band_tiles):
+    """File offset of every band's first tile in build_tiff's layout: tile_sizes of the whole file in tile order,
+    band_tiles = the number of tiles of each band, in rank order."""
+    cum = np.concatenate([[0], np.cumsum(np.asarray(tile_sizes, dtype=np.int64))])
+    first = np.concatenate([[0], np.cumsum(np.asarray(band_tiles, dtype=np.int64))])[:-1]
+    head = tiff_head_len(tile_sizes)
+    return [head + int(cum[k]) for k in first]
 
 
 # ------------------------------------------------------------------------------------------------- container: read
@@ -195,6 +240,12 @@ class TiffInfo(object):
 
 
 # ------------------------------------------------------------------------------------------------------- the classes
+def _np_dtype(data):
+    if isinstance(data, np.ndarray):
+        return data.dtype
+    return np.dtype(str(data.dtype).replace("torch.", ""))
+
+
 def _torch():
     import torch
     if not torch.cuda.is_available():
@@ -214,48 +265,94 @@ class RasterReader(object):
         self.nodata = self._info.nodata
         self.nodatasubst = nodatasubst
 
-    def read_device(self, device=0):
+    def _blocks(self, b0, b1, dev):
+        """Block rows [b0, b1) of the file on `dev`: (the compressed blocks one after the other, their offsets, their
+        lengths, the scratch the decode inflates into, the number of blocks).  Only these blocks are read, with seek +
+        readinto into one pinned buffer."""
         torch = _torch()
         t = self._info
-        dev = torch.device("cuda", device)
-        nblocks = len(t.offsets)
+        bx = -(-t.cols // t.block_w)
+        k0, k1 = b0 * bx, b1 * bx
+        if len(t.offsets) < k1 or len(t.counts) < k1:
+            raise ValueError("%s: %d blocks listed, %d needed" % (self.filepath, min(len(t.offsets), len(t.counts)), k1))
+        counts = t.counts[k0:k1]
+        nblocks = k1 - k0
         # the compressed blocks, one after the other, in one pinned buffer
-        total = sum(t.counts)
+        total = sum(counts)
         host = torch.empty(max(total, 1), dtype=torch.uint8).pin_memory()
         hv = host.numpy()
         offs = np.zeros(nblocks, np.uint64)
         pos = 0
         with open(self.filepath, "rb") as f:
             for k in range(nblocks):
-                f.seek(t.offsets[k])
-                f.readinto(memoryview(hv)[pos:pos + t.counts[k]])
+                f.seek(t.offsets[k0 + k])
+                f.readinto(memoryview(hv)[pos:pos + counts[k]])
                 offs[k] = pos
-                pos += t.counts[k]
+                pos += counts[k]
         block_bytes = t.block_w * t.block_h * t.sample_bytes
-        compressed = t.compression != 1
         d_in = host.to(dev, non_blocking=True)
         d_off = torch.from_numpy(offs.view(np.int64)).to(dev)
-        d_len = torch.from_numpy(np.asarray(t.counts, dtype=np.uint32).view(np.int32)).to(dev)
+        d_len = torch.from_numpy(np.asarray(counts, dtype=np.uint32).view(np.int32)).to(dev)
         scratch = torch.empty(nblocks * block_bytes, dtype=torch.uint8, device=dev)
-        if not compressed:
+        if t.compression == 1:
             # raw blocks: lined up at the block stride (the last strip may be short)
             for k in range(nblocks):
                 o = int(offs[k])
-                scratch[k * block_bytes:k * block_bytes + t.counts[k]] = d_in[o:o + t.counts[k]]
-        out = torch.empty((t.rows, t.cols), dtype=getattr(torch, np.dtype(t.dtype).name), device=dev)
-        # `if self.nodata and self.nodatasubst is not None` (io.py:69): a nodata value of 0 is never substituted
+                scratch[k * block_bytes:k * block_bytes + counts[k]] = d_in[o:o + counts[k]]
+        return d_in, d_off, d_len, scratch, nblocks
+
+    def _subst(self):
+        """(subst_mode, nodata, subst) of the decode.  `if self.nodata and self.nodatasubst is not None` (io.py:69):
+        a nodata value of 0 is never substituted."""
         mode = 0
         if self.nodata and self.nodatasubst is not None:
             mode = 2 if np.isnan(self.nodata) else 1
+        return (mode, float(self.nodata) if self.nodata is not None else 0.0,
+                float(self.nodatasubst) if self.nodatasubst is not None else 0.0)
+
+    def read_device(self, device=0):
+        torch = _torch()
+        t = self._info
+        dev = torch.device("cuda", device)
+        d_in, d_off, d_len, scratch, nblocks = self._blocks(0, -(-t.rows // t.block_h), dev)
+        out = torch.empty((t.rows, t.cols), dtype=getattr(torch, np.dtype(t.dtype).name), device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
         with _lib.lock:
             _lib.check(_lib.lib().ms_init(dev.index or 0), "ms_init")
             _lib.check(_lib.lib().ms_tiff_decode_dev(
                 d_in.data_ptr(), d_off.data_ptr(), d_len.data_ptr(), nblocks, t.block_w, t.block_h, t.sample_bytes,
-                t.sample_format, t.predictor, scratch.data_ptr(), out.data_ptr(), t.rows, t.cols, mode,
-                float(self.nodata) if self.nodata is not None else 0.0,
-                float(self.nodatasubst) if self.nodatasubst is not None else 0.0, 1 if compressed else 0,
-                ctypes.c_void_p(stream)), "RasterReader.read")
+                t.sample_format, t.predictor, scratch.data_ptr(), out.data_ptr(), t.rows, t.cols, *self._subst(),
+                1 if t.compression != 1 else 0, ctypes.c_void_p(stream)), "RasterReader.read")
+        return out
+
+    def read_rows(self, r0, r1, device=0, out=None):
+        """Rows [r0, r1) of the raster as a cuda tensor, the same values as read_device()[r0:r1], nodata substituted
+        alike.  Only the blocks (tiles or strips) that meet those rows are read from the file and decoded, so a row
+        band of a raster that no single device holds reads its own share of the file.  out: a contiguous tensor of
+        shape (r1 - r0, cols) and the file's dtype on `device` to decode into (for example BandPipeline.dem).  Not a
+        collective: every band reads on its own."""
+        t = self._info
+        r0, r1 = int(r0), int(r1)
+        if not 0 <= r0 < r1 <= t.rows:
+            raise ValueError("read_rows: rows [%d, %d) are not inside [0, %d)" % (r0, r1, t.rows))
+        torch = _torch()
+        dev = torch.device("cuda", device) if not isinstance(device, torch.device) else device
+        dt = getattr(torch, np.dtype(t.dtype).name)
+        if out is None:
+            out = torch.empty((r1 - r0, t.cols), dtype=dt, device=dev)
+        elif (tuple(out.shape) != (r1 - r0, t.cols) or out.dtype != dt or not out.is_contiguous()
+              or out.device != dev):
+            raise ValueError("read_rows: out must be a contiguous %s tensor of shape (%d, %d) on %s"
+                             % (dt, r1 - r0, t.cols, dev))
+        b0, b1 = r0 // t.block_h, -(-r1 // t.block_h)
+        d_in, d_off, d_len, scratch, nblocks = self._blocks(b0, b1, dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        with _lib.lock:
+            _lib.check(_lib.lib().ms_init(dev.index or 0), "ms_init")
+            _lib.check(_lib.lib().ms_tiff_decode_rows_dev(
+                d_in.data_ptr(), d_off.data_ptr(), d_len.data_ptr(), nblocks, t.block_w, t.block_h, t.sample_bytes,
+                t.sample_format, t.predictor, scratch.data_ptr(), out.data_ptr(), t.rows, t.cols, b0, r0, r1 - r0,
+                *self._subst(), 1 if t.compression != 1 else 0, ctypes.c_void_p(stream)), "RasterReader.read_rows")
         return out
 
     def read(self):
@@ -276,12 +373,8 @@ class RasterWriter(object):
         self.nodata = nodata
         self.stats = {}
 
-    def write(self, data, device=0):
-        torch = _torch()
-        if isinstance(data, np.ndarray):
-            dtype = data.dtype
-        else:
-            dtype = np.dtype(str(data.dtype).replace("torch.", ""))
+    def _predictor(self, dtype):
+        """The GDAL datatype (set on the first write) and the predictor the reference gives GDAL for `dtype`."""
         if not self.datatype:
             # io.py:124-136: the four types the reference knows, predictor 2 for all but float64
             if dtype == np.float64:
@@ -297,13 +390,18 @@ class RasterWriter(object):
                 self.options['predictor'] = 2
             else:
                 raise NotImplementedError("Cannot determine GDAL datatype for numpy datatype {}".format(dtype))
+        return int(self.options.get('predictor', 1))
+
+    def write(self, data, device=0):
+        torch = _torch()
+        dtype = _np_dtype(data)
+        predictor = self._predictor(dtype)
         if len(data.shape) != 2:
             raise ValueError("RasterWriter.write: a 2-D array is required")
         dev = torch.device("cuda", device)
         d = torch.from_numpy(np.ascontiguousarray(data)).to(dev) if isinstance(data, np.ndarray) else data.contiguous()
         rows, cols = int(d.shape[0]), int(d.shape[1])
         es = d.element_size()
-        predictor = int(self.options.get('predictor', 1))
         L = _lib.lib()
         tiles = (-(-rows // TILE)) * (-(-cols // TILE))
         with _lib.lock:
@@ -331,3 +429,196 @@ class RasterWriter(object):
             f.write(memoryview(host.numpy()))
             f.write(tail)
         self.stats = {"raw_bytes": rows * cols * es, "file_bytes": len(head) + total + len(tail), "tiles": tiles}
+
+    STAGE_BYTES = 64 << 20          # each of write_band's two pinned staging buffers
+    ENCODE_SLOT_BYTES = 1 << 30     # write_band's tile slots per encode call (at least one tile row)
+
+    def write_band(self, comm, band, r0, rows, device=0):
+        """Collective over `comm` (bands.ThreadComm or bands.DistComm): every rank passes its own `band`, rows
+        [r0, r0 + band.shape[0]) of a rows x cols raster, and together they write ONE file, byte for byte what write()
+        writes for the whole raster.  No rank holds more than its band:
+          * tile row t belongs to the band holding row 256 t (band_tile_plan); the band that owns the tile row across
+            its last row receives the rows it lacks (fewer than 256) from the following bands, all other tile rows are
+            encoded straight from the band's rows;
+          * the tile sizes (one int per tile) are gathered, every rank computes the same container and its own offset;
+            rank 0 creates the file with the header and its final size, then every rank writes its tiles at its
+            offset and rank 0 the tag directory.
+        Memory per rank: on the device, the band, its compressed tiles and at most ENCODE_SLOT_BYTES of tile slots; on
+        the host, two pinned staging buffers of STAGE_BYTES (the device-to-host copy of one overlaps the file write of
+        the other) and O(tiles of the file) for the sizes and the tag directory - independent of the raster's size
+        otherwise.  All ranks must see the same file system (one host).
+        Bands that do not tile [0, rows) in rank order, or disagree on cols or dtype, make every rank raise ValueError
+        before any device work; a failure on one rank (allocation, encode, an unwritable path, a short write) makes
+        every rank raise, and rank 0 removes the partial file."""
+        import torch
+        try:
+            dtype = _np_dtype(band)
+            code = list(_DTYPES).index(dtype) if dtype in _DTYPES else len(_DTYPES)
+        except TypeError:
+            dtype, code = None, -1
+        two_d = len(band.shape) == 2
+        r0, rows = int(r0), int(rows)
+        mine = [r0, r0 + int(band.shape[0]) if two_d else -1, int(band.shape[1]) if two_d else -1, code, rows]
+        where = band.device if isinstance(band, torch.Tensor) else torch.device("cpu")
+        got = comm.all_gather(torch.tensor(mine, dtype=torch.int64, device=where)).cpu().tolist()
+        bounds = [(a, b) for a, b, _, _, _ in got]
+        ok = (got[0][0] == 0 and got[-1][1] == rows and rows >= 1
+              and all(g[1] >= g[0] and g[2] >= 1 and g[2:] == got[0][2:] for g in got)
+              and all(got[k][0] == got[k - 1][1] for k in range(1, len(got))))
+        if not ok:
+            raise ValueError("write_band: the bands (r0, r1, cols, dtype, rows) %s do not tile the rows of one raster "
+                             "in rank order" % got)
+        torch = _torch()
+        predictor = self._predictor(dtype)
+        cols, r1, rank = got[0][2], bounds[comm.rank][1], comm.rank
+        dev = torch.device("cuda", device) if not isinstance(device, torch.device) else device
+        plans = band_tile_plan(bounds, rows)
+        plan = plans[rank]
+        tiles_x = -(-cols // TILE)
+        fail, made = [None], [False]
+
+        def agree():
+            """all ranks learn whether any rank failed; every rank raises (rank 0 removes the file it made first)"""
+            bad = comm.all_reduce(torch.tensor([0 if fail[0] is None else 1], dtype=torch.int32, device=dev), "max")
+            if int(bad.item()):
+                if made[0]:
+                    os.remove(self.filepath)
+                if fail[0] is not None:
+                    raise fail[0]
+                raise RuntimeError("write_band: %s: the write failed on another rank" % self.filepath)
+
+        L = _lib.lib()
+        try:
+            d = (torch.from_numpy(np.ascontiguousarray(band)) if isinstance(band, np.ndarray) else band)
+            d = d.to(dev).contiguous()
+            es = d.element_size()
+            u8 = d.view(torch.uint8)
+            with _lib.lock:
+                _lib.check(L.ms_init(dev.index or 0), "ms_init")
+                slot = int(L.ms_tiff_tile_slot(es))
+        except (RuntimeError, ValueError, OSError, MemoryError) as e:
+            fail[0] = e
+        agree()
+        # the rows of the tile row across each band's last row, from the bands that hold them
+        recv = None
+        if any(p["send"] is not None for p in plans):
+            chunks = [u8[:0]] * comm.size
+            if plan["send"] is not None:
+                dest, a, b = plan["send"]
+                chunks[dest] = u8[a - r0:b - r0]
+            got = comm.all_to_all_var(chunks)
+            if plan["recv"]:
+                recv = torch.cat([got[src] for src, _, _ in plan["recv"]])
+        stream = torch.cuda.current_stream(dev)
+        sizes_h, packed = [], []
+        ev = [torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)]
+        try:
+            ev[0].record(stream)
+            per = max(1, self.ENCODE_SLOT_BYTES // (tiles_x * slot))         # tile rows per encode call
+            slots = None
+
+            def encode(src):
+                nonlocal slots
+                n = -(-int(src.shape[0]) // TILE) * tiles_x
+                if slots is None or slots.numel() < n * slot:
+                    slots = torch.empty(min(per, plan["own"][1] - plan["own"][0]) * tiles_x * slot, dtype=torch.uint8,
+                                        device=dev)
+                sizes = torch.empty(n, dtype=torch.int32, device=dev)
+                st = ctypes.c_void_p(stream.cuda_stream)
+                with _lib.lock:
+                    _lib.check(L.ms_tiff_encode_dev(src.data_ptr(), es, int(src.shape[0]), cols, predictor,
+                                                    slots.data_ptr(), slot, sizes.data_ptr(), st), "write_band")
+                offs = torch.cumsum(sizes.long(), 0) - sizes.long()
+                h = sizes.cpu().numpy().astype(np.int64)
+                out = torch.empty(int(h.sum()), dtype=torch.uint8, device=dev)
+                with _lib.lock:
+                    _lib.check(L.ms_tiff_pack_dev(slots.data_ptr(), slot, sizes.data_ptr(), offs.data_ptr(), n,
+                                                  out.data_ptr(), st), "write_band")
+                sizes_h.append(h)
+                packed.append(out)
+
+            t0, t1 = plan["inner"]
+            for t in range(t0, t1, per):
+                a, b = t * TILE, min(min(t + per, t1) * TILE, rows)
+                encode(d[a - r0:b - r0])
+            if plan["cross"] is not None:
+                a = plan["cross"] * TILE
+                slab = torch.empty((min(a + TILE, rows) - a, cols), dtype=d.dtype, device=dev)
+                slab[:r1 - a] = d[a - r0:]
+                slab.view(torch.uint8)[r1 - a:] = recv
+                encode(slab)
+            ev[1].record(stream)
+        except (RuntimeError, ValueError, OSError, MemoryError) as e:
+            fail[0] = e
+        agree()
+        # the container: every rank computes the same one from the gathered sizes
+        mine = np.concatenate(sizes_h) if sizes_h else np.zeros(0, np.int64)
+        parts = comm.all_gather_var(torch.from_numpy(mine).to(dev))
+        band_tiles = [int(x.numel()) for x in parts]
+        tile_sizes = torch.cat(parts).cpu().numpy()
+        head, tail = build_tiff(rows, cols, dtype, predictor, tile_sizes, self.transform, self.crs, self.nodata)
+        data = int(tile_sizes.sum())
+        size = len(head) + data + len(tail)
+        offset = band_file_offsets(tile_sizes, band_tiles)[rank]
+        if rank == 0:
+            try:
+                with open(self.filepath, "wb") as f:
+                    made[0] = True
+                    f.write(head)
+                    f.truncate(size)
+            except OSError as e:
+                fail[0] = e
+        agree()
+        try:
+            fd = os.open(self.filepath, os.O_WRONLY)
+            try:
+                self._pwrite_device(fd, packed, offset, dev)
+                if rank == 0:
+                    _pwrite_all(fd, memoryview(tail), len(head) + data)
+            finally:
+                os.close(fd)
+        except (RuntimeError, ValueError, OSError, MemoryError) as e:
+            fail[0] = e
+        agree()
+        ev[1].synchronize()
+        self.stats = {"raw_bytes": rows * cols * es, "file_bytes": size, "tiles": len(tile_sizes),
+                      "band_tiles": band_tiles[rank], "band_bytes": int(mine.sum()),
+                      "exchanged_bytes": 0 if recv is None else recv.numel(), "encode_ms": ev[0].elapsed_time(ev[1])}
+
+    def _pwrite_device(self, fd, parts, offset, dev):
+        """The device tensors `parts` (uint8), one after the other, to `fd` at `offset`: device-to-host copies into two
+        pinned buffers of at most STAGE_BYTES taking turns, each copy overlapping the file write of the other buffer."""
+        import torch
+        total = sum(int(p.numel()) for p in parts)
+        if total == 0:
+            return
+        cap = min(self.STAGE_BYTES, total)
+        bufs = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        pieces = [(p, a, min(a + cap, int(p.numel()))) for p in parts for a in range(0, int(p.numel()), cap)]
+        side = torch.cuda.Stream(device=dev)
+        side.wait_stream(torch.cuda.current_stream(dev))
+        done = [None, None]
+
+        def issue(i):
+            p, a, b = pieces[i]
+            with torch.cuda.stream(side):
+                bufs[i % 2][:b - a].copy_(p[a:b], non_blocking=True)
+                done[i % 2] = torch.cuda.Event()
+                done[i % 2].record(side)
+
+        issue(0)
+        pos = offset
+        for i, (p, a, b) in enumerate(pieces):
+            if i + 1 < len(pieces):
+                issue(i + 1)            # the buffer of piece i - 1, whose write has returned
+            done[i % 2].synchronize()
+            _pwrite_all(fd, memoryview(bufs[i % 2].numpy())[:b - a], pos)
+            pos += b - a
+
+
+def _pwrite_all(fd, view, pos):
+    while len(view):
+        n = os.pwrite(fd, view, pos)
+        if n <= 0:
+            raise OSError("short write at byte %d" % pos)
+        view, pos = view[n:], pos + n
