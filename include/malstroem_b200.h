@@ -192,37 +192,29 @@ int ms_band_nf_verify_dev(ms_band *band, const float *dem, const double *fnf, do
  * then treats it as a lake cell, not as a seed) and their count is returned. */
 int ms_band_nf_ban_dev(ms_band *band, const float *dem, const double *fnf, double short_eps, double diag_eps, int reset,
                        int64_t *nviol, void *stream);
-/* The same solve fused over NVLink peer memory: every band's solver kernel runs at the same time and the bands feed
- * each other's tile queues and halo rows directly (system-scope atomics and stores into blocks mapped through CUDA
- * IPC), instead of one host-driven halo exchange per crossing of a band edge.  create: allocates the band's shared
- * block, info80 (HOST, 80 bytes) describes it; open: maps every rank's block (infos: world x 80 bytes gathered from
- * all ranks, rows_all: own rows of every band; HOST pointers).  Per solve: init, halo exchange, seedcand, halo
- * exchange, prepare (returns queued tiles), all ranks synchronise, arm, all ranks synchronise, solve (skip when no
- * rank has queued tiles), halo exchange, verify. */
+/* The same solve fused over NVLink peer memory, on the INTEGER RASTER of the single-GPU path (fill.py:174-232 /
+ * _fill.pyx:72-124 as above): every band's solver kernel runs at the same time and the bands feed each other's tile
+ * queues and halo rows directly (system-scope atomics and stores into blocks mapped through CUDA IPC), instead of one
+ * host-driven halo exchange per crossing of a band edge.  create: allocates the band's shared block, info80 (HOST,
+ * 80 bytes) describes it; open: maps every rank's block (infos: world x 80 bytes gathered from all ranks, rows_all:
+ * own rows of every band; HOST pointers).  Per solve: edgefix: fixed flags (seed or raster border) of the band's
+ * first / last own row (cols bytes each) - the caller hands them to the neighbours, whose halo rows they describe.
+ * prepare: the band's padded int32 distance raster, its edge rows stored into the neighbours' mailboxes (peer
+ * memory), FIFO := tiles holding lake cells; *queued, *irbad (the band does not fit the integer form).  All ranks
+ * synchronise, arm (a band with queued tiles counts itself active), synchronise, solve (all ranks at once; skipped
+ * when no rank has queued tiles): solve_launch returns once the solver kernel is queued, and the host is free for
+ * CPU work until solve_wait (no library call on this band in between).  finish: the float64 surface written once and
+ * verified against the fixed-point equation with the halo rows (*nviol), the D8 codes of the band's rows
+ * (flow.py:142-167, edges of the raster flowing outward) on the way.  When any rank reports irbad, a solver error or
+ * a violation, the host-driven init / solve / verify calls above take over on every rank. */
 int ms_band_nf_shared_create(ms_band *band, void *info80);
 int ms_band_nf_shared_open(ms_band *band, int rank, int world, const void *infos, const int64_t *rows_all);
-int ms_band_nf_seedcand_dev(ms_band *band, const float *filled, double *fnf, double short_eps, double diag_eps,
-                            double cap_bound, void *stream);
-int ms_band_nf_p2p_prepare_dev(ms_band *band, const double *fnf, int64_t *queued, void *stream);
-int ms_band_nf_p2p_arm_dev(ms_band *band, void *stream);
-int ms_band_nf_p2p_solve_dev(ms_band *band, const float *filled, double *fnf, double short_eps, double diag_eps,
-                             double cap_bound, int64_t *tile_visits, void *stream);
-
-/* The same fused solve on the INTEGER RASTER of the single-GPU path (fill.py:174-232 / _fill.pyx:72-124 as above; the
- * W-based form above stays as the fall-back for rasters that do not fit the integer form).  edgefix: fixed flags
- * (seed or raster border) of the band's first / last own row (cols bytes each) - the caller hands them to the
- * neighbours, whose halo rows they describe.  prepare: the band's padded int32 distance raster, its edge rows stored
- * into the neighbours' mailboxes (peer memory), FIFO := tiles holding lake cells; *queued, *irbad (the band does not
- * fit the integer form).  All ranks synchronise, ms_band_nf_p2p_arm_dev, synchronise, solve (all ranks at once):
- * solve_launch returns once the solver kernel is queued, and the host is free for CPU work until solve_wait (no
- * library call on this band in between).  finish: the float64 surface written once and verified against the
- * fixed-point equation with the halo rows (*nviol), the D8 codes of the band's rows (flow.py:142-167, edges of the
- * raster flowing outward) on the way. */
 int ms_band_nf_ir_edgefix_dev(ms_band *band, const float *dem, const float *filled, uint8_t *fix_top, uint8_t *fix_bot,
                               void *stream);
 int ms_band_nf_ir_prepare_dev(ms_band *band, const float *dem, const float *filled, double short_eps, double diag_eps,
                               double cap_bound, const uint8_t *fix_top, const uint8_t *fix_bot, int64_t *queued,
                               int *irbad, void *stream);
+int ms_band_nf_p2p_arm_dev(ms_band *band, void *stream);
 int ms_band_nf_ir_solve_launch_dev(ms_band *band, const float *filled, double short_eps, double diag_eps, void *stream);
 int ms_band_nf_ir_solve_wait_dev(ms_band *band, int64_t *tile_visits, int *irbad, void *stream);
 int ms_band_nf_ir_finish_dev(ms_band *band, const float *dem, const float *filled, double *fnf, uint8_t *flowdir,

@@ -78,10 +78,7 @@ SIGNATURES = {
     "ms_band_nf_ban_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_int, c_p, c_p]),
     "ms_band_nf_shared_create": (c_int, [c_p, c_p]),
     "ms_band_nf_shared_open": (c_int, [c_p, c_int, c_int, c_p, c_p]),
-    "ms_band_nf_seedcand_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_dbl, c_p]),
-    "ms_band_nf_p2p_prepare_dev": (c_int, [c_p, c_p, c_p, c_p]),
     "ms_band_nf_p2p_arm_dev": (c_int, [c_p, c_p]),
-    "ms_band_nf_p2p_solve_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_dbl, c_p, c_p]),
     "ms_band_nf_ir_edgefix_dev": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_band_nf_ir_prepare_dev": (c_int, [c_p, c_p, c_p, c_dbl, c_dbl, c_dbl, c_p, c_p, c_p, c_p, c_p]),
     "ms_band_nf_ir_solve_launch_dev": (c_int, [c_p, c_p, c_dbl, c_dbl, c_p]),

@@ -412,8 +412,6 @@ class BandPipeline(object):
         self._flowdir_done = False
         if self.p2p and self._noflats_ir(st):
             return
-        if self.p2p and self._noflats_p2p(st):
-            return
         self._call("ms_band_nf_ban_dev", self.h, None, None, 0.0, 0.0, 1, None, st)      # no bans from an earlier run
 
         def attempt(cap):
@@ -474,7 +472,7 @@ class BandPipeline(object):
         at once and exchanging edge rows and tile activations over NVLink peer memory; the finishing pass writes the
         surface once, verifies it with the halo rows and writes the D8 codes on the way.  Every decision is taken on
         values all ranks share (gathered / reduced), so the ranks stay in step; returns False when the raster does
-        not fit the integer form or the verification rejects the result (the W-based paths take over)."""
+        not fit the integer form or the verification rejects the result (the host-driven loop takes over)."""
         comm, dev, cols = self.comm, self.device, self.cols
         i64, cint = ctypes.c_int64, ctypes.c_int
         cap_bound = float(_lib.lib().ms_nf_cap_bound(self.R, self.cols, self.diag))
@@ -492,6 +490,7 @@ class BandPipeline(object):
         # one gather: also the barrier after which every band's edge rows are in its neighbours' mailboxes
         allq = comm.all_gather(torch.tensor([q.value, bad.value + err], dtype=torch.int64, device=dev)).cpu()
         if int(allq[:, 1].sum()) > 0:
+            self.stats["noflat_ir"] = 0
             return False
         visits = i64(0)
         if int(allq[:, 0].sum()) > 0:
@@ -518,43 +517,6 @@ class BandPipeline(object):
         if ok:
             self._flowdir_done = True
         return ok
-
-    def _noflats_p2p(self, st):
-        """The capped solve with all bands' solver kernels running at once and exchanging over NVLink peer memory.
-        Returns False if the verification stencil rejects the result (the host-driven generic path takes over)."""
-        comm, dev = self.comm, self.device
-        fnf = self.ext["fnf"]
-        i64 = ctypes.c_int64
-        cap_bound = float(_lib.lib().ms_nf_cap_bound(self.R, self.cols, self.diag))
-        ns = i64(0)
-        self._call("ms_band_nf_init_dev", self.h, _p(self.dem), _p(self.out["filled"]), _p(self.out["fnf"]),
-                   ctypes.byref(ns), st)
-        self._halo(fnf)
-        self._call("ms_band_nf_seedcand_dev", self.h, _p(self.out["filled"]), _p(self.out["fnf"]), self.short, self.diag,
-                   cap_bound, st)
-        self._halo(fnf)
-        self._tick("nf_init")
-        q = i64(0)
-        self._call("ms_band_nf_p2p_prepare_dev", self.h, _p(self.out["fnf"]), ctypes.byref(q), st)
-        torch.cuda.synchronize(dev)
-        allq = comm.all_gather(torch.tensor([q.value], dtype=torch.int64, device=dev)).cpu()      # also a barrier
-        visits = i64(0)
-        if int(allq.sum()) > 0:
-            self._call("ms_band_nf_p2p_arm_dev", self.h, st)
-            comm.all_reduce(torch.zeros(1, dtype=torch.int32, device=dev), "sum").cpu()           # barrier
-            self._call("ms_band_nf_p2p_solve_dev", self.h, _p(self.out["filled"]), _p(self.out["fnf"]), self.short,
-                       self.diag, cap_bound, ctypes.byref(visits), st)
-        self._tick("nf_p2p_solve")
-        self._halo(fnf)
-        nv = i64(0)
-        self._call("ms_band_nf_verify_dev", self.h, _p(self.dem), _p(self.out["fnf"]), self.short, self.diag,
-                   ctypes.byref(nv), st)
-        bad = comm.all_reduce(torch.tensor([nv.value], dtype=torch.int64, device=dev), "sum")
-        self._tick("nf_verify")
-        nbad = int(bad.item())
-        self.stats.update(noflat_exchanges=0, noflat_tile_visits=visits.value, noflat_capped=1, noflat_p2p=1,
-                          noflat_p2p_violations=nbad, noflat_p2p_queued=allq.view(-1).tolist())
-        return nbad == 0
 
     def _accum(self, st):
         comm, dev, cols = self.comm, self.device, self.cols

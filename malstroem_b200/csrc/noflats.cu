@@ -397,23 +397,24 @@ constexpr int NF_RUNNING = 256;
 constexpr int NF_RING_SLACK = 2048;
 
 // ---- row bands fused over NVLink peer memory (P2P) ---------------------------------------------------------
-// Every band's solver runs at the same time, one cooperative launch per GPU.  A band's FIFO, tile flags and two
-// "mailbox" rows (the neighbours' edge rows, i.e. this band's halo rows of the surface) live in one block that the
-// neighbouring ranks map through CUDA IPC.  A tile on a band edge whose ring changed stores its edge row into the
-// neighbour's mailbox and queues the neighbour's tile with system-scope atomics — the wave of a lake that spans
-// bands runs on without a host round trip.  Termination: each band counts its queued + running tiles; the number
-// of bands with a non-zero count lives on rank 0; whoever brings that to zero raises `done` on every rank.
+// Every band's solver (k_nf_solve_ir, below) runs at the same time, one cooperative launch per GPU.  A band's FIFO,
+// tile flags and two "mailbox" rows (the neighbours' edge rows, i.e. this band's halo rows of the integer raster)
+// live in one block that the neighbouring ranks map through CUDA IPC.  A tile on a band edge whose ring changed
+// stores its edge row into the neighbour's mailbox and queues the neighbour's tile with system-scope atomics — the
+// wave of a lake that spans bands runs on without a host round trip.  Termination: each band counts its queued +
+// running tiles; the number of bands with a non-zero count lives on rank 0; whoever brings that to zero raises
+// `done` on every rank.
 constexpr int NF_MAXRANKS = 16;
 struct NfPeer {
     int *tileflag;     // the neighbour band's tile flag words
     int *ring;         // ... its FIFO
     NfCtl *ctl;
-    void *mail;        // ... its mailbox row facing this band (float64 surface row, or padded int32 distance row)
+    void *mail;        // ... its mailbox row facing this band (padded int32 distance row)
     int tiles_y, cap;
 };
 struct NfP2P {
     NfPeer up, down;                // null pointers where the band is not open
-    void *mail_top, *mail_bot;      // this band's own halo rows of the surface (written by the neighbours)
+    void *mail_top, *mail_bot;      // this band's own halo rows of the integer raster (written by the neighbours)
     int *gactive;                   // rank 0: bands with queued or running tiles
     int *done_all[NF_MAXRANKS];     // every rank's ctl->done
     int world;
@@ -482,7 +483,7 @@ template <bool CAP>
 __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ zsrc, double *W, int *ring, int cap,
                                                   int *tileflag, const int *__restrict__ tilesides, NfCtl *ctl, int rows, int cols, int tiles_x,
                                                   int tiles_y, double sh, double dg, int use_int, double capB,
-                                                  int open, const NfP2P *pp) {
+                                                  int open) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double *sw = reinterpret_cast<double *>(smem_raw);
     float *sz = reinterpret_cast<float *>(smem_raw + (NF_T + 2) * NF_LD * 8);
@@ -493,20 +494,19 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // rows the aprons may read: a band that continues above / below has a halo row there
     const int rlo = (open & 1) ? -1 : 0, rhi = rows + ((open & 2) ? 1 : 0);
-    const bool p2p = pp != nullptr;
-    // halo rows of the surface: the ext rows of W, or (P2P) the mailboxes the neighbours write
-    const double *halo_top = p2p ? (const double *)pp->mail_top : W - (long long)cols;
-    const double *halo_bot = p2p ? (const double *)pp->mail_bot : W + (long long)rows * cols;
-    if (!p2p && *(volatile unsigned *)&ctl->tail == 0) return;      // nothing was queued (tail only grows)
+    // halo rows of the surface: the ext rows of W
+    const double *halo_top = W - (long long)cols;
+    const double *halo_bot = W + (long long)rows * cols;
+    if (*(volatile unsigned *)&ctl->tail == 0) return;      // nothing was queued (tail only grows)
 
     for (;;) {
         // The next tile is taken by thread 32 while thread 0 is still signing off the previous one (below): both are
         // chains of global atomics, and nobody touches S between the barrier that ends a visit and this point.
         if (tid == 32) {
-            const int t = nf_take(ring, cap, ctl, p2p, pp);
+            const int t = nf_take(ring, cap, ctl, false, nullptr);
             if (t >= 0) {
                 // taken: while the tile runs, neighbours only leave their side bits; they are looked at when it ends
-                S.flags = (p2p ? atomicExch_system(tileflag + t, NF_RUNNING) : atomicExch(tileflag + t, NF_RUNNING)) & NF_SIDES;
+                S.flags = atomicExch(tileflag + t, NF_RUNNING) & NF_SIDES;
                 S.dirty[1] = 0;
                 S.dirty[2] = 0;
                 S.chgmask = 0;
@@ -540,25 +540,15 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
                     if (tid >= 9 || (!dy && !dx)) return;
                     if (!(nbm & (1 << ((dy + 1) * 3 + (dx + 1))))) return;
                     int y = ty + dy, x = tx + dx;
-                    if (x < 0 || x >= tiles_x) return;
+                    // a tile of the neighbouring band: the host exchanges the halo rows and queues it there
+                    if (x < 0 || x >= tiles_x || y < 0 || y >= tiles_y) return;
                     // which side of the neighbour looks at us
                     int bits = (dy < 0 ? 2 : 0) | (dy > 0 ? 1 : 0) | (dx < 0 ? 8 : 0) | (dx > 0 ? 4 : 0);
                     if (dy && dx) bits = dy < 0 ? 2 : 1;      // a corner: one block of that side is enough
-                    if (y < 0 || y >= tiles_y) {
-                        // the tile lies in the neighbouring band: its flag word and FIFO are on another GPU
-                        if (!p2p) return;
-                        const NfPeer &q = y < 0 ? pp->up : pp->down;
-                        if (!q.tileflag) return;
-                        int nbq = (y < 0 ? q.tiles_y - 1 : 0) * tiles_x + x;
-                        if (atomicOr_system(q.tileflag + nbq, bits) == 0) nf_push(q.ring, q.cap, q.ctl, nbq, true, pp->gactive);
-                        return;
-                    }
                     int nb = y * tiles_x + x;
                     if (!(__ldg(tilesides + nb) & bits)) return;      // nothing there that could change
                     // an idle tile (no side bits yet, not running) is queued by whoever sets its first side bit
-                    if (p2p) {
-                        if (atomicOr_system(tileflag + nb, bits) == 0) nf_push(ring, cap, ctl, nb, true, pp->gactive);
-                    } else if (atomicOr(tileflag + nb, bits) == 0) nf_push(ring, cap, ctl, nb);
+                    if (atomicOr(tileflag + nb, bits) == 0) nf_push(ring, cap, ctl, nb);
                 }
         };
         bool solved = false;
@@ -714,17 +704,6 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
                         nbm = __reduce_or_sync(0xffffffffu, nbm);
                         if (lane == 0 && nbm) atomicOr(&S.nb, nbm);
                     }
-                    if (p2p) {
-                        // the band's edge rows go into the neighbours' mailboxes before their tiles are queued
-                        __threadfence();
-                        __syncthreads();
-                        if (ty == 0 && pp->up.mail && (S.ring & 1) && tid < NF_T && c0 + tid < cols)
-                            ((double *)pp->up.mail)[c0 + tid] = __ldcg(W + c0 + tid);
-                        if (ty == tiles_y - 1 && pp->down.mail && (S.ring & 2) && tid >= NF_T && tid < 2 * NF_T &&
-                            c0 + tid - NF_T < cols)
-                            ((double *)pp->down.mail)[c0 + tid - NF_T] = __ldcg(W + (long long)(rows - 1) * cols + c0 + tid - NF_T);
-                        __threadfence_system();
-                    }
                     __threadfence();
                     __syncthreads();
                     push_neighbours();
@@ -798,17 +777,6 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
                         if (c + 1 < cols) W[(size_t)r * cols + c + 1] = p[1];
                     }
                 }
-                if (p2p) {
-                    // the band's edge rows go into the neighbours' mailboxes before their tiles are queued
-                    __threadfence();
-                    __syncthreads();
-                    if (ty == 0 && pp->up.mail && (S.ring & 1) && tid < NF_T && c0 + tid < cols)
-                        ((double *)pp->up.mail)[c0 + tid] = __ldcg(W + c0 + tid);
-                    if (ty == tiles_y - 1 && pp->down.mail && (S.ring & 2) && tid >= NF_T && tid < 2 * NF_T &&
-                        c0 + tid - NF_T < cols)
-                        ((double *)pp->down.mail)[c0 + tid - NF_T] = __ldcg(W + (long long)(rows - 1) * cols + c0 + tid - NF_T);
-                    __threadfence_system();
-                }
                 __threadfence();
                 __syncthreads();
                 if (tid == 0) {
@@ -857,17 +825,9 @@ __global__ void __launch_bounds__(256, 4) k_nf_solve(const float *__restrict__ z
         __syncthreads();
         if (tid == 0) {
             // this tile: side bits that arrived while it ran mean it has to run again
-            if (p2p) {
-                if (atomicAnd_system(tileflag + t, ~NF_RUNNING) & NF_SIDES) nf_push(ring, cap, ctl, t, true, pp->gactive);
-                __threadfence_system();
-                // the band runs dry: one band less is active; the last one ends every rank's kernel
-                if (atomicSub_system(&ctl->pending, 1) == 1 && atomicSub_system(pp->gactive, 1) == 1)
-                    for (int k = 0; k < pp->world; k++) *(volatile int *)pp->done_all[k] = 1;
-            } else {
-                if (atomicAnd(tileflag + t, ~NF_RUNNING) & NF_SIDES) nf_push(ring, cap, ctl, t);
-                __threadfence();
-                if (atomicSub(&ctl->pending, 1) == 1) atomicExch(&ctl->done, 1);
-            }
+            if (atomicAnd(tileflag + t, ~NF_RUNNING) & NF_SIDES) nf_push(ring, cap, ctl, t);
+            __threadfence();
+            if (atomicSub(&ctl->pending, 1) == 1) atomicExch(&ctl->done, 1);
         }
     }
 }
@@ -1671,7 +1631,7 @@ template <bool CAP>
 static int nf_launch_solve(const float *zsrc, double *W, int *ring, int cap, int *tileflag, const int *tilesides,
                            NfCtl *ctl, int rows,
                            int cols, int tiles_x, int tiles_y, int ntiles, double sh, double dg, int use_int,
-                           double capB, int open, int64_t units, cudaStream_t s, const NfP2P *pp = nullptr) {
+                           double capB, int open, int64_t units, cudaStream_t s) {
     static int grid_blocks = 0;
     if (!grid_blocks) {
         MS_CUDA(cudaFuncSetAttribute(k_nf_solve<CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, NF_SMEM));
@@ -1685,9 +1645,9 @@ static int nf_launch_solve(const float *zsrc, double *W, int *ring, int cap, int
     void *args[] = {(void *)&zsrc, (void *)&W, (void *)&ring, (void *)&cap, (void *)&tileflag, (void *)&tilesides,
                     (void *)&ctl,
                     (void *)&rows, (void *)&cols, (void *)&tiles_x, (void *)&tiles_y, (void *)&sh, (void *)&dg,
-                    (void *)&use_int, (void *)&capB, (void *)&open, (void *)&pp};
+                    (void *)&use_int, (void *)&capB, (void *)&open};
     // consumers wait on the FIFO, so every CTA must be resident: cooperative launch guarantees it (or fails)
-    int g = (grid_blocks < ntiles || pp) ? grid_blocks : ntiles;
+    int g = grid_blocks < ntiles ? grid_blocks : ntiles;
     prof_units(units);
     if (g_prof) prof_begin(CAP ? "k_nf_solve<true>" : "k_nf_solve<false>", s);
     cudaError_t e = cudaLaunchCooperativeKernel((const void *)k_nf_solve<CAP>, dim3(g), dim3(256), args, NF_SMEM, s);
@@ -2018,9 +1978,8 @@ static NfSharedLayout nf_layout(int64_t rows, int64_t cols) {
     L.off_flag = take((size_t)L.ntiles * sizeof(int));
     L.off_sides = take((size_t)L.ntiles * sizeof(int));
     L.off_ring = take((size_t)L.cap * sizeof(int));
-    // a mailbox row holds cols float64 (W-based solver) or the padded int32 row of the integer raster
-    size_t mail = (size_t)cols * sizeof(double), mail_ir = ((size_t)L.tiles_x * NF_T + 8) * sizeof(int);
-    if (mail_ir > mail) mail = mail_ir;
+    // a mailbox row holds the padded int32 row of the integer raster
+    size_t mail = ((size_t)L.tiles_x * NF_T + 8) * sizeof(int);
     L.off_mtop = take(mail);
     L.off_mbot = take(mail);
     L.total = o;
@@ -2120,46 +2079,6 @@ int ms_band_nf_shared_open(ms_band *B, int rank, int world, const void *infos, c
     return MS_OK;
 }
 
-/* CAP only: the candidates the fixed neighbours offer (needs the halo rows of fnf after ms_band_nf_init_dev) */
-int ms_band_nf_seedcand_dev(ms_band *B, const float *filled, double *fnf, double short_eps, double diag_eps,
-                            double cap_bound, void *stream) {
-    using namespace ms;
-    MS_TRY(ensure_init());
-    if (!B || !filled || !fnf) { set_error("band no-flats: null pointer"); return MS_ERR_ARG; }
-    cudaStream_t s = (cudaStream_t)stream;
-    NfBandBufs nb;
-    MS_TRY(nf_band_bufs(B, &nb));
-    dim3 g2(cdiv(B->cols, 64), cdiv(B->rows, 4));
-    MS_LAUNCH(k_nf_seedcand, g2, 256, 0, s, filled, fnf, nb.ctl, (int)B->rows, (int)B->cols, short_eps, diag_eps, cap_bound,
-              B->open);
-    return MS_OK;
-}
-
-/* P2P step 1 (after init, seed candidates and a halo exchange of fnf): mailboxes := halo rows, FIFO := flagged tiles,
- * rank 0 clears the active-band counter.  Returns the number of queued tiles.  The caller synchronises all ranks. */
-int ms_band_nf_p2p_prepare_dev(ms_band *B, const double *fnf, int64_t *queued, void *stream) {
-    using namespace ms;
-    MS_TRY(ensure_init());
-    if (!B || !B->nf_pp_dev || !fnf || !queued) { set_error("band no-flats P2P: not set up"); return MS_ERR_ARG; }
-    cudaStream_t s = (cudaStream_t)stream;
-    NfBandBufs nb;
-    MS_TRY(nf_band_bufs(B, &nb));
-    NfSharedLayout L = nf_layout(B->rows, B->cols);
-    char *base = (char *)B->nf_shared;
-    size_t rowb = (size_t)B->cols * sizeof(double);
-    if (B->open & 1) MS_CUDA(cudaMemcpyAsync(base + L.off_mtop, fnf - B->cols, rowb, cudaMemcpyDeviceToDevice, s));
-    if (B->open & 2) MS_CUDA(cudaMemcpyAsync(base + L.off_mbot, fnf + B->rows * B->cols, rowb, cudaMemcpyDeviceToDevice, s));
-    MS_CUDA(cudaMemsetAsync(nb.ring, 0xff, (size_t)nb.cap_ring * sizeof(int), s));
-    MS_CUDA(cudaMemsetAsync(nb.ctl, 0, sizeof(NfCtl), s));
-    if (B->nf_rank == 0) MS_CUDA(cudaMemsetAsync(base + L.off_gactive, 0, sizeof(int), s));
-    MS_LAUNCH(k_nf_compact, cdiv(nb.ntiles, 256), 256, 0, s, nb.tileflag, nb.ring, nb.ctl, nb.ntiles);
-    NfCtl *h = (NfCtl *)(host_flags().h + 32);
-    MS_TRY(ms::readback(h, nb.ctl, sizeof(NfCtl), s));
-    MS_TRY(ms::stream_sync(s));
-    *queued = h->pending;
-    return MS_OK;
-}
-
 /* P2P step 2 (all ranks prepared): a band with queued tiles counts itself active.  The caller synchronises again. */
 int ms_band_nf_p2p_arm_dev(ms_band *B, void *stream) {
     using namespace ms;
@@ -2170,29 +2089,6 @@ int ms_band_nf_p2p_arm_dev(ms_band *B, void *stream) {
     MS_CUDA(cudaMemcpy(&pp, B->nf_pp_dev, sizeof(pp), cudaMemcpyDeviceToHost));
     MS_LAUNCH(k_nf_arm, 1, 1, 0, s, (NfCtl *)B->nf_shared, pp.gactive);
     MS_TRY(ms::stream_sync(s));
-    return MS_OK;
-}
-
-/* P2P step 3: the solve, all ranks at once (capped fast path).  Ends when no band has work left. */
-int ms_band_nf_p2p_solve_dev(ms_band *B, const float *filled, double *fnf, double short_eps, double diag_eps,
-                             double cap_bound, int64_t *tile_visits, void *stream) {
-    using namespace ms;
-    MS_TRY(ensure_init());
-    if (!B || !B->nf_pp_dev || !filled || !fnf) { set_error("band no-flats P2P: not set up"); return MS_ERR_ARG; }
-    cudaStream_t s = (cudaStream_t)stream;
-    NfBandBufs nb;
-    MS_TRY(nf_band_bufs(B, &nb));
-    MS_TRY(nf_launch_solve<true>(filled, fnf, nb.ring, nb.cap_ring, nb.tileflag, nb.tilesides, nb.ctl, (int)B->rows,
-                                 (int)B->cols, nb.tiles_x, nb.tiles_y, nb.ntiles, short_eps, diag_eps, g_nf_use_int,
-                                 cap_bound, B->open, B->rows * B->cols, s, (const NfP2P *)B->nf_pp_dev));
-    NfCtl *h = (NfCtl *)(host_flags().h + 32);
-    MS_TRY(ms::readback(h, nb.ctl, sizeof(NfCtl), s));
-    MS_TRY(ms::stream_sync(s));
-    if (h->done != 1) {
-        set_error("band no-flats P2P: solver stopped early (done=%d, pending=%d)", h->done, h->pending);
-        return MS_ERR_NOCONV;
-    }
-    if (tile_visits) *tile_visits = h->visits;
     return MS_OK;
 }
 

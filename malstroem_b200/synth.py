@@ -231,3 +231,18 @@ def pit_chain_dem(rows, cols, period=64):
     dem[1, c] = 60.0
     dem[0, c] = 5.0
     return dem
+
+
+def sea_bowl_dem(rows, cols):
+    """A bowl below sea level inside a rim of 30, drained by one channel at exactly 0 through the rim to the left
+    edge of the raster: the whole interior is one lake whose fill level is 0.0, spanning every row band.  Zero has no
+    binade, so the integer form of the no-flats solver refuses the raster and the float64 solver runs, on one GPU
+    and across bands (a coastal DEM with the sea at 0 does the same)."""
+    y, x = np.mgrid[0:rows, 0:cols].astype(np.float64)
+    bowl = ((y - rows / 2) / rows) ** 2 + ((x - cols / 2) / cols) ** 2
+    dem = (-20.0 + 39.0 * bowl).astype(np.float32)          # at most -0.5: no interior cell rounds to 0
+    dem = (np.round(dem * 1000) / 1000).astype(np.float32)
+    dem[:, :3] = dem[:, -3:] = 30.0
+    dem[:3, :] = dem[-3:, :] = 30.0
+    dem[rows // 3, :40] = 0.0                               # the outlet channel through the rim
+    return dem

@@ -18,6 +18,7 @@ KINDS = {
     "comb": lambda R, C: synth.mask_dem(synth.comb_mask(R, C)),
     "speckle": lambda R, C: synth.mask_dem(synth.speckle_mask(R, C)),
     "pit_chain": lambda R, C: synth.pit_chain_dem(R, C),
+    "sea_bowl": lambda R, C: synth.sea_bowl_dem(R, C),
 }
 
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
