@@ -244,6 +244,13 @@ int ms_band_cc_local_dev(ms_band *band, const void *data, int dtype, int64_t cel
                          int64_t *root_bot, void *stream);
 int ms_cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
                          int64_t *out_root, int64_t *out_global, int64_t capacity, int64_t *n_out);
+/* The same merge for regions of equal value (label polygonisation on bands): val_top / val_bot hold the cells' values
+ * (G * cols each, like the roots); two cells across a band edge join only if their values are equal, and diagonal
+ * neighbours only if connect8 != 0.  ms_cc_boundary_merge is this merge with every non-negative root joining its three
+ * neighbours. */
+int ms_cc_boundary_merge_values(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
+                                const int32_t *val_top, const int32_t *val_bot, int connect8, int64_t *out_root,
+                                int64_t *out_global, int64_t capacity, int64_t *n_out);
 int ms_band_cc_count_dev(ms_band *band, const int32_t *rerooted, int64_t n_rerooted, int64_t *count, void *stream);
 int ms_band_cc_root_labels_dev(ms_band *band, const int32_t *roots, int64_t n_roots, int64_t label_offset,
                                int32_t *labels_out, void *stream);
@@ -458,6 +465,47 @@ int ms_polygonize(const int32_t *labels, int64_t rows, int64_t cols, int connect
                   int64_t *counts3);
 int ms_polygonize_fetch(int64_t *ring_vertex_offset, int32_t *ring_value, int64_t *ring_cell, int64_t *ring_region,
                         uint8_t *ring_hole, int32_t *vertex_row, int32_t *vertex_col);
+
+/* Label polygonisation on a row band (malstroem_b200/vector.py polygonize_band; DESIGN.md 8(f4)).  `lab` points at
+ * the band's first row of `rows` x `cols` cells; halo bit 0 / 1: the row above (lab - cols) / below (lab + rows * cols)
+ * holds the neighbouring band's edge row.  Every buffer is the caller's, on the device unless named host; edge numbers
+ * are the band's own (0 .. n_edges - 1, in raster order: by cell, then top / right / bottom / left); the band's global
+ * edge numbers start at the sum of the lower bands' n_edges.  At most 2^30 cells and 2^31 - 1024 edges per band.
+ *  count: eoff[rows * cols] = first edge of every cell; *n_edges (host); row_eoff / row_mask [2 cols] = first edge and
+ *    side mask (bit 0 top .. 3 left) of the first and the last row's cells, for the neighbours' halo.
+ *  edges: halo_eoff (global) / halo_mask [2 cols] = the neighbours' row_eoff + their base / row_mask for the rows
+ *    above and below (ignored where the halo bit is clear).  Writes ecell[n_edges] = (cell << 2) | side, succ = local
+ *    successor (an exit, whose successor lies in another band: itself), lead = ring key << 32 (key: leader | 2^31 on a
+ *    ring closed in the band, else the slot of the exit ending the edge's chain), rank = steps to the leader / exit
+ *    << 32.  Exit slots [4 cols]: 2 c + {0, 1} for the top / left side of first-row cell c, 2 cols + 2 c + {0, 1} for
+ *    the right / bottom side of last-row cell c: exit_edge (-1: none), exit_next = global successor, exit_corner = 1
+ *    if that successor turns.
+ *  place: units = closed rings (head: the leader) and segments (head: the entry), numbered in head order; ishead,
+ *    uidx, ulen, ustart, placed, corner, vidx [n_edges] as for one GPU (corner at a segment's first edge: 0); per exit
+ *    slot seg_entry, seg_min (smallest edge), seg_tmin (its position from the entry).  counts2 (host) = units,
+ *    vertices.
+ *  emit: vrow / vcol [nverts] (global lattice rows, row0 = the band's first row), the unit table [units]: u_head,
+ *    u_len, u_vstart, u_vcount, u_value, u_root (global cell index of the region root within the band), u_slot (-1:
+ *    a closed ring); root_rows [2 cols]: region roots of the first and last row (-1: nodata), for
+ *    ms_cc_boundary_merge_values. */
+int ms_band_poly_count_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                           int32_t nodata, int32_t *eoff, int64_t *n_edges, int32_t *row_eoff, uint8_t *row_mask,
+                           void *stream);
+int ms_band_poly_edges_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                           int32_t nodata, const int32_t *eoff, int64_t n_edges, const int64_t *halo_eoff,
+                           const uint8_t *halo_mask, uint32_t *ecell, int32_t *succ, uint64_t *lead, uint64_t *rank,
+                           int32_t *exit_edge, int64_t *exit_next, uint8_t *exit_corner, void *stream);
+int ms_band_poly_place_dev(int64_t cols, int64_t n_edges, const uint32_t *ecell, const int32_t *succ,
+                           const uint64_t *lead, const uint64_t *rank, int32_t *ishead, int32_t *uidx, int32_t *ulen,
+                           int32_t *ustart, uint32_t *placed, int32_t *corner, int32_t *vidx, int32_t *seg_entry,
+                           int32_t *seg_min, int32_t *seg_tmin, int64_t *counts2, void *stream);
+int ms_band_poly_emit_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                          int32_t nodata, int64_t row0, int64_t n_edges, const uint32_t *ecell, const uint64_t *lead,
+                          const int32_t *ishead, const int32_t *uidx, const int32_t *ulen, const int32_t *ustart,
+                          const uint32_t *placed, const int32_t *corner, const int32_t *vidx, int64_t nverts,
+                          int32_t *vrow, int32_t *vcol, int32_t *u_head, int32_t *u_len, int32_t *u_vstart,
+                          int32_t *u_vcount, int32_t *u_value, int64_t *u_root, int32_t *u_slot, int64_t *root_rows,
+                          void *stream);
 
 /* ---- Bluespot water levels and water-depth rasters after rain events.
  * Bluespot l >= 1 is the set of cells with labels == l; z = dem widened to float64, F = the plain fill (uniform over

@@ -90,6 +90,7 @@ SIGNATURES = {
     "ms_band_accum_finish_dev": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_band_cc_local_dev": (c_int, [c_p, c_p, c_int, c_i64, c_p, c_p, c_p]),
     "ms_cc_boundary_merge": (c_int, [c_int, c_i64, c_p, c_p, c_p, c_p, c_i64, c_p]),
+    "ms_cc_boundary_merge_values": (c_int, [c_int, c_i64, c_p, c_p, c_p, c_p, c_int, c_p, c_p, c_i64, c_p]),
     "ms_band_cc_count_dev": (c_int, [c_p, c_p, c_i64, c_p, c_p]),
     "ms_band_cc_root_labels_dev": (c_int, [c_p, c_p, c_i64, c_i64, c_p, c_p]),
     "ms_band_cc_finish_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_p, c_p]),
@@ -121,6 +122,14 @@ SIGNATURES = {
     "ms_polygonize_dev": (c_int, [c_p, c_i64, c_i64, c_int, c_int, ctypes.c_int32, c_p, c_p]),
     "ms_polygonize": (c_int, [c_p, c_i64, c_i64, c_int, c_int, ctypes.c_int32, c_p]),
     "ms_polygonize_fetch": (c_int, [c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ms_band_poly_count_dev": (c_int, [c_p, c_i64, c_i64, c_int, c_int, c_int, ctypes.c_int32, c_p, c_p, c_p, c_p, c_p]),
+    "ms_band_poly_edges_dev": (c_int, [c_p, c_i64, c_i64, c_int, c_int, c_int, ctypes.c_int32, c_p, c_i64, c_p, c_p, c_p,
+                                       c_p, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ms_band_poly_place_dev": (c_int, [c_i64, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p,
+                                       c_p, c_p]),
+    "ms_band_poly_emit_dev": (c_int, [c_p, c_i64, c_i64, c_int, c_int, c_int, ctypes.c_int32, c_i64, c_i64, c_p, c_p, c_p,
+                                      c_p, c_p, c_p, c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p,
+                                      c_p, c_p]),
     "ms_bluespot_network_dev": (c_int, [c_p, c_dbl, c_int, c_i64, c_p, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ms_flood_levels_dev": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_dbl, c_i64, c_p, c_p, c_p, c_p]),
     "ms_flood_levels": (c_int, [c_p, c_p, c_p, c_i64, c_i64, c_i64, c_p, c_dbl, c_i64, c_p, c_p, c_p]),

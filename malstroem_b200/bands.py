@@ -203,6 +203,58 @@ def label_owner(labels, offsets):
     return torch.searchsorted(offsets, labels, right=False) - 1
 
 
+def ring_segments(entry, nxt, length, mn, tmin, cv, kmin, nextc):
+    """The rings that cross band edges, from their segments (DESIGN.md §8(f4)).  A segment is the run of a ring's
+    edges inside one band from an entry (predecessor in another band) to an exit (successor in another band); per
+    segment (int64 tensors [S], global edge numbers): entry, nxt = the entry of the segment that follows, length, mn =
+    its smallest edge, tmin = mn's offset from the entry, cv = corners at offsets 1 .. length - 1, kmin = corners at
+    offsets 1 .. tmin - 1, nextc = 1 if the following segment's entry starts at a corner.
+    Returns per ring (sorted by leader = smallest edge of the ring): leader, L (edges), V (vertices), first (the
+    segment holding the leader); per segment: ring, centry (its entry starts at a corner), eoff = ring position of its
+    entry, voff = ring vertex index of its first corner (the entry's if centry).  An edge at offset t is at ring
+    position (eoff + t) mod L; the u-th corner after the entry is vertex (voff + centry + u) mod V.  Pointer doubling
+    over the segments: ceil(log2(S + 1)) rounds cover every ring."""
+    S, dev = entry.numel(), entry.device
+    i64 = torch.int64
+    if S == 0:
+        e = torch.zeros(0, dtype=i64, device=dev)
+        return {"leader": e, "L": e, "V": e, "first": e, "ring": e, "centry": e, "eoff": e, "voff": e}
+    idx = torch.arange(S, dtype=i64, device=dev)
+    order = torch.argsort(entry)
+    at = torch.searchsorted(entry[order], nxt).clamp(max=S - 1)
+    if not bool((entry[order][at] == nxt).all()):
+        raise ValueError("ring_segments: a segment is followed by no segment's entry")
+    p = order[at]
+    pred = torch.empty_like(p)
+    pred[p] = idx
+    if not bool((p[pred] == idx).all()):
+        raise ValueError("ring_segments: two segments are followed by the same segment")
+    centry = nextc[pred]
+    cvt = centry + cv
+    rounds = int(S).bit_length()
+    lead, jump = mn.clone(), p.clone()
+    for _ in range(rounds):
+        lead, jump = torch.minimum(lead, lead[jump]), jump[jump]
+    first = mn == lead
+    leader, ring = torch.unique(lead, return_inverse=True)
+    nr = leader.numel()
+    L = torch.zeros(nr, dtype=i64, device=dev).index_add_(0, ring, length)
+    V = torch.zeros(nr, dtype=i64, device=dev).index_add_(0, ring, cvt)
+    fidx = torch.zeros(nr, dtype=i64, device=dev).scatter_(0, ring[first], idx[first])
+    # edges / corners from every segment's entry up to the leader segment's entry, going forward
+    w = torch.where(first, 0, length)
+    wv = torch.where(first, 0, cvt)
+    tgt = torch.where(first, idx, p)
+    for _ in range(rounds):
+        w, wv, tgt = w + w[tgt], wv + wv[tgt], tgt[tgt]
+    Ls, Vs = L[ring], V[ring].clamp(min=1)
+    eoff = (Ls - w - tmin[fidx][ring]) % Ls
+    before = torch.where(tmin > 0, centry, 0) + kmin          # corners of the leader's segment before the leader
+    voff = (Vs - wv - before[fidx][ring]) % Vs
+    return {"leader": leader, "L": L, "V": V, "first": fidx, "ring": ring, "centry": centry, "eoff": eoff,
+            "voff": voff}
+
+
 def cc_plan(roots, globals_, cell_lo, cell_hi):
     """From the merged boundary roots (numpy int64, ascending `roots`, their component's smallest root `globals_`):
     the band's re-rooted local roots, the component roots it owns, and the sorted list of all component roots."""

@@ -248,9 +248,10 @@ extern "C" {
  * of the G bands, the root of every cell of the band's first / last row (-1 = background), G * cols entries each.
  * Output: every distinct root seen on an interior band edge, ascending, with the root of its merged component.
  * Pure CPU code (a few thousand cells): runs identically on every rank. */
-int ms_cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
-                         int64_t *out_root, int64_t *out_global, int64_t capacity, int64_t *n_out) {
-    if (nbands < 1 || cols < 1 || !root_top || !root_bot || !n_out) { ms::set_error("cc_boundary_merge: bad argument"); return MS_ERR_ARG; }
+static int cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
+                             const int32_t *val_top, const int32_t *val_bot, int connect8, int64_t *out_root,
+                             int64_t *out_global, int64_t capacity, int64_t *n_out) {
+    if (nbands < 1 || cols < 1 || !root_top || !root_bot || !n_out || (!val_top != !val_bot)) { ms::set_error("cc_boundary_merge: bad argument"); return MS_ERR_ARG; }
     // distinct roots: cells of one component are consecutive along a row, so only the first cell of each run is kept
     // before sorting (a few thousand ids instead of 2 * cols per band edge)
     std::vector<int64_t> ids;
@@ -276,12 +277,13 @@ int ms_cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, cons
     auto index_of = [&](int64_t v) { return (int)(std::lower_bound(ids.begin(), ids.end(), v) - ids.begin()); };
     for (int g = 0; g + 1 < nbands; g++) {
         const int64_t *bot = root_bot + (int64_t)g * cols, *top = root_top + (int64_t)(g + 1) * cols;
+        const int32_t *vb = val_bot ? val_bot + (int64_t)g * cols : nullptr, *vt = val_top ? val_top + (int64_t)(g + 1) * cols : nullptr;
         int64_t last_a = -1, last_b = -1;
         for (int64_t c = 0; c < cols; c++) {
             int64_t a = bot[c];
             if (a < 0) continue;
             for (int64_t d = -1; d <= 1; d++) {
-                if (c + d < 0 || c + d >= cols) continue;
+                if (c + d < 0 || c + d >= cols || (d != 0 && !connect8) || (vb && vb[c] != vt[c + d])) continue;
                 int64_t b = top[c + d];
                 if (b < 0 || (a == last_a && b == last_b)) continue;      // the same pair again along a run
                 last_a = a;
@@ -299,6 +301,19 @@ int ms_cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, cons
         if (out_global) out_global[k] = ids[find((int)k)];
     }
     return MS_OK;
+}
+
+int ms_cc_boundary_merge(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
+                         int64_t *out_root, int64_t *out_global, int64_t capacity, int64_t *n_out) {
+    return cc_boundary_merge(nbands, cols, root_top, root_bot, nullptr, nullptr, 1, out_root, out_global, capacity, n_out);
+}
+
+int ms_cc_boundary_merge_values(int nbands, int64_t cols, const int64_t *root_top, const int64_t *root_bot,
+                                const int32_t *val_top, const int32_t *val_bot, int connect8, int64_t *out_root,
+                                int64_t *out_global, int64_t capacity, int64_t *n_out) {
+    if (!val_top || !val_bot) { ms::set_error("cc_boundary_merge_values: null value rows"); return MS_ERR_ARG; }
+    return cc_boundary_merge(nbands, cols, root_top, root_bot, val_top, val_bot, connect8, out_root, out_global,
+                             capacity, n_out);
 }
 
 int ms_version(void) { return 110; }

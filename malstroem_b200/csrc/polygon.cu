@@ -51,15 +51,19 @@ void poly_release() {
     g_poly = PolyHold();
 }
 
+// The kernels walk rows [0, rows) of `lab`; rows [r_lo, r_hi) may be read as neighbours.  One GPU: r_lo = 0,
+// r_hi = rows.  A row band: r_lo = -1 / r_hi = rows + 1 where the neighbouring band's edge row is present as a halo row
+// (lab - cols, lab + rows * cols), so that masks and successors on the band's first and last rows are the raster's.
 struct PolyGrid {
     const int32_t *lab;
     int rows, cols;
     int connect8, has_nodata;
     int32_t nodata;
+    int r_lo, r_hi;
 };
 
 __device__ inline bool poly_same(const PolyGrid &g, int r, int c, int32_t v) {
-    return r >= 0 && r < g.rows && c >= 0 && c < g.cols && g.lab[(size_t)r * g.cols + c] == v;
+    return r >= g.r_lo && r < g.r_hi && c >= 0 && c < g.cols && g.lab[(int64_t)r * g.cols + c] == v;
 }
 
 // sides of the cell that are boundary edges: bit 0 top, 1 right, 2 bottom, 3 left
@@ -80,8 +84,22 @@ __global__ void __launch_bounds__(256) k_poly_count(PolyGrid g, int *cnt) {
 __device__ __constant__ const int kFR[4] = {0, 1, 0, -1}, kFC[4] = {1, 0, -1, 0};
 __device__ __constant__ const int kRR[4] = {1, 0, -1, 0}, kRC[4] = {0, -1, 0, 1};
 
+// A row band's view of its neighbours (all null on one GPU, where no successor leaves the raster's rows).  A successor
+// on a halo row is an EXIT: it gets the slot (row above: 2 c + {top 0, left 1}, row below: 2 cols + 2 c + {right 0,
+// bottom 1}) as its ring key, points at itself and leaves its global successor in the slot; every other edge's key is
+// its number with bit 31 set, so that pointer doubling gives a chain's edges the slot of their exit and a closed ring's
+// edges (bit 31 set) their leader.
+struct PolyHalo {
+    const int64_t *eoff;          // [2][cols]: global first edge number of the halo cells (above, below)
+    const uint8_t *mask;          // [2][cols]: their side masks
+    int32_t *exit_edge;           // [4 cols]: local edge number in the slot (-1: none)
+    int64_t *exit_next;           // [4 cols]: global number of its successor
+    uint8_t *exit_corner;         // [4 cols]: 1 if that successor starts at a corner
+};
+constexpr unsigned kPolyChainBit = 0x80000000u;
+
 __global__ void __launch_bounds__(256) k_poly_edges(PolyGrid g, const int *__restrict__ eoff, uint32_t *ecell,
-                                                    int *succ, unsigned long long *state) {
+                                                    int *succ, unsigned long long *state, PolyHalo hb) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int64_t)g.rows * g.cols) return;
     int r = (int)(i / g.cols), c = (int)(i - (int64_t)r * g.cols);
@@ -102,12 +120,24 @@ __global__ void __launch_bounds__(256) k_poly_edges(PolyGrid g, const int *__res
         if (left) { nr = alr; nc = alc; ns = (s + 3) & 3; }
         else if (straight) { nr = arr; nc = arc; ns = s; }
         else { nr = r; nc = c; ns = (s + 1) & 3; }
+        ecell[e] = (uint32_t)((i << 2) | s);
+        if (nr < 0 || nr >= g.rows) {         // only on a band with a halo row
+            const int h = nr < 0 ? 0 : 1;
+            const int slot = 2 * h * g.cols + 2 * c + ((s == 0 || s == 1) ? 0 : 1);
+            hb.exit_edge[slot] = e;
+            hb.exit_next[slot] = hb.eoff[h * g.cols + nc] + __popc(hb.mask[h * g.cols + nc] & ((1 << ns) - 1));
+            hb.exit_corner[slot] = ns != s;
+            succ[e] = e;
+            state[e] = ((unsigned long long)(unsigned)slot << 32) | (unsigned)e;
+            e++;
+            continue;
+        }
         const int64_t j = (int64_t)nr * g.cols + nc;
         const int nmask = (nr == r && nc == c) ? mask : poly_mask(g, nr, nc, v);
         const int q = eoff[j] + __popc(nmask & ((1 << ns) - 1));
-        ecell[e] = (uint32_t)((i << 2) | s);
         succ[e] = q;
-        state[e] = ((unsigned long long)(unsigned)e << 32) | (unsigned)q;      // (leader so far, jump)
+        const unsigned key = hb.exit_edge ? ((unsigned)e | kPolyChainBit) : (unsigned)e;
+        state[e] = ((unsigned long long)key << 32) | (unsigned)q;      // (leader so far, jump)
         e++;
     }
 }
@@ -125,13 +155,16 @@ __global__ void __launch_bounds__(256) k_poly_minjump(const unsigned long long *
     if (l != lx) *changed = 1;
 }
 
-// hi word: steps from here to the jump target; lo word: the jump target (the leader points at itself, 0 steps)
+// hi word: steps from here to the jump target; lo word: the jump target (the leader points at itself, 0 steps; on a
+// band an exit too, which ends its chain; key_bit: kPolyChainBit on a band, else 0)
 __global__ void __launch_bounds__(256) k_poly_rankinit(const unsigned long long *__restrict__ lead_state,
-                                                       const int *__restrict__ succ, unsigned long long *c, int n) {
+                                                       const int *__restrict__ succ, unsigned long long *c, int n,
+                                                       unsigned key_bit) {
     int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     const unsigned lead = (unsigned)(lead_state[e] >> 32);
-    c[e] = lead == (unsigned)e ? (unsigned long long)(unsigned)e : ((1ull << 32) | (unsigned)succ[e]);
+    const int q = succ[e];
+    c[e] = (lead == ((unsigned)e | key_bit) || q == e) ? (unsigned long long)(unsigned)e : ((1ull << 32) | (unsigned)q);
 }
 
 __global__ void __launch_bounds__(256) k_poly_rankjump(const unsigned long long *__restrict__ a, unsigned long long *b,
@@ -174,8 +207,8 @@ __global__ void __launch_bounds__(256) k_poly_place(const unsigned long long *__
 }
 
 __global__ void __launch_bounds__(256) k_poly_emit(const uint32_t *__restrict__ placed, const int *__restrict__ corner,
-                                                   const int *__restrict__ vidx, int cols, int32_t *vrow, int32_t *vcol,
-                                                   int n) {
+                                                   const int *__restrict__ vidx, int cols, int row0, int32_t *vrow,
+                                                   int32_t *vcol, int n) {
     int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n || !corner[k]) return;
     const uint32_t ec = placed[k];
@@ -184,7 +217,7 @@ __global__ void __launch_bounds__(256) k_poly_emit(const uint32_t *__restrict__ 
     const int r = (int)(i / cols), c = (int)(i - (int64_t)r * cols);
     // start vertex of the side: top (r, c), right (r, c + 1), bottom (r + 1, c + 1), left (r + 1, c)
     const int v = vidx[k];
-    vrow[v] = r + (s >= 2 ? 1 : 0);
+    vrow[v] = row0 + r + (s >= 2 ? 1 : 0);
     vcol[v] = c + ((s == 1 || s == 2) ? 1 : 0);
 }
 
@@ -217,9 +250,12 @@ __global__ void __launch_bounds__(256) k_poly_parinit(int *par, int64_t n) {
     if (i < n) par[i] = (int)i;
 }
 
+// the cells of rows [0, rows) only: a band joins its regions to its neighbours' afterwards (ms_cc_boundary_merge_values)
 __global__ void __launch_bounds__(256) k_poly_union(PolyGrid g, int *par) {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int64_t)g.rows * g.cols) return;
+    g.r_lo = 0;
+    g.r_hi = g.rows;
     int r = (int)(i / g.cols), c = (int)(i - (int64_t)r * g.cols);
     const int32_t v = g.lab[i];
     if (g.has_nodata && v == g.nodata) return;
@@ -286,7 +322,7 @@ int polygonize_dev_impl(const int32_t *labels, int64_t rows, int64_t cols, int c
     }
     poly_release();
     const int64_t n = rows * cols;
-    PolyGrid g{labels, (int)rows, (int)cols, connect8 ? 1 : 0, has_nodata ? 1 : 0, nodata};
+    PolyGrid g{labels, (int)rows, (int)cols, connect8 ? 1 : 0, has_nodata ? 1 : 0, nodata, 0, (int)rows};
     int64_t *h = host_flags().h;
     DevBuf<int> eoff;
     DevBuf<int64_t> total;
@@ -317,12 +353,13 @@ int polygonize_dev_impl(const int32_t *labels, int64_t rows, int64_t cols, int c
     MS_TRY(succ.alloc((size_t)ne, s));
     MS_TRY(sa.alloc((size_t)ne, s));
     MS_TRY(sb.alloc((size_t)ne, s));
-    MS_LAUNCH(k_poly_edges, cdiv(n, 256), 256, 0, s, g, (const int *)eoff.p, ecell.p, succ.p, sa.p);
+    MS_LAUNCH(k_poly_edges, cdiv(n, 256), 256, 0, s, g, (const int *)eoff.p, ecell.p, succ.p, sa.p, PolyHalo{});
     unsigned long long *a = sa.p, *b = sb.p;
     MS_TRY(jump_rounds(false, &a, &b, ne, s));
     unsigned long long *lead_state = a;       // hi word = the ring's leader; the other buffer is free again
     MS_TRY(ra.alloc((size_t)ne, s));
-    MS_LAUNCH(k_poly_rankinit, cdiv(ne, 256), 256, 0, s, (const unsigned long long *)lead_state, (const int *)succ.p, ra.p, ne);
+    MS_LAUNCH(k_poly_rankinit, cdiv(ne, 256), 256, 0, s, (const unsigned long long *)lead_state, (const int *)succ.p, ra.p, ne,
+              0u);
     unsigned long long *c = ra.p, *d = b;
     MS_TRY(jump_rounds(true, &c, &d, ne, s));
     unsigned long long *rank = c;
@@ -360,7 +397,7 @@ int polygonize_dev_impl(const int32_t *labels, int64_t rows, int64_t cols, int c
     MS_TRY(hold_alloc(&g_poly.vrow, (size_t)nverts));
     MS_TRY(hold_alloc(&g_poly.vcol, (size_t)nverts));
     MS_LAUNCH(k_poly_emit, cdiv(ne, 256), 256, 0, s, (const uint32_t *)placed.p, (const int *)corner.p, (const int *)vidx.p,
-              (int)cols, g_poly.vrow, g_poly.vcol, ne);
+              (int)cols, 0, g_poly.vrow, g_poly.vcol, ne);
     MS_LAUNCH(k_poly_ring, cdiv(ne, 256), 256, 0, s, g, (const int *)isleader.p, (const int *)ridx.p, (const int *)rstart.p,
               (const int *)vidx.p, (const uint32_t *)ecell.p, par.p, g_poly.voff, g_poly.value, g_poly.cell, g_poly.region,
               g_poly.hole, ne, nrings, nverts);
@@ -370,6 +407,133 @@ int polygonize_dev_impl(const int32_t *labels, int64_t rows, int64_t cols, int c
     g_poly.nedges = E;
     counts3[0] = nrings;
     counts3[1] = nverts;
+    return MS_OK;
+}
+
+
+// ---- row bands (DESIGN.md §8(f4), malstroem_b200/vector.py polygonize_band) -------------------------------------------
+// Every buffer that lives from one phase to the next belongs to the caller: the bands of one process run these calls
+// from several threads.  Edge numbers are the band's own (0 .. n_edges - 1); the band's first edge has global number
+// base = the edge counts of the lower bands, so local order is global order.  After the doubling an edge's ring key
+// says what it is: bit 31 set -> a closed ring of the band (key - bit 31 = its leader), else the slot of the exit that
+// ends its chain.  A chain starts at an ENTRY (an edge whose predecessor lies in another band) and runs to its exit: a
+// SEGMENT.  Units = closed rings and segments, numbered by their head (the leader, the entry) in edge order; every
+// edge is placed at (unit start + position), the leader / the entry at position 0.
+
+static inline PolyGrid poly_band_grid(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8,
+                                          int has_nodata, int32_t nodata) {
+    return PolyGrid{lab, (int)rows, (int)cols, connect8 ? 1 : 0, has_nodata ? 1 : 0, nodata, (halo & 1) ? -1 : 0,
+                    (int)rows + ((halo & 2) ? 1 : 0)};
+}
+
+// local first edge number and side mask of the band's first and last row (for the neighbours' halo)
+__global__ void __launch_bounds__(256) k_poly_band_rows(PolyGrid g, const int *__restrict__ eoff, int32_t *row_eoff,
+                                                        uint8_t *row_mask) {
+    int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= 2 * g.cols) return;
+    const int r = k < g.cols ? 0 : g.rows - 1, c = k < g.cols ? k : k - g.cols;
+    const int64_t i = (int64_t)r * g.cols + c;
+    row_eoff[k] = eoff[i];
+    row_mask[k] = (uint8_t)poly_mask(g, r, c, g.lab[i]);
+}
+
+// predecessor flags; the smallest edge of every segment (by its exit's slot)
+__global__ void __launch_bounds__(256) k_poly_band_pred(const unsigned long long *__restrict__ lead_state,
+                                                        const int *__restrict__ succ, int *haspred, int *seg_min, int n) {
+    int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    const int q = succ[e];
+    if (q != e) haspred[q] = 1;
+    const unsigned key = (unsigned)(lead_state[e] >> 32);
+    if (!(key & kPolyChainBit)) atomicMin((unsigned *)seg_min + key, (unsigned)e);
+}
+
+// unit heads and lengths (scanned into unit number / unit start); a segment's entry registers in its exit's slot
+__global__ void __launch_bounds__(256) k_poly_band_heads(const unsigned long long *__restrict__ lead_state,
+                                                         const unsigned long long *__restrict__ rank,
+                                                         const int *__restrict__ succ, const int *__restrict__ haspred,
+                                                         int *ishead, int *ulen, int *seg_entry, int n) {
+    int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    const unsigned key = (unsigned)(lead_state[e] >> 32);
+    bool h;
+    int len = 0;
+    if (key & kPolyChainBit) {
+        h = key == ((unsigned)e | kPolyChainBit);
+        if (h) len = (int)(rank[succ[e]] >> 32) + 1;
+    } else {
+        h = !haspred[e];
+        if (h) { len = (int)(rank[e] >> 32) + 1; seg_entry[key] = e; }
+    }
+    ishead[e] = h;
+    ulen[e] = len;
+}
+
+// as k_poly_place, for closed rings (position from the leader) and segments (position from the entry: length - 1 -
+// steps to the exit); a segment's first slot stays 0 here (its corner flag depends on the band before it)
+__global__ void __launch_bounds__(256) k_poly_band_place(const unsigned long long *__restrict__ lead_state,
+                                                         const unsigned long long *__restrict__ rank,
+                                                         const int *__restrict__ succ, const uint32_t *__restrict__ ecell,
+                                                         const int *__restrict__ ustart, const int *__restrict__ ulen,
+                                                         const int *__restrict__ seg_entry,
+                                                         const int *__restrict__ seg_min, uint32_t *placed, int *corner,
+                                                         int *seg_tmin, int n) {
+    int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    const unsigned key = (unsigned)(lead_state[e] >> 32);
+    const int d = (int)(rank[e] >> 32);
+    const int q = succ[e];
+    const bool ring = key & kPolyChainBit;
+    const int head = ring ? (int)(key & ~kPolyChainBit) : seg_entry[key];
+    const int L = ulen[head], base = ustart[head];
+    const int pos = ring ? (d == 0 ? 0 : L - d) : L - 1 - d;
+    placed[base + pos] = ecell[e];
+    if (ring) corner[base + (pos + 1 == L ? 0 : pos + 1)] = (ecell[q] & 3u) != (ecell[e] & 3u);
+    else {
+        if (q != e) corner[base + pos + 1] = (ecell[q] & 3u) != (ecell[e] & 3u);
+        if ((unsigned)seg_min[key] == (unsigned)e) seg_tmin[key] = pos;
+    }
+}
+
+// the unit table: head edge, length, first vertex, vertex count, value, region root (global cell index of the band's
+// local root), exit slot (-1: a closed ring)
+__global__ void __launch_bounds__(256) k_poly_band_units(PolyGrid g, const unsigned long long *__restrict__ lead_state,
+                                                         const int *__restrict__ ishead, const int *__restrict__ uidx,
+                                                         const int *__restrict__ ustart, const int *__restrict__ ulen,
+                                                         const int *__restrict__ vidx, const uint32_t *__restrict__ ecell,
+                                                         int *par, int64_t cell0, int n, int nverts, int32_t *u_head,
+                                                         int32_t *u_len, int32_t *u_vstart, int32_t *u_vcount,
+                                                         int32_t *u_value, int64_t *u_root, int32_t *u_slot) {
+    int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n || !ishead[e]) return;
+    const int k = uidx[e];
+    const int a = ustart[e], L = ulen[e];
+    const int v0 = vidx[a];
+    const unsigned key = (unsigned)(lead_state[e] >> 32);
+    const int i = (int)(ecell[e] >> 2);
+    u_head[k] = e;
+    u_len[k] = L;
+    u_vstart[k] = v0;
+    u_vcount[k] = (a + L < n ? vidx[a + L] : nverts) - v0;
+    u_value[k] = g.lab[i];
+    u_root[k] = cell0 + poly_root(par, i);
+    u_slot[k] = (key & kPolyChainBit) ? -1 : (int)key;
+}
+
+// region roots (global cell index, -1 for nodata) of the band's first and last row
+__global__ void __launch_bounds__(256) k_poly_band_rowroots(PolyGrid g, int *par, int64_t cell0, int64_t *root_rows) {
+    int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= 2 * g.cols) return;
+    const int r = k < g.cols ? 0 : g.rows - 1, c = k < g.cols ? k : k - g.cols;
+    const int i = r * g.cols + c;
+    root_rows[k] = (g.has_nodata && g.lab[i] == g.nodata) ? -1 : cell0 + poly_root(par, i);
+}
+
+static int band_poly_args(const int32_t *lab, int64_t rows, int64_t cols, int halo) {
+    if (!lab || rows < 1 || cols < 1 || rows * cols > (1ll << 30) || (halo & ~3)) {
+        set_error("band polygonize: unsupported band %lld x %lld (halo %d)", (long long)rows, (long long)cols, halo);
+        return MS_ERR_ARG;
+    }
     return MS_OK;
 }
 
@@ -392,6 +556,131 @@ int ms_polygonize(const int32_t *labels, int64_t rows, int64_t cols, int connect
     int32_t *l = nullptr;
     MS_TRY(hc.in(labels, (size_t)(rows * cols), s, &l));
     return ms::polygonize_dev_impl(l, rows, cols, connect8, has_nodata, nodata, counts3, s);
+}
+
+int ms_band_poly_count_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                           int32_t nodata, int32_t *eoff, int64_t *n_edges, int32_t *row_eoff, uint8_t *row_mask,
+                           void *stream) {
+    MS_TRY(ms::ensure_init());
+    MS_TRY(ms::band_poly_args(lab, rows, cols, halo));
+    if (!eoff || !n_edges || !row_eoff || !row_mask) { ms::set_error("band_poly_count: null pointer"); return MS_ERR_ARG; }
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = rows * cols;
+    ms::PolyGrid g = ms::poly_band_grid(lab, rows, cols, halo, connect8, has_nodata, nodata);
+    ms::DevBuf<int64_t> total;
+    MS_TRY(total.alloc(1, s));
+    MS_LAUNCH(ms::k_poly_count, ms::cdiv(n, 256), 256, 0, s, g, eoff);
+    MS_TRY(ms::exclusive_scan_i32(eoff, eoff, n, total.p, s));
+    MS_LAUNCH(ms::k_poly_band_rows, ms::cdiv(2 * cols, 256), 256, 0, s, g, (const int *)eoff, row_eoff, row_mask);
+    int64_t *h = ms::host_flags().h;
+    MS_TRY(ms::readback(h, total.p, sizeof(int64_t), s));
+    MS_TRY(ms::stream_sync(s));
+    *n_edges = h[0];
+    if (h[0] < 0 || h[0] >= (1ll << 31) - 1024) {
+        ms::set_error("band polygonize: %lld boundary edges in one band do not fit", (long long)h[0]);
+        return MS_ERR_ARG;
+    }
+    return MS_OK;
+}
+
+int ms_band_poly_edges_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                           int32_t nodata, const int32_t *eoff, int64_t n_edges, const int64_t *halo_eoff,
+                           const uint8_t *halo_mask, uint32_t *ecell, int32_t *succ, uint64_t *lead, uint64_t *rank,
+                           int32_t *exit_edge, int64_t *exit_next, uint8_t *exit_corner, void *stream) {
+    MS_TRY(ms::ensure_init());
+    MS_TRY(ms::band_poly_args(lab, rows, cols, halo));
+    if (n_edges < 1 || n_edges >= (1ll << 31) - 1024 || !eoff || !halo_eoff || !halo_mask || !ecell || !succ || !lead ||
+        !rank || !exit_edge || !exit_next || !exit_corner) {
+        ms::set_error("band_poly_edges: bad argument");
+        return MS_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = rows * cols;
+    const int ne = (int)n_edges;
+    ms::PolyGrid g = ms::poly_band_grid(lab, rows, cols, halo, connect8, has_nodata, nodata);
+    MS_CUDA(cudaMemsetAsync(exit_edge, 0xff, (size_t)4 * cols * sizeof(int32_t), s));
+    ms::PolyHalo hb{halo_eoff, halo_mask, exit_edge, exit_next, exit_corner};
+    unsigned long long *sa = (unsigned long long *)lead, *sr = (unsigned long long *)rank;
+    MS_LAUNCH(ms::k_poly_edges, ms::cdiv(n, 256), 256, 0, s, g, eoff, ecell, succ, sa, hb);
+    ms::DevBuf<unsigned long long> tmp;
+    MS_TRY(tmp.alloc((size_t)ne, s));
+    unsigned long long *a = sa, *b = tmp.p;
+    MS_TRY(ms::jump_rounds(false, &a, &b, ne, s));
+    if (a != sa) MS_CUDA(cudaMemcpyAsync(sa, a, (size_t)ne * 8, cudaMemcpyDeviceToDevice, s));
+    MS_LAUNCH(ms::k_poly_rankinit, ms::cdiv(ne, 256), 256, 0, s, (const unsigned long long *)sa, (const int *)succ, sr, ne,
+              ms::kPolyChainBit);
+    a = sr;
+    b = tmp.p;
+    MS_TRY(ms::jump_rounds(true, &a, &b, ne, s));
+    if (a != sr) MS_CUDA(cudaMemcpyAsync(sr, a, (size_t)ne * 8, cudaMemcpyDeviceToDevice, s));
+    return ms::stream_sync(s);
+}
+
+int ms_band_poly_place_dev(int64_t cols, int64_t n_edges, const uint32_t *ecell, const int32_t *succ,
+                           const uint64_t *lead, const uint64_t *rank, int32_t *ishead, int32_t *uidx, int32_t *ulen,
+                           int32_t *ustart, uint32_t *placed, int32_t *corner, int32_t *vidx, int32_t *seg_entry,
+                           int32_t *seg_min, int32_t *seg_tmin, int64_t *counts2, void *stream) {
+    MS_TRY(ms::ensure_init());
+    if (cols < 1 || n_edges < 1 || n_edges >= (1ll << 31) - 1024 || !ecell || !succ || !lead || !rank || !ishead ||
+        !uidx || !ulen || !ustart || !placed || !corner || !vidx || !seg_entry || !seg_min || !seg_tmin || !counts2) {
+        ms::set_error("band_poly_place: bad argument");
+        return MS_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const int ne = (int)n_edges;
+    const unsigned long long *ls = (const unsigned long long *)lead, *rk = (const unsigned long long *)rank;
+    MS_CUDA(cudaMemsetAsync(corner, 0, (size_t)ne * sizeof(int), s));       // first the predecessor flags
+    MS_CUDA(cudaMemsetAsync(seg_min, 0xff, (size_t)4 * cols * sizeof(int), s));        // compared as unsigned
+    MS_LAUNCH(ms::k_poly_band_pred, ms::cdiv(ne, 256), 256, 0, s, ls, (const int *)succ, corner, seg_min, ne);
+    MS_LAUNCH(ms::k_poly_band_heads, ms::cdiv(ne, 256), 256, 0, s, ls, rk, (const int *)succ, (const int *)corner, ishead,
+              ulen, seg_entry, ne);
+    ms::DevBuf<int64_t> total;
+    MS_TRY(total.alloc(1, s));
+    int64_t *h = ms::host_flags().h;
+    MS_TRY(ms::exclusive_scan_i32(ishead, uidx, ne, total.p, s));
+    MS_TRY(ms::readback(h, total.p, sizeof(int64_t), s));
+    MS_TRY(ms::stream_sync(s));
+    counts2[0] = h[0];
+    MS_TRY(ms::exclusive_scan_i32(ulen, ustart, ne, total.p, s));
+    MS_CUDA(cudaMemsetAsync(corner, 0, (size_t)ne * sizeof(int), s));
+    MS_LAUNCH(ms::k_poly_band_place, ms::cdiv(ne, 256), 256, 0, s, ls, rk, (const int *)succ, ecell, (const int *)ustart,
+              (const int *)ulen, (const int *)seg_entry, (const int *)seg_min, placed, corner, seg_tmin, ne);
+    MS_TRY(ms::exclusive_scan_i32(corner, vidx, ne, total.p, s));
+    MS_TRY(ms::readback(h, total.p, sizeof(int64_t), s));
+    MS_TRY(ms::stream_sync(s));
+    counts2[1] = h[0];
+    return MS_OK;
+}
+
+int ms_band_poly_emit_dev(const int32_t *lab, int64_t rows, int64_t cols, int halo, int connect8, int has_nodata,
+                          int32_t nodata, int64_t row0, int64_t n_edges, const uint32_t *ecell, const uint64_t *lead,
+                          const int32_t *ishead, const int32_t *uidx, const int32_t *ulen, const int32_t *ustart,
+                          const uint32_t *placed, const int32_t *corner, const int32_t *vidx, int64_t nverts,
+                          int32_t *vrow, int32_t *vcol, int32_t *u_head, int32_t *u_len, int32_t *u_vstart,
+                          int32_t *u_vcount, int32_t *u_value, int64_t *u_root, int32_t *u_slot, int64_t *root_rows,
+                          void *stream) {
+    MS_TRY(ms::ensure_init());
+    MS_TRY(ms::band_poly_args(lab, rows, cols, halo));
+    if (n_edges < 1 || n_edges >= (1ll << 31) - 1024 || nverts < 0 || nverts > n_edges || !ecell || !lead || !ishead ||
+        !uidx || !ulen || !ustart || !placed || !corner || !vidx || !vrow || !vcol || !u_head || !u_len || !u_vstart ||
+        !u_vcount || !u_value || !u_root || !u_slot || !root_rows) {
+        ms::set_error("band_poly_emit: bad argument");
+        return MS_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = rows * cols, cell0 = row0 * cols;
+    const int ne = (int)n_edges;
+    ms::PolyGrid g = ms::poly_band_grid(lab, rows, cols, halo, connect8, has_nodata, nodata);
+    MS_LAUNCH(ms::k_poly_emit, ms::cdiv(ne, 256), 256, 0, s, placed, corner, vidx, (int)cols, (int)row0, vrow, vcol, ne);
+    ms::DevBuf<int> par;
+    MS_TRY(par.alloc((size_t)n, s));
+    MS_LAUNCH(ms::k_poly_parinit, ms::cdiv(n, 256), 256, 0, s, par.p, n);
+    MS_LAUNCH(ms::k_poly_union, ms::cdiv(n, 256), 256, 0, s, g, par.p);
+    MS_LAUNCH(ms::k_poly_band_units, ms::cdiv(ne, 256), 256, 0, s, g, (const unsigned long long *)lead, ishead, uidx,
+              ustart, ulen, vidx, ecell, par.p, cell0, ne, (int)nverts, u_head, u_len, u_vstart, u_vcount, u_value,
+              u_root, u_slot);
+    MS_LAUNCH(ms::k_poly_band_rowroots, ms::cdiv(2 * cols, 256), 256, 0, s, g, par.p, cell0, root_rows);
+    return ms::stream_sync(s);
 }
 
 /* copies the rings of the last ms_polygonize* call to host arrays (sizes from its counts) and releases them */
